@@ -2,7 +2,7 @@
 """bench.py -- BWT build throughput (Mbp/s) of the deBWT hot path on B200, next to the CPU reference.
 
 Contract (one JSON line on stdout, printed by rank 0):
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3] [--dump-outputs DIR]
   N > 1 is launched by the driver through torch.distributed.run (one rank per GPU).
 
 Default workload: BASELINE.json configs[2], the 3.1 Gbp human-genome-sized sequence with interspersed repeat families
@@ -21,6 +21,8 @@ detection -> branch codes -> segmented sort -> BWT emission) over the genome.
           (tests/golden/workload_sha.json) and the GPU LF-inversion verifier (debwt_verify_*: the BWT inverted by
           its LF mapping must reproduce the input text)
 --impl reference times the reference's own CPU implementation on a bounded prefix of the same workload.
+--dump-outputs DIR writes the BWT of the last timed step (a seeded sample of its rows) to DIR; the workloads are seeded,
+so two builds of the project run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -122,6 +124,34 @@ def expected_sha(name: str):
         return json.load(open(p)).get(name)
     except (OSError, ValueError):
         return None
+
+
+DUMP_ROWS = 1 << 22     # BWT rows sampled by --dump-outputs: 12 B each (float64 row + float32 code), 48 MB at most
+
+
+def dump_outputs(out_dir: str, words, sharp, dollar, n_rows: int) -> dict:
+    """Writes the BWT a caller receives (packed words, '#' rows, '$' row) as float arrays that two builds can be
+    compared with, output for output:
+      sharp_rows.npy, dollar_row.npy : float64, every row (exact: rows < 2^53)
+      bwt_rows.npy, bwt_codes.npy    : float64 row numbers and float32 symbol codes (0-3 = A,C,G,T, 4 = '#', 5 = '$') of
+                                       DUMP_ROWS rows, one seeded pick from each of DUMP_ROWS equal slices of the BWT (all
+                                       rows when there are fewer)"""
+    import numpy as np
+    words = np.asarray(words).view(np.uint64)
+    if n_rows <= DUMP_ROWS:
+        rows = np.arange(n_rows, dtype=np.uint64)
+    else:
+        edges = np.arange(DUMP_ROWS + 1, dtype=np.uint64) * np.uint64(n_rows) // np.uint64(DUMP_ROWS)
+        rows = np.random.default_rng(20261020).integers(edges[:-1], edges[1:], dtype=np.uint64)
+    codes = (words[rows >> np.uint64(5)] >> (np.uint64(62) - np.uint64(2) * (rows & np.uint64(31)))) & np.uint64(3)
+    codes[np.isin(rows, sharp)] = 4
+    codes[rows == np.uint64(dollar[0])] = 5
+    arrays = {"sharp_rows": np.asarray(sharp).astype(np.float64), "dollar_row": np.asarray(dollar).astype(np.float64),
+              "bwt_rows": rows.astype(np.float64), "bwt_codes": codes.astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "rows_sampled": int(rows.size), "rows": n_rows}
 
 
 # ------------------------------------------------------------------------------------------------
@@ -378,6 +408,10 @@ def ours(args, rank, world, local_rank):
     launches = int(binding.lib().debwt_launch_count() - l0)
     clocks = clk.summary()
     ms_dev = dev_ms / args.steps
+    dumped = None
+    if args.dump_outputs:                                 # before the e2e leg reuses h_out
+        sharp, dollar = b.result_into(h_out.data_ptr())
+        dumped = dump_outputs(args.dump_outputs, h_out.numpy(), sharp, dollar, n)
 
     for _ in range(2):
         step_e2e()
@@ -421,6 +455,8 @@ def ours(args, rank, world, local_rank):
         "verify": verify,
         "bwt_sha256": sha,
     }
+    if dumped:
+        line["dump_outputs"] = dumped
     b.close()
     if not args.no_file_to_file:
         try:
@@ -707,12 +743,18 @@ def main():
     ap.add_argument("--orchestrator", default="c", choices=["c", "python"],
                     help="N > 1: the sharded build behind the C ABI (csrc/shard.cu) or the Python harness debwt_b200/dist.py")
     ap.add_argument("--sharded", action="store_true", help="use the sharded (multi-GPU) code path even at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single-GPU path: write the BWT of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.no_clocks:
         os.environ["DEBWT_NO_CLOCKS"] = "1"
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1 or args.sharded):
+        ap.error("--dump-outputs is implemented for the single-GPU path only")
     if args.impl == "reference":
         reference_arm(args, rank, world)
         return
