@@ -157,6 +157,43 @@ class BwtBuilder:
         check(lib().debwt_index_count(self._h, _ptr(blob), _ptr(offs), len(pats), _ptr(out)))
         return out
 
+    def set_result(self, words: np.ndarray, n_symbols: int, sharp: np.ndarray, dollar):
+        """Load a finished result (the reference's three outputs, e.g. from `read_outputs` or `build_multi`) in place of a
+        build, to query it with count / sample_sa / sa / locate / verify."""
+        words = np.ascontiguousarray(words, dtype=np.uint64)
+        sharp = np.ascontiguousarray(sharp, dtype=np.uint64)
+        if words.size != (n_symbols + 31) // 32:
+            raise DebwtError(f"set_result: {words.size} words for {n_symbols} symbols (expected {(n_symbols + 31) // 32})")
+        dollar = int(np.asarray(dollar).reshape(-1)[0])
+        check(lib().debwt_set_result(self._h, _ptr(words), n_symbols, _ptr(sharp), sharp.size, dollar))
+
+    def sample_sa(self, rate: int = 32) -> float:
+        """Sample the suffix array every `rate` text positions (power of two, 1..1024); returns the device ms."""
+        ms = ctypes.c_float()
+        check(lib().debwt_index_sample_sa(self._h, rate, ctypes.byref(ms)))
+        return float(ms.value)
+
+    def sa(self, rows) -> np.ndarray:
+        """SA[r] (text position of the suffix in row r) for every row in `rows`; needs sample_sa"""
+        rows = np.ascontiguousarray(rows, dtype=np.uint64)
+        out = np.empty(rows.size, dtype=np.uint64)
+        check(lib().debwt_index_sa(self._h, _ptr(rows), rows.size, _ptr(out)))
+        return out
+
+    def locate(self, patterns: Sequence) -> tuple[np.ndarray, np.ndarray]:
+        """(hit_offsets u64[len + 1], positions u64[hits]): pattern i occurs at positions[hit_offsets[i]:hit_offsets[i+1]],
+        in suffix-array order; needs sample_sa"""
+        pats = [p.encode() if isinstance(p, str) else bytes(p) for p in patterns]
+        offs = np.zeros(len(pats) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(p) for p in pats])
+        blob = np.frombuffer(b"".join(pats) + b"\0", dtype=np.uint8)
+        hits = np.zeros(len(pats) + 1, dtype=np.uint64)
+        check(lib().debwt_index_locate(self._h, _ptr(blob), _ptr(offs), len(pats), _ptr(hits), c_p(0), 0))
+        pos = np.empty(int(hits[-1]), dtype=np.uint64)
+        if pos.size:
+            check(lib().debwt_index_locate(self._h, _ptr(blob), _ptr(offs), len(pats), _ptr(hits), _ptr(pos), pos.size))
+        return hits, pos
+
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""
         bad, ms = c_u64(), ctypes.c_float()
@@ -186,6 +223,31 @@ def write_outputs(path: str, words: np.ndarray, sharp: np.ndarray, dollar: np.nd
     words.astype("<u8", copy=False).tofile(path)
     sharp.astype("<u8", copy=False).tofile(path + ".#")
     dollar.astype("<u8", copy=False).tofile(path + ".$")
+
+
+def read_outputs(path: str, n_symbols: int):
+    """The inverse of `write_outputs`: (words, sharp, dollar) from the three files.  The files do not hold N, so the
+    caller passes it; the word file must hold exactly ceil(N / 32) words."""
+    words = np.fromfile(path, dtype="<u8").astype(np.uint64, copy=False)
+    if words.size != (n_symbols + 31) // 32:
+        raise DebwtError(f"{path}: {words.size} words, but {n_symbols} symbols need {(n_symbols + 31) // 32}")
+    sharp = np.fromfile(path + ".#", dtype="<u8").astype(np.uint64, copy=False)
+    dollar = np.fromfile(path + ".$", dtype="<u8").astype(np.uint64, copy=False)
+    if dollar.size != 1:
+        raise DebwtError(f"{path}.$: {dollar.size} values, expected 1")
+    return words, sharp, dollar
+
+
+def record_offsets(positions, seps) -> tuple[np.ndarray, np.ndarray]:
+    """Text positions in T = S1 # S2 # ... Sn $ to (record index, offset in that record).  `seps` are the separator
+    positions (join_records); a separator maps to its record with offset = the record's length."""
+    pos = np.asarray(positions, dtype=np.uint64)
+    seps = np.asarray(seps, dtype=np.uint64)
+    if pos.size and int(pos.max()) > int(seps[-1]):
+        raise ValueError(f"position {int(pos.max())} is beyond the text ({int(seps[-1]) + 1} symbols)")
+    rec = np.searchsorted(seps, pos, side="left")
+    starts = np.concatenate(([0], seps[:-1] + 1)).astype(np.uint64)
+    return rec.astype(np.int64), pos - starts[rec]
 
 
 # ---- per-kernel entry points (parity tests) -------------------------------------------------------

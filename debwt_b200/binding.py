@@ -77,6 +77,10 @@ _SIGS = {
     "debwt_index_sizes": (ctypes.c_int, [c_p, ctypes.POINTER(c_u64)]),
     "debwt_index_copy": (ctypes.c_int, [c_p, c_p, c_p]),
     "debwt_index_count": (ctypes.c_int, [c_p, c_p, c_p, c_u64, c_p]),
+    "debwt_set_result": (ctypes.c_int, [c_p, c_p, c_u64, c_p, c_u64, c_u64]),
+    "debwt_index_sample_sa": (ctypes.c_int, [c_p, ctypes.c_uint32, ctypes.POINTER(ctypes.c_float)]),
+    "debwt_index_sa": (ctypes.c_int, [c_p, c_p, c_u64, c_p]),
+    "debwt_index_locate": (ctypes.c_int, [c_p, c_p, c_p, c_u64, c_p, c_p, c_u64]),
     "debwt_verify_text": (ctypes.c_int, [c_p, c_p, c_u64, ctypes.POINTER(c_u64), ctypes.POINTER(ctypes.c_float)]),
     "debwt_verify_text_device": (ctypes.c_int, [c_p, c_p, c_u64, ctypes.POINTER(c_u64), ctypes.POINTER(ctypes.c_float)]),
     "debwt_verify_bwt_device": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_u64, c_p, ctypes.POINTER(c_u64),

@@ -163,6 +163,7 @@ void reset_input(debwt_ctx* c) {
     c->d_sharp_count = nullptr;
     c->d_dollar = nullptr;
     c->built = false;
+    c->loaded = false;
     c->stats = debwt_stats{};
 }
 
@@ -301,6 +302,7 @@ int debwt_set_text_device(debwt_ctx* c, const void* d_text, uint64_t n, const ui
 int debwt_build(debwt_ctx* c, int k) {
     if (!c) FAIL("null context");
     if (k < 12 || k > 32) FAIL("-k: k-mer length (from 12 to 32, default 32)");      // src/main.c:45-46
+    if (c->loaded) FAIL("the context holds a loaded result (debwt_set_result), not an input: set an input before building");
     if (c->n == 0) FAIL("no input set");
     if (bind_device(c->device)) return -1;
     const u8* ascii = c->d_ascii_ext ? c->d_ascii_ext : c->d_ascii;
@@ -574,6 +576,44 @@ int debwt_result_copy(debwt_ctx* c, uint64_t* bwt_words, uint64_t* sharp_rows, u
     std::sort(sharp.begin(), sharp.begin() + cnt);                      // ascending (src/insertCase3.c:84-95)
     if (sharp_rows) std::copy(sharp.begin(), sharp.begin() + cnt, sharp_rows);
     if (dollar_row) *dollar_row = dol;
+    return 0;
+}
+
+int debwt_set_result(debwt_ctx* c, const uint64_t* bwt_words, uint64_t n_symbols, const uint64_t* sharp_rows, uint64_t n_sharp,
+                     uint64_t dollar_row) {
+    if (!c || !bwt_words || (n_sharp && !sharp_rows)) FAIL("null argument");
+    if (bind_device(c->device)) return -1;
+    reset_input(c);
+    c->n = 0; c->n_rec = 0; c->n_words = 0;
+    c->seps.clear();
+    if (n_symbols == 0) FAIL("set_result: no symbols");
+    if (dollar_row >= n_symbols) FAIL("set_result: the '$' row " + std::to_string(dollar_row) + " is not below n_symbols");
+    std::vector<u64> sorted(sharp_rows, sharp_rows + n_sharp);
+    std::sort(sorted.begin(), sorted.end());
+    for (u64 i = 0; i < n_sharp; ++i) {
+        if (sorted[i] >= n_symbols) FAIL("set_result: a '#' row (" + std::to_string(sorted[i]) + ") is not below n_symbols");
+        if (i && sorted[i] == sorted[i - 1]) FAIL("set_result: the '#' row " + std::to_string(sorted[i]) + " is listed twice");
+        if (sorted[i] == dollar_row) FAIL("set_result: the '$' row is also listed as a '#' row");
+    }
+    // where a build leaves its result (debwt_build: d_bwt, d_sharp, d_sharp_count, d_dollar)
+    const u64 R = n_sharp + 1, nbw = (n_symbols + 31) / 32;
+    if (dalloc(c->pool, &c->d_bwt, nbw + 1) || dalloc(c->pool, &c->d_sharp, R + 1) || dalloc(c->pool, &c->d_sharp_count, 4) ||
+        dalloc(c->pool, &c->d_dollar, 2))
+        return -1;
+    const u32 cnt = (u32)n_sharp;
+    if (n_sharp != cnt) FAIL("set_result: too many '#' rows");
+    CUDA_TRY(cudaMemcpyAsync(c->d_bwt, bwt_words, nbw * 8, cudaMemcpyHostToDevice, c->st));
+    CUDA_TRY(cudaMemsetAsync(c->d_bwt + nbw, 0, 8, c->st));
+    CUDA_TRY(cudaMemsetAsync(c->d_sharp, 0, (R + 1) * 8, c->st));
+    if (n_sharp) CUDA_TRY(cudaMemcpyAsync(c->d_sharp, sorted.data(), n_sharp * 8, cudaMemcpyHostToDevice, c->st));
+    CUDA_TRY(cudaMemsetAsync(c->d_sharp_count, 0, 16, c->st));
+    CUDA_TRY(cudaMemcpyAsync(c->d_sharp_count, &cnt, 4, cudaMemcpyHostToDevice, c->st));
+    CUDA_TRY(cudaMemcpyAsync(c->d_dollar, &dollar_row, 8, cudaMemcpyHostToDevice, c->st));
+    CUDA_TRY(cudaStreamSynchronize(c->st));
+    c->n = n_symbols; c->n_rec = R; c->n_words = nbw;
+    c->stats.n_symbols = n_symbols; c->stats.n_records = R;
+    c->built = true;
+    c->loaded = true;
     return 0;
 }
 

@@ -134,9 +134,16 @@ struct debwt_ctx {
     u64 c_array[6] = {0, 0, 0, 0, 0, 0};
     u64 dollar_row = 0;
     bool indexed = false;
+    // sampled suffix array (index.cu, debwt_index_sample_sa); own cudaMalloc allocations, dropped with the index
+    u64* d_sa_bits = nullptr;         // [ceil(N / 32)]: sampled-row mask of the word (low half) | sampled rows before it (high)
+    u32* d_sa_vals = nullptr;         // SA values of the sampled rows, in row order
+    u32 sa_rate = 0;                  // 0 = not sampled
+    u64 n_sa_samples = 0;
+    bool loaded = false;              // the result came from debwt_set_result, not from a build
 };
 
 namespace debwt {
 void drop_index(debwt_ctx* c);        // index.cu
+void drop_samples(debwt_ctx* c);      // index.cu
 }
 

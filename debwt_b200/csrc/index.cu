@@ -207,19 +207,199 @@ __global__ void lf_walk_kernel(FmView f, const u8* __restrict__ tail, u64 steps,
     *bad = nb;
 }
 
+// pattern symbol: A, C, G, T in either case -> 0..3, anything else -> 4 (occurs nowhere)
+__device__ __forceinline__ u32 pattern_symbol(u8 c) {
+    switch (c & 0xDFu) {
+        case 'A': return 0u;
+        case 'C': return 1u;
+        case 'G': return 2u;
+        case 'T': return 3u;
+        default: return 4u;
+    }
+}
+
+// backward search of pats[lo .. hi): the rows [sp, ep) whose suffixes start with the pattern (empty when ep <= sp)
+__device__ __forceinline__ void fm_range(const FmView& f, const u8* __restrict__ pats, u64 lo, u64 hi, u64& sp_out, u64& ep_out) {
+    u64 sp = 0, ep = f.n;
+    for (u64 i = hi; i > lo && sp < ep; --i) {
+        const u32 c = pattern_symbol(pats[i - 1]);
+        if (c > 3u) { sp = ep = 0; break; }
+        sp = f.C[c] + occ_before(f, c, sp);
+        ep = f.C[c] + (ep == f.n ? f.C[c + 1] - f.C[c] : occ_before(f, c, ep));
+    }
+    sp_out = sp;
+    ep_out = ep > sp ? ep : sp;
+}
+
 // backward search of one pattern per thread (count only)
 __global__ void __launch_bounds__(TPB) fm_count_kernel(FmView f, const u8* __restrict__ pats, const u64* __restrict__ offs, u64 m,
                                                       u64* __restrict__ counts) {
     const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
     if (t >= m) return;
-    u64 sp = 0, ep = f.n;                                                         // rows [sp, ep)
-    for (u64 i = offs[t + 1]; i > offs[t] && sp < ep; --i) {
-        const u32 c = ascii_symbol(pats[i - 1]);
-        if (c > 3u) { sp = ep = 0; break; }
-        sp = f.C[c] + occ_before(f, c, sp);
-        ep = f.C[c] + (ep == f.n ? f.C[c + 1] - f.C[c] : occ_before(f, c, ep));
+    u64 sp, ep;
+    fm_range(f, pats, offs[t], offs[t + 1], sp, ep);
+    counts[t] = ep - sp;
+}
+
+// ---- sampled suffix array ----------------------------------------------------------------------------------------
+// After the list ranking, row r is at text position SA[r] = (d(r) + 1) mod N (d = low half of its node).  Rows with
+// SA[r] % rate == 0 are sampled: bits[w] = mask of the sampled rows of word w (low half) | sampled rows in words < w (high
+// half), vals[] = their SA values in row order.  The '$' row (SA = 0) is always sampled, so an LF walk from any row reaches
+// a sampled row within rate - 1 steps without wrapping around the text.
+struct SaView {
+    const u64* bits;
+    const u32* vals;
+    u32 rate;
+};
+
+__device__ __forceinline__ u64 block_exclusive_scan_u64(u64 v, u64* total, u64* smem /* 32 u64 */) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    u64 inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const u64 t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += t;
     }
-    counts[t] = ep > sp ? ep - sp : 0;
+    __syncthreads();
+    if (lane == 31) smem[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        u64 w = lane < TPB / 32 ? smem[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const u64 t = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= o) w += t;
+        }
+        smem[lane] = w;
+    }
+    __syncthreads();
+    if (total) *total = smem[TPB / 32 - 1];
+    return (warp ? smem[warp - 1] : 0) + inc - v;
+}
+
+// the sampled-row mask of word (first word of this warp) + lane; every warp covers 32 words = 1024 rows, one coalesced row
+// per lane and step.  `bad` counts rows whose walk did not reach the end (LF is not one N-cycle).
+__device__ __forceinline__ u32 sa_word_mask(const u64* __restrict__ node, u64 n, u64 w0, u32 rate, unsigned long long* bad) {
+    const u32 lane = threadIdx.x & 31;
+    u32 mine = 0, off_cycle = 0;
+    for (u32 j = 0; j < 32; ++j) {
+        const u64 r = (w0 + j) * 32 + lane;
+        bool take = false;
+        if (r < n) {
+            const u64 a = node[r];
+            if ((u32)(a >> 32) != NIL) ++off_cycle;
+            const u64 pos = (u64)(u32)a + 1 == n ? 0 : (u64)(u32)a + 1;
+            take = (pos & (rate - 1)) == 0;
+        }
+        const u32 m = __ballot_sync(0xffffffffu, take);
+        if (lane == j) mine = m;
+    }
+    if (bad) {
+        off_cycle = __reduce_add_sync(0xffffffffu, off_cycle);
+        if (lane == 0 && off_cycle) atomicAdd(bad, (unsigned long long)off_cycle);
+    }
+    return mine;
+}
+
+// per block of TPB words: number of sampled rows; rows off the one cycle into *bad
+__global__ void __launch_bounds__(TPB) sa_count_kernel(const u64* __restrict__ node, u64 n, u32 rate, u64* __restrict__ block_tot,
+                                                      unsigned long long* __restrict__ bad) {
+    __shared__ u64 sm[32];
+    const u64 w0 = (u64)blockIdx.x * TPB + (threadIdx.x & ~31u);
+    const u32 m = sa_word_mask(node, n, w0, rate, bad);
+    u64 tot;
+    block_exclusive_scan_u64(__popc(m), &tot, sm);
+    if (threadIdx.x == 0) block_tot[blockIdx.x] = tot;
+}
+
+// exclusive scan of nb u64 (one block, sequential over chunks); the total goes to base[nb]
+__global__ void __launch_bounds__(TPB) scan_u64_kernel(const u64* __restrict__ in, u64 nb, u64* __restrict__ base) {
+    __shared__ u64 sm[32];
+    u64 carry = 0;
+    for (u64 b = 0; b < nb; b += TPB) {
+        const u64 i = b + threadIdx.x;
+        u64 tot;
+        const u64 ex = block_exclusive_scan_u64(i < nb ? in[i] : 0, &tot, sm);
+        if (i < nb) base[i] = carry + ex;
+        carry += tot;
+    }
+    if (threadIdx.x == 0) base[nb] = carry;
+}
+
+// bits[w] for every word, and the SA value of every sampled row at its rank
+__global__ void __launch_bounds__(TPB) sa_write_kernel(const u64* __restrict__ node, u64 n, u64 nwords, u32 rate,
+                                                      const u64* __restrict__ block_base, u64* __restrict__ bits,
+                                                      u32* __restrict__ vals) {
+    __shared__ u64 sm[32];
+    const u32 lane = threadIdx.x & 31;
+    const u64 w0 = (u64)blockIdx.x * TPB + (threadIdx.x & ~31u);
+    const u32 m = sa_word_mask(node, n, w0, rate, nullptr);
+    const u64 before = block_base[blockIdx.x] + block_exclusive_scan_u64(__popc(m), nullptr, sm);
+    if (w0 + lane < nwords) bits[w0 + lane] = (before << 32) | m;
+    for (u32 j = 0; j < 32; ++j) {
+        const u32 mj = __shfl_sync(0xffffffffu, m, j);
+        const u64 bj = __shfl_sync(0xffffffffu, before, j);
+        if ((mj >> lane) & 1u) {
+            const u64 a = node[(w0 + j) * 32 + lane];
+            vals[bj + __popc(mj & ((1u << lane) - 1u))] = (u64)(u32)a + 1 == n ? 0u : (u32)a + 1u;
+        }
+    }
+}
+
+// SA[r]: LF steps from r until a sampled row, whose value plus the steps taken is the answer (at most rate - 1 steps)
+__device__ __forceinline__ u64 sa_of(const FmView& f, const SaView& s, u64 r) {
+    for (u32 steps = 0; steps < s.rate; ++steps) {
+        const u64 b = s.bits[r >> 5];
+        const u32 m = (u32)b, bit = 1u << (r & 31);
+        if (m & bit) return (u64)s.vals[(b >> 32) + __popc(m & (bit - 1u))] + steps;
+        r = lf_of(f, r);
+    }
+    return ~0ull;                                                                 // not reached for a sampled BWT
+}
+
+__global__ void __launch_bounds__(TPB) sa_lookup_kernel(FmView f, SaView s, const u64* __restrict__ rows, u64 m, u64* __restrict__ out) {
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (t < m) out[t] = sa_of(f, s, rows[t]);
+}
+
+// per pattern: first row of its range and its hit count
+__global__ void __launch_bounds__(TPB) fm_range_kernel(FmView f, const u8* __restrict__ pats, const u64* __restrict__ offs, u64 m,
+                                                      u64* __restrict__ sp_out, u64* __restrict__ counts) {
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (t >= m) return;
+    u64 sp, ep;
+    fm_range(f, pats, offs[t], offs[t + 1], sp, ep);
+    sp_out[t] = sp;
+    counts[t] = ep - sp;
+}
+
+// per block of TPB patterns: total hits
+__global__ void __launch_bounds__(TPB) hit_count_kernel(const u64* __restrict__ counts, u64 m, u64* __restrict__ block_tot) {
+    __shared__ u64 sm[32];
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    u64 tot;
+    block_exclusive_scan_u64(t < m ? counts[t] : 0, &tot, sm);
+    if (threadIdx.x == 0) block_tot[blockIdx.x] = tot;
+}
+
+// hit_offsets[t] = hits of the patterns before t; hit_offsets[m] = all hits
+__global__ void __launch_bounds__(TPB) hit_offsets_kernel(const u64* __restrict__ counts, u64 m, const u64* __restrict__ block_base,
+                                                         u64* __restrict__ hit_offsets) {
+    __shared__ u64 sm[32];
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    const u64 v = t < m ? counts[t] : 0;
+    const u64 ex = block_base[blockIdx.x] + block_exclusive_scan_u64(v, nullptr, sm);
+    if (t < m) hit_offsets[t] = ex;
+    if (t + 1 == m) hit_offsets[m] = ex + v;
+}
+
+// one thread per hit: its pattern by binary search over hit_offsets, then SA of row sp + j, in SA order
+__global__ void __launch_bounds__(TPB) locate_kernel(FmView f, SaView s, const u64* __restrict__ hit_offsets, const u64* __restrict__ sp,
+                                                    u64 m, u64 total, u64* __restrict__ positions) {
+    const u64 h = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (h >= total) return;
+    const u64 i = upper_bound_u64(hit_offsets, 0, m + 1, h) - 1;                 // last pattern whose hits start at or before h
+    positions[h] = sa_of(f, s, sp[i] + (h - hit_offsets[i]));
 }
 
 FmView view_of(const debwt_ctx* c) {
@@ -230,9 +410,19 @@ FmView view_of(const debwt_ctx* c) {
     return f;
 }
 
+SaView sa_view_of(const debwt_ctx* c) { return SaView{c->d_sa_bits, c->d_sa_vals, c->sa_rate}; }
+
 }  // namespace
 
+void drop_samples(debwt_ctx* c) {
+    if (c->d_sa_bits) cudaFree(c->d_sa_bits);
+    if (c->d_sa_vals) cudaFree(c->d_sa_vals);
+    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr;
+    c->sa_rate = 0;
+}
+
 void drop_index(debwt_ctx* c) {
+    drop_samples(c);
     if (c->d_occ) cudaFree(c->d_occ);
     if (c->d_spec_bits) cudaFree(c->d_spec_bits);
     if (c->d_sharp_sorted) cudaFree(c->d_sharp_sorted);
@@ -347,6 +537,26 @@ int debwt_index_count(debwt_ctx* c, const char* patterns, const uint64_t* offset
     return 0;
 }
 
+// List ranking of the LF walk by pointer jumping (Wyllie), shared by the verifier and the SA sampler.  d_a, d_b: N u64 each;
+// on return d_a holds the ranked list: for every row r the high half is NIL iff r's walk reached the end of the list, and
+// the low half is then the number of LF steps from r to that end.  d_live: one u32 of device scratch.
+static int rank_lf(cudaStream_t st, const FmView& f, u64*& d_a, u64*& d_b, u32* d_live) {
+    const u64 n = f.n;
+    lf_init_kernel<<<grid_for(n), TPB, 0, st>>>(f, d_a);
+    DEBWT_COUNT(1);
+    for (int rounds = 0; rounds < 34; ++rounds) {
+        u32 live = 0;
+        CUDA_TRY(cudaMemsetAsync(d_live, 0, 4, st));
+        jump_kernel<<<grid_for(n), TPB, 0, st>>>(d_a, d_b, n, d_live);
+        DEBWT_COUNT(1);
+        CUDA_TRY(cudaMemcpyAsync(&live, d_live, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        std::swap(d_a, d_b);
+        if (!live) break;
+    }
+    return 0;
+}
+
 static int verify_indexed(debwt_ctx* c, const void* d_text, uint64_t* n_bad_out, float* ms_out) {
     if (c->n >= 0xFFFFFFFFull) FAIL("verify: N must be below 2^32 - 1");
     CUDA_TRY(cudaSetDevice(c->device));
@@ -366,19 +576,7 @@ static int verify_indexed(debwt_ctx* c, const void* d_text, uint64_t* n_bad_out,
     CUDA_TRY(cudaEventCreate(&e0)); CUDA_TRY(cudaEventCreate(&e1));
     CUDA_TRY(cudaEventRecord(e0, st));
     const FmView f = view_of(c);
-    lf_init_kernel<<<grid_for(n), TPB, 0, st>>>(f, d_a);
-    DEBWT_COUNT(1);
-    int rounds = 0;
-    for (; rounds < 34; ++rounds) {
-        u32 live = 0;
-        CUDA_TRY(cudaMemsetAsync(d_live, 0, 4, st));
-        jump_kernel<<<grid_for(n), TPB, 0, st>>>(d_a, d_b, n, d_live);
-        DEBWT_COUNT(1);
-        CUDA_TRY(cudaMemcpyAsync(&live, d_live, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        std::swap(d_a, d_b);
-        if (!live) break;
-    }
+    if (rank_lf(st, f, d_a, d_b, d_live)) return -1;
     CUDA_TRY(cudaMemsetAsync(d_bad, 0, 8, st));
     lf_check_kernel<<<grid_for(n), TPB, 0, st>>>(f, d_a, static_cast<const u8*>(d_text), d_bad);
     DEBWT_COUNT(1);
@@ -468,6 +666,143 @@ int debwt_verify_text(debwt_ctx* c, const char* text, uint64_t n_symbols, uint64
     const int rc = debwt_verify_text_device(c, d_t, n_symbols, n_bad_out, ms_out);
     cudaFree(d_t);
     return rc;
+}
+
+int debwt_index_sample_sa(debwt_ctx* c, uint32_t rate, float* ms_out) {
+    if (!c || !c->built) FAIL("no result: call debwt_build first");
+    if (rate < 1 || rate > 1024 || (rate & (rate - 1))) FAIL("sample_sa: the rate must be a power of two from 1 to 1024");
+    if (c->n >= 0xFFFFFFFFull)
+        FAIL("sample_sa: N = " + std::to_string(c->n) + " symbols; the list ranking that samples the suffix array needs N below 2^32 - 1");
+    if (debwt_index_build(c)) return -1;
+    CUDA_TRY(cudaSetDevice(c->device));
+    drop_samples(c);
+    cudaStream_t st = c->st;
+    const u64 n = c->n, nwords = (n + 31) / 32, nb = (nwords + TPB - 1) / TPB;
+    u64 *d_a = nullptr, *d_b = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_a), n * 8) != cudaSuccess || cudaMalloc(reinterpret_cast<void**>(&d_b), n * 8) != cudaSuccess) {
+        cudaGetLastError();
+        if (d_a) cudaFree(d_a);
+        FAIL("sample_sa: not enough device memory for the list-ranking buffers (16 bytes per symbol)");
+    }
+    // scratch: live flag, bad-row count, block totals (nb), their scan (nb + 1)
+    u64* d_s = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_s), (2 * nb + 3) * 8) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d_a); cudaFree(d_b);
+        FAIL("sample_sa: out of device memory");
+    }
+    u32* d_live = reinterpret_cast<u32*>(d_s);
+    unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(d_s + 1);
+    u64 *d_tot = d_s + 2, *d_base = d_s + 2 + nb;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    auto fail = [&](const std::string& msg) {
+        cudaStreamSynchronize(st);
+        cudaGetLastError();
+        cudaFree(d_a); cudaFree(d_b); cudaFree(d_s);
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+        drop_samples(c);
+        set_error(msg);
+        return -1;
+    };
+    if (cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess || cudaEventRecord(e0, st) != cudaSuccess)
+        return fail(std::string("sample_sa: ") + cudaGetErrorString(cudaGetLastError()));
+    const FmView f = view_of(c);
+    if (rank_lf(st, f, d_a, d_b, d_live)) return fail(debwt_last_error());
+    if (cudaMemsetAsync(d_bad, 0, 8, st) != cudaSuccess) return fail(std::string("sample_sa: ") + cudaGetErrorString(cudaGetLastError()));
+    sa_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_a, n, rate, d_tot, d_bad);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
+    DEBWT_COUNT(2);
+    unsigned long long bad = 0;
+    u64 n_samples = 0;
+    if (cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaMemcpyAsync(&n_samples, d_base + nb, 8, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(std::string("sample_sa: ") + cudaGetErrorString(cudaGetLastError()));
+    if (bad)
+        return fail("sample_sa: the result is not a BWT: " + std::to_string(bad) + " of " + std::to_string(n) +
+                    " rows are not on the one N-cycle of its LF mapping");
+    if (n_samples != (n + rate - 1) / rate) return fail("internal: wrong number of sampled rows");
+    if (cudaMalloc(reinterpret_cast<void**>(&c->d_sa_bits), nwords * 8) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&c->d_sa_vals), n_samples * 4) != cudaSuccess)
+        return fail("sample_sa: out of device memory for the samples");
+    sa_write_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_a, n, nwords, rate, d_base, c->d_sa_bits, c->d_sa_vals);
+    DEBWT_COUNT(1);
+    float ms = 0;
+    if (cudaEventRecord(e1, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess ||
+        cudaEventElapsedTime(&ms, e0, e1) != cudaSuccess)
+        return fail(std::string("sample_sa: ") + cudaGetErrorString(cudaGetLastError()));
+    cudaEventDestroy(e0); cudaEventDestroy(e1);
+    cudaFree(d_a); cudaFree(d_b); cudaFree(d_s);
+    c->sa_rate = rate;
+    c->n_sa_samples = n_samples;
+    if (ms_out) *ms_out = ms;
+    return 0;
+}
+
+int debwt_index_sa(debwt_ctx* c, const uint64_t* rows, uint64_t n_rows, uint64_t* positions) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (n_rows == 0) return 0;
+    if (!rows || !positions) FAIL("null argument");
+    for (u64 i = 0; i < n_rows; ++i)
+        if (rows[i] >= c->n) FAIL("index_sa: row " + std::to_string(rows[i]) + " (argument " + std::to_string(i) + ") is not below N = " + std::to_string(c->n));
+    CUDA_TRY(cudaSetDevice(c->device));
+    u64* d = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d), n_rows * 16));
+    CUDA_TRY(cudaMemcpyAsync(d, rows, n_rows * 8, cudaMemcpyHostToDevice, c->st));
+    sa_lookup_kernel<<<grid_for(n_rows), TPB, 0, c->st>>>(view_of(c), sa_view_of(c), d, n_rows, d + n_rows);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(positions, d + n_rows, n_rows * 8, cudaMemcpyDeviceToHost, c->st));
+    CUDA_TRY(cudaStreamSynchronize(c->st));
+    CUDA_TRY(cudaGetLastError());
+    cudaFree(d);
+    return 0;
+}
+
+int debwt_index_locate(debwt_ctx* c, const char* patterns, const uint64_t* offsets, uint64_t n_patterns, uint64_t* hit_offsets,
+                       uint64_t* positions, uint64_t positions_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !hit_offsets || (n_patterns && !patterns)) FAIL("null argument");
+    hit_offsets[0] = 0;
+    if (n_patterns == 0) return 0;
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t st = c->st;
+    const u64 m = n_patterns, bytes = offsets[m], nb = (m + TPB - 1) / TPB;
+    // one block: patterns | offsets (m + 1) | sp (m) | counts (m) | hit offsets (m + 1) | block totals (nb) | their scan (nb + 1)
+    const u64 words = (bytes + 16 + 7) / 8;
+    u64* d = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d), (words + 4 * m + 2 * nb + 3) * 8));
+    u8* d_p = reinterpret_cast<u8*>(d);
+    u64 *d_o = d + words, *d_sp = d_o + m + 1, *d_cnt = d_sp + m, *d_hit = d_cnt + m, *d_tot = d_hit + m + 1, *d_base = d_tot + nb;
+    CUDA_TRY(cudaMemcpyAsync(d_p, patterns, bytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_o, offsets, (m + 1) * 8, cudaMemcpyHostToDevice, st));
+    const FmView f = view_of(c);
+    fm_range_kernel<<<grid_for(m), TPB, 0, st>>>(f, d_p, d_o, m, d_sp, d_cnt);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_base, d_hit);
+    DEBWT_COUNT(4);
+    CUDA_TRY(cudaMemcpyAsync(hit_offsets, d_hit, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    const u64 total = hit_offsets[m];
+    if (!positions || total == 0) { cudaFree(d); return 0; }                  // size query
+    if (total > positions_cap) {
+        cudaFree(d);
+        FAIL("index_locate: the patterns have " + std::to_string(total) + " hits; positions holds " + std::to_string(positions_cap));
+    }
+    u64* d_pos = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_pos), total * 8) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d);
+        FAIL("index_locate: out of device memory for " + std::to_string(total) + " hits");
+    }
+    locate_kernel<<<grid_for(total), TPB, 0, st>>>(f, sa_view_of(c), d_hit, d_sp, m, total, d_pos);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(positions, d_pos, total * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    cudaFree(d); cudaFree(d_pos);
+    return 0;
 }
 
 }  // extern "C"

@@ -162,8 +162,36 @@ int debwt_index_sizes(const debwt_ctx* ctx, uint64_t* occ_rows);
 /* occ: occ_rows * 4 u64 (may be NULL); c_array: 6 u64 = first row of the suffixes starting with A, C, G, T, '#', '$' */
 int debwt_index_copy(debwt_ctx* ctx, uint64_t* occ, uint64_t* c_array);
 /* Backward search (count only) of n_patterns ACGT strings on the device; pattern i = patterns[offsets[i] .. offsets[i+1]).
-   Uses occ / C the way findSeg does (src/LFsearch.c:167-235). */
+   Uses occ / C the way findSeg does (src/LFsearch.c:167-235).  A pattern with a symbol other than A, C, G, T (either case)
+   counts 0. */
 int debwt_index_count(debwt_ctx* ctx, const char* patterns, const uint64_t* offsets, uint64_t n_patterns, uint64_t* counts);
+/* Loads a finished result into the context in place of a build: the reference's three outputs (bwt_words: ceil(N/32) u64
+   as debwt_result_copy writes them; sharp_rows: n_sharp rows holding '#', any order; dollar_row), in host memory.  The files
+   do not determine N, so the caller passes it.  Use it to query a result of the sharded build (debwt_build_multi,
+   debwt_shard_*), of host/deBWT or of the reference.  Resets the input like debwt_set_*; afterwards debwt_result_*,
+   debwt_index_* and debwt_verify_text* work as after debwt_build, and debwt_build fails until a new input is set.  Checks
+   dollar_row < N and that the '#' rows are distinct, below N and not the '$' row; then every other row holds a base, so
+   the base counts plus n_sharp + 1 add up to N.  Whether the array is a BWT at all is found by debwt_index_sample_sa.
+   Held in the context's arena (N/4 bytes) until the next input or result. */
+int debwt_set_result(debwt_ctx* ctx, const uint64_t* bwt_words, uint64_t n_symbols, const uint64_t* sharp_rows, uint64_t n_sharp,
+                     uint64_t dollar_row);
+/* Sampled suffix array (locate support; the reference has none): ranks the LF walk like the verifier (16 bytes of scratch
+   HBM per symbol, freed on return; N < 2^32 - 1) and keeps SA[r] for every row whose text position is a multiple of
+   `rate` (a power of two, 1..1024): a u64 per 32 rows (sampled-row mask | sampled rows before) and ceil(N / rate) u32
+   values, i.e. N/4 + 4N/rate bytes of HBM.  Builds the occ / C tables first if needed.  Fails, keeping no samples, when the
+   result is not a BWT (its LF mapping is not one N-cycle).  Kept until the next build / input / set_result or the next
+   call.  *ms_out (optional) = device time. */
+int debwt_index_sample_sa(debwt_ctx* ctx, uint32_t rate, float* ms_out);
+/* positions[i] = SA[rows[i]], the text position of the suffix in row rows[i] (at most rate - 1 LF steps per row on the
+   device).  Every row must be < N; otherwise nothing is written. */
+int debwt_index_sa(debwt_ctx* ctx, const uint64_t* rows, uint64_t n_rows, uint64_t* positions);
+/* Locate: backward search of every pattern (as debwt_index_count; A, C, G, T in either case, so a pattern with any other
+   symbol has no hits and the empty pattern has N: every suffix), then the text positions of all hits in SA order:
+   positions[hit_offsets[i] + j] = SA[sp_i + j] for the rows [sp_i, sp_i + count_i) of pattern i.  hit_offsets[n_patterns + 1]
+   is always written (hit_offsets[i + 1] - hit_offsets[i] = count_i); positions == NULL is a size query; more hits than
+   positions_cap fails and names the number needed.  Needs debwt_index_sample_sa. */
+int debwt_index_locate(debwt_ctx* ctx, const char* patterns, const uint64_t* offsets, uint64_t n_patterns, uint64_t* hit_offsets,
+                       uint64_t* positions, uint64_t positions_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
