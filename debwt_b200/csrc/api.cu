@@ -139,7 +139,11 @@ __global__ void splitmix_fill_kernel(u64* keys, u64 n, u64 seed) {
 template <typename T>
 int check_seps(const T* seps, u64 n_rec, u64 n) {
     if (n_rec == 0) FAIL("no records");
-    if (n >= (1ull << 32) - 64) FAIL("text too long for one device in this build (n_symbols must be < 2^32 - 64)");
+    // the sort takes at most 2^32 - 65537 keys (radix_sort_u64) and there are N - 32 R of them: refuse such a text here,
+    // before anything is allocated, rather than in K3 with a message about keys
+    if (n >= (1ull << 32) - 64 || (n > 32 * n_rec && n - 32 * n_rec >= (1ull << 32) - (1ull << 16)))
+        FAIL("text too long for one device: N = " + std::to_string(n) + " symbols in R = " + std::to_string(n_rec) +
+             " records; one device takes N < 2^32 - 64 and N - 32 R < 2^32 - 65536 (so N <= 2^32 - 65505 for one record)");
     u64 start = 0;
     for (u64 r = 0; r < n_rec; ++r) {
         if (seps[r] < start || seps[r] - start <= 32) FAIL("Length <= 32!");      // src/collect#$.c:41-45
@@ -164,6 +168,8 @@ void reset_input(debwt_ctx* c) {
     c->d_dollar = nullptr;
     c->built = false;
     c->loaded = false;
+    c->n = 0;                            // a refused input leaves no input behind: debwt_build then says so
+    c->n_rec = 0;
     c->stats = debwt_stats{};
 }
 
@@ -303,10 +309,10 @@ int debwt_build(debwt_ctx* c, int k) {
     if (!c) FAIL("null context");
     if (k < 12 || k > 32) FAIL("-k: k-mer length (from 12 to 32, default 32)");      // src/main.c:45-46
     if (c->loaded) FAIL("the context holds a loaded result (debwt_set_result), not an input: set an input before building");
+    if (c->ing.active) FAIL("streaming input is still open: call debwt_ingest_end first");
     if (c->n == 0) FAIL("no input set");
     if (bind_device(c->device)) return -1;
     const u8* ascii = c->d_ascii_ext ? c->d_ascii_ext : c->d_ascii;
-    if (c->ing.active) FAIL("streaming input is still open: call debwt_ingest_end first");
     if (!ascii && !c->d_packed) FAIL("input was consumed by a previous build; set it again");
     cudaStream_t st = c->st;
     DevPool& pool = c->pool;

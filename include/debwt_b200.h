@@ -81,7 +81,10 @@ int debwt_set_ambiguity_policy(debwt_ctx* ctx, int resolve, uint64_t seed);
 /* ---- input: replaces collect()'s FASTA pass, src/collect#$.c:27-90 ---------------------------- */
 /* Host records: `seqs[i]` points at `lens[i]` bases (ACGT, either case; no terminator needed).
    Every record must be longer than 32 bp (src/collect#$.c:41-45) and contain only ACGT.
-   The text T = S1 # S2 # ... Sn $ is assembled on the device (H2D copy happens here). */
+   The text T = S1 # S2 # ... Sn $ is assembled on the device (H2D copy happens here).
+   Size limit of one device, checked by every input call (debwt_set_*, debwt_ingest_end) before anything is allocated:
+   N < 2^32 - 64 symbols and N - 32 R < 2^32 - 65536 k-mer keys for R records, i.e. N <= min(2^32 - 65537 + 32 R,
+   2^32 - 65); for one record N <= 2^32 - 65505.  Larger texts take the multi-GPU path. */
 int debwt_set_records(debwt_ctx* ctx, const char* const* seqs, const uint64_t* lens, uint64_t n_records);
 /* Same, from one host buffer that already holds T as ASCII ('#' between records, '$' last).
    `seps[i]` = offset of the i-th separator (ascending; the last one is n_symbols-1). */
