@@ -21,7 +21,6 @@
 #include "stages.cuh"
 #include "special.cuh"
 #include "ctx.cuh"
-#include "dist_kernels.cuh"
 
 namespace debwt {
 
@@ -342,7 +341,7 @@ int debwt_build(debwt_ctx* c, int k) {
         CUDA_TRY(cudaMemsetAsync(d_err, 0, 16, st));
         PackPolicy pol;
         pol.resolve = c->resolve_ambiguous; pol.seed = c->ambiguity_seed;
-        if (k_pack(ascii, n, d_text, d_err, st, pol)) return -1;
+        if (k_pack_words(ascii, n, d_text, text_words(n), d_err, st, pol)) return -1;
         if (c->d_ascii) { pool.adopt(c->d_ascii, n + 64); c->d_ascii = nullptr; }
     }
     mark();                                                                     // ev1
@@ -474,7 +473,7 @@ int debwt_build(debwt_ctx* c, int k) {
     if (group_by_sort) {
         if (k_flag_positions_keys(d_text, n, d_seps, R, bt, id_shift, d_mo, d_bka, d_bcount, st)) return -1;
     } else if (k_flag_positions(d_text, n, d_seps, R, bt, d_mo, d_blue, st)) return -1;
-    if (k_patch_bits(d_mo, d_emit, h_emit_pos.size(), st)) return -1;
+    if (k_patch_bits(d_mo, 0, n, d_emit, h_emit_pos.size(), st)) return -1;
     if (scan_exclusive_u32(d_mo, d_wp, nbw, true, d_scanws, d_tot, st)) return -1;
     u64 n_codes = 0, n_appended = 0;
     CUDA_TRY(cudaMemcpyAsync(&n_codes, d_tot, 8, cudaMemcpyDeviceToHost, st));
@@ -487,8 +486,8 @@ int debwt_build(debwt_ctx* c, int k) {
     if (dalloc(pool, &d_codes, ncw) || dalloc(pool, &d_sep, ncw + 1)) return -1;
     CUDA_TRY(cudaMemsetAsync(d_codes, 0, ncw * 8, st));
     CUDA_TRY(cudaMemsetAsync(d_sep, 0, (ncw + 1) * 4, st));
-    if (k_emit_codes(d_text, n, d_mo, d_wp, d_codes, st)) return -1;
-    if (k_mark_sep_codes(d_mo, d_wp, d_tail, R, d_sep, d_tail_idx, st)) return -1;
+    if (k_emit_codes(d_text, 0, nbw, d_mo, d_wp, 0, d_codes, st)) return -1;
+    if (k_mark_sep_codes(d_mo, d_wp, 0, n, 0, d_tail, R, d_sep, d_tail_idx, st)) return -1;
     if (group_by_sort) {
         if (k_blue_keys_fix(d_bka, bt.n_blue, d_mo, d_wp, st)) return -1;
         SortWorkspace bws;
@@ -501,7 +500,7 @@ int debwt_build(debwt_ctx* c, int k) {
     } else if (bt.n_blue >= nbw / 4) {
         u64* d_mw = nullptr;
         if (dalloc(pool, &d_mw, nbw + 2) || k_blue_fix_interleaved(d_blue, bt.n_blue, d_mo, d_wp, nbw + 1, d_mw, st)) return -1;
-    } else if (k_blue_fix(d_blue, bt.n_blue, d_mo, d_wp, st)) return -1;
+    } else if (k_blue_fix(d_blue, bt.n_blue, d_mo, d_wp, 0, 0, st)) return -1;
     u64 dollar_index = 0;
     CUDA_TRY(cudaMemcpyAsync(&dollar_index, d_tail_idx + (R - 1), 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -537,8 +536,8 @@ int debwt_build(debwt_ctx* c, int k) {
         return -1;
     CUDA_TRY(cudaMemsetAsync(c->d_sharp_count, 0, 16, st));
     CUDA_TRY(cudaMemsetAsync(c->d_dollar, 0xff, 16, st));
-    if (k_fill_case2(d_gmask, nk, n, d_rows, nspec, c->d_bwt, st)) return -1;
-    if (k_emit_blue(d_blue, bt, d_ins, nspec, c->d_bwt, c->d_sharp, c->d_sharp_count, c->d_dollar, st)) return -1;
+    if (k_fill_case2(d_gmask, nk, 0, n, d_rows, nspec, 0, nbw, c->d_bwt, st)) return -1;
+    if (k_emit_blue(d_blue, bt, 0, d_ins, nspec, c->d_bwt, c->d_sharp, c->d_sharp_count, c->d_dollar, st)) return -1;
     if (k_emit_special(d_rows, d_chr, nspec, c->d_bwt, st)) return -1;
     mark();                                                                     // ev8
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -801,7 +800,7 @@ int debwt_k_pack(int device, const char* text, uint64_t n, uint64_t* words_out) 
     if (s.get(&d_a, n + 64) || s.get(&d_w, text_words(n)) || s.get(&d_e, 4)) return -1;
     CUDA_TRY(cudaMemcpyAsync(d_a, text, n, cudaMemcpyHostToDevice, s.st));
     CUDA_TRY(cudaMemsetAsync(d_e, 0, 16, s.st));
-    if (k_pack(d_a, n, d_w, d_e, s.st)) return -1;
+    if (k_pack_words(d_a, n, d_w, text_words(n), d_e, s.st)) return -1;
     u32 e = 0;
     CUDA_TRY(cudaMemcpyAsync(&e, d_e, 4, cudaMemcpyDeviceToHost, s.st));
     CUDA_TRY(cudaMemcpyAsync(words_out, d_w, ((n + 32 + 31) / 32) * 8, cudaMemcpyDeviceToHost, s.st));
@@ -820,7 +819,7 @@ int debwt_k_extract(int device, const char* text, uint64_t n, const uint64_t* se
     CUDA_TRY(cudaMemcpyAsync(d_a, text, n, cudaMemcpyHostToDevice, s.st));
     CUDA_TRY(cudaMemcpyAsync(d_s, seps, R * 8, cudaMemcpyHostToDevice, s.st));
     CUDA_TRY(cudaMemsetAsync(d_e, 0, 16, s.st));
-    if (k_pack(d_a, n, d_w, d_e, s.st) || k_extract(d_w, n, d_s, R, d_k, s.st)) return -1;
+    if (k_pack_words(d_a, n, d_w, text_words(n), d_e, s.st) || k_extract(d_w, n, d_s, R, d_k, s.st)) return -1;
     CUDA_TRY(cudaMemcpyAsync(keys_out, d_k, nk * 8, cudaMemcpyDeviceToHost, s.st));
     CUDA_TRY(cudaStreamSynchronize(s.st));
     return 0;
@@ -891,7 +890,7 @@ int debwt_k_group_masks(int device, const char* text, uint64_t n, const uint64_t
     CUDA_TRY(cudaMemsetAsync(d_e, 0, 16, s.st));
     CUDA_TRY(cudaMemsetAsync(d_g, 0, (nk + 2) * 2, s.st));
     u64* d_keys = nullptr;
-    if (k_pack(d_a, n, d_w, d_e, s.st) || k_extract(d_w, n, d_s, R, d_ka, s.st) ||
+    if (k_pack_words(d_a, n, d_w, text_words(n), d_e, s.st) || k_extract(d_w, n, d_s, R, d_ka, s.st) ||
         radix_sort_u64(d_ka, d_kb, nk, ws, s.st, &d_keys) || k_build_key_index(d_keys, nk, ki, s.st) ||
         k_mark_edges(d_keys, nk, ki, d_g, s.st) || k_mark_heads_tails(d_w, d_s, R, d_keys, nk, ki, d_g, s.st) ||
         k_propagate(d_keys, nk, d_g, s.st))

@@ -51,11 +51,6 @@ int debwt_dev_pack(const void* d_ascii, uint64_t n, void* d_words, uint64_t nwor
     return k_pack_words(P8(d_ascii), n, P64(d_words), nwords, P32(d_err), S(stream));
 }
 
-int debwt_dev_extract(const void* d_words, uint64_t pos_lo, uint64_t pos_hi, const void* d_seps, uint64_t n_rec,
-                      uint64_t idx_base, void* d_keys, void* stream) {
-    return k_extract_range(P64(d_words), pos_lo, pos_hi, P64(d_seps), n_rec, idx_base, P64(d_keys), S(stream));
-}
-
 int debwt_dev_extract_slice(const void* d_words, uint64_t n_symbols, uint64_t pos_lo, uint64_t pos_hi, const void* d_seps,
                             uint64_t n_rec, uint64_t idx_base, void* d_keys, void* stream) {
     return k_extract_slice(P64(d_words), n_symbols, pos_lo, pos_hi, P64(d_seps), n_rec, idx_base, P64(d_keys), S(stream));
@@ -267,7 +262,7 @@ int debwt_dev_flag_slice(const void* d_words, uint64_t pos_lo, uint64_t pos_hi, 
 
 int debwt_dev_patch_bits_slice(void* d_mo_bits, uint64_t pos_lo, uint64_t pos_hi, const void* d_positions, uint64_t m,
                                void* stream) {
-    return k_patch_bits_slice(P32(d_mo_bits), pos_lo, pos_hi, P64(d_positions), m, S(stream));
+    return k_patch_bits(P32(d_mo_bits), pos_lo, pos_hi, P64(d_positions), m, S(stream));
 }
 
 int debwt_dev_scan_popc(const void* d_mo_bits, void* d_word_prefix, uint64_t nbw, uint64_t* total, void* d_workspace,
@@ -285,19 +280,19 @@ int debwt_dev_scan_popc(const void* d_mo_bits, void* d_word_prefix, uint64_t nbw
 
 int debwt_dev_emit_codes_slice(const void* d_words, uint64_t word_lo, uint64_t nbw, const void* d_mo_bits,
                                const void* d_word_prefix, uint64_t code_base, void* d_codes, void* stream) {
-    return k_emit_codes_slice(P64(d_words), word_lo, nbw, P32(d_mo_bits), P32(d_word_prefix), code_base, P64(d_codes), S(stream));
+    return k_emit_codes(P64(d_words), word_lo, nbw, P32(d_mo_bits), P32(d_word_prefix), code_base, P64(d_codes), S(stream));
 }
 
 int debwt_dev_mark_sep_slice(const void* d_mo_bits, const void* d_word_prefix, uint64_t pos_lo, uint64_t pos_hi,
                              uint64_t code_base, const void* d_positions, uint64_t m, void* d_sep, void* d_out_idx,
                              void* stream) {
-    return k_mark_sep_slice(P32(d_mo_bits), P32(d_word_prefix), pos_lo, pos_hi, code_base, P64(d_positions), m, P32(d_sep),
+    return k_mark_sep_codes(P32(d_mo_bits), P32(d_word_prefix), pos_lo, pos_hi, code_base, P64(d_positions), m, P32(d_sep),
                             P64(d_out_idx), S(stream));
 }
 
 int debwt_dev_fix_records(void* d_rec_entry, uint64_t m, const void* d_mo_bits, const void* d_word_prefix, uint64_t pos_lo,
                           uint64_t code_base, void* stream) {
-    return k_fix_records(P64(d_rec_entry), m, P32(d_mo_bits), P32(d_word_prefix), pos_lo, code_base, S(stream));
+    return k_blue_fix(P64(d_rec_entry), m, P32(d_mo_bits), P32(d_word_prefix), pos_lo, code_base, S(stream));
 }
 
 int debwt_dev_scatter_blue(const void* d_rec_entry, const void* d_rec_local, uint64_t m, const void* d_kmer,
@@ -316,15 +311,15 @@ int debwt_dev_sort_blue(void* d_blue, const void* d_kmer, const void* d_blue_u32
 
 int debwt_dev_fill_range(const void* d_gmask, uint64_t n_keys, uint64_t key_base, uint64_t n_symbols,
                          const void* d_spec_rows, uint64_t m, uint64_t word_lo, uint64_t word_hi, void* d_bwt, void* stream) {
-    return k_fill_range(P16(d_gmask), n_keys, key_base, n_symbols, P64(d_spec_rows), m, word_lo, word_hi, P64(d_bwt), S(stream));
+    return k_fill_case2(P16(d_gmask), n_keys, key_base, n_symbols, P64(d_spec_rows), m, word_lo, word_hi, P64(d_bwt), S(stream));
 }
 
 int debwt_dev_emit_blue(const void* d_blue, const void* d_kmer, const void* d_head_u32, const void* d_blue_u32,
                         uint64_t n_branch, uint64_t n_blue, uint64_t key_base, const void* d_spec_ins, uint64_t m,
                         void* d_bwt, void* d_sharp_rows, void* d_sharp_count_u32, void* d_dollar_row, void* stream) {
     BranchTable bt = BT(d_kmer, d_head_u32, d_blue_u32, nullptr, nullptr, 0, n_branch, n_blue);
-    return k_emit_blue_base(P64(d_blue), bt, key_base, P64(d_spec_ins), m, P64(d_bwt), P64(d_sharp_rows),
-                            P32(d_sharp_count_u32), P64(d_dollar_row), S(stream));
+    return k_emit_blue(P64(d_blue), bt, key_base, P64(d_spec_ins), m, P64(d_bwt), P64(d_sharp_rows), P32(d_sharp_count_u32),
+                       P64(d_dollar_row), S(stream));
 }
 
 int debwt_dev_emit_special(const void* d_spec_rows, const void* d_spec_chr, uint64_t m, void* d_bwt, void* stream) {

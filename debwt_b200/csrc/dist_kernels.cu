@@ -1,13 +1,13 @@
-// Stages of the sharded (multi-GPU) path -- SURVEY.md section 8e / K12.
+// Stages that only the sharded (multi-GPU) build runs -- SURVEY.md section 8e / K12.
 //
 // The reference has no distributed code; this is new.  The text is split by position into G 32-aligned
 // slices, keys are range-partitioned by sampled splitters on k-mer boundaries and exchanged once
-// (all-to-all over NVLink, issued by the host through torch.distributed / NCCL), after which every
-// device owns a contiguous key range = a contiguous run of BWT rows.  These kernels are the slice- and
-// range-aware variants of the single-GPU stages plus the bucket-by-owner partition.
+// (all-to-all over NVLink), after which every device owns a contiguous key range = a contiguous run of
+// BWT rows.  This file holds the owner of an item, the bucket-by-owner partition and the peer-store
+// exchange, the in-edge queries that cross key ranges, the K9 flagging of a position slice against the
+// global branch table and the scatter of received blue entries into their segments.  The stages that
+// both builds run live in stages.cu and take the slice or key range as parameters.
 #include "dist_kernels.cuh"
-
-#include <cstdlib>
 
 #include "stages_dev.cuh"
 
@@ -17,18 +17,6 @@ namespace {
 
 constexpr int TPB = 256;
 inline unsigned grid_for(u64 work, int per_block) { return (unsigned)((work + per_block - 1) / per_block); }
-
-// ---- K2 on a position slice ----------------------------------------------------------------
-__global__ void __launch_bounds__(TPB) extract_range_kernel(const u64* __restrict__ words, u64 pos_lo, u64 pos_hi,
-                                                           const u64* __restrict__ seps, u64 n_rec, u64 idx_base,
-                                                           u64* __restrict__ keys) {
-    const u64 p = pos_lo + (u64)blockIdx.x * TPB + threadIdx.x;
-    if (p >= pos_hi) return;
-    const u64 r = record_of(seps, n_rec, p);
-    if (r >= n_rec) return;
-    if (p + KMER > seps[r]) return;
-    st_stream(keys + (p - (u64)KMER * r - idx_base), text_window32(words, p));
-}
 
 // ---- K12 bucket by owner ----------------------------------------------------------------------
 // owner of an item = number of splitters <= (item & mask); ~0 items are dropped (dest 255)
@@ -150,63 +138,18 @@ __global__ void __launch_bounds__(TPB) partition_scatter_kernel(const u64* __res
     }
 }
 
-// Fused bucket + exchange: same ordering logic as partition_scatter_kernel, but every destination has its
-// own base pointer -- the receive buffer of that rank, mapped into this process through CUDA IPC -- so
-// the keys cross NVLink as coalesced peer stores straight from the partition kernel; no staging buffer,
-// no separate all-to-all.  dst[d] already points at this rank's slot inside rank d's buffer.
+// Fused bucket + exchange: the ordering of partition_scatter_kernel, but every destination has its own base pointer --
+// the receive buffer of that rank, mapped into this process (CUDA IPC or peer access) -- so the keys cross NVLink as peer
+// stores straight from the partition kernel: no staging buffer in global memory, no separate all-to-all.  dst.ptr[d]
+// already points at this rank's slot inside rank d's buffer.
 struct PeerDst {
     u64* ptr[MAX_RANKS];
 };
 
-__global__ void __launch_bounds__(TPB) partition_scatter_p2p_kernel(const u64* __restrict__ a, OwnerFn owner, u64 n, u32 n_ranks,
-                                                                   u64* __restrict__ cursors, PeerDst dst) {
-    constexpr int NW = TPB / 32;
-    __shared__ u32 s_wcnt[NW][MAX_RANKS];
-    __shared__ u64 s_base[MAX_RANKS];
-    const u32 lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const u32 lt = lanemask_lt();
-    const u64 base = (u64)blockIdx.x * PART_TILE;
-    u8 dd[PART_ITEMS];
-    u32 mine = 0;
-#pragma unroll
-    for (int j = 0; j < PART_ITEMS; ++j) {
-        const u64 i = base + (u64)j * TPB + threadIdx.x;
-        const u32 d = i < n ? owner(a, i) : 255u;
-        dd[j] = (u8)d;
-        for (u32 g = 0; g < n_ranks; ++g) {
-            const u32 bal = __ballot_sync(0xffffffffu, d == g);
-            if (lane == g) mine += __popc(bal);
-        }
-    }
-    if (lane < MAX_RANKS) s_wcnt[warp][lane] = lane < n_ranks ? mine : 0;
-    __syncthreads();
-    if (threadIdx.x < n_ranks) {
-        u32 run = 0;
-        for (int w = 0; w < NW; ++w) { const u32 c = s_wcnt[w][threadIdx.x]; s_wcnt[w][threadIdx.x] = run; run += c; }
-        s_base[threadIdx.x] = run ? atomicAdd(&cursors[threadIdx.x], (u64)run) : 0;
-    }
-    __syncthreads();
-    u32 run = lane < n_ranks ? s_wcnt[warp][lane] : 0;
-#pragma unroll
-    for (int j = 0; j < PART_ITEMS; ++j) {
-        const u64 i = base + (u64)j * TPB + threadIdx.x;
-        const u32 d = dd[j];
-        u32 rank = 0, add = 0;
-        for (u32 g = 0; g < n_ranks; ++g) {
-            const u32 bal = __ballot_sync(0xffffffffu, d == g);
-            if (d == g) rank = __popc(bal & lt);
-            if (lane == g) add = __popc(bal);
-        }
-        const u32 start = __shfl_sync(0xffffffffu, run, d < n_ranks ? d : 0);
-        if (d < n_ranks) dst.ptr[d][s_base[d] + start + rank] = a[i];
-        run += add;
-    }
-}
-
-// Same exchange with the block's tile first reordered by destination in shared memory: consecutive threads then store
-// consecutive items of one destination's run, so every peer store of a warp is one contiguous 256-byte run instead of
-// G short ones (a 32-64 byte store per destination and warp row reached only a fifth of the NVLink bandwidth on the
-// 3.1 Gbp build; profiles/r01_c3_3p1gbp_8gpu.log).
+// The block's tile is first reordered by destination in shared memory: consecutive threads then store consecutive items
+// of one destination's run, so every peer store of a warp is one contiguous 256-byte run instead of G short ones (the
+// stores straight from registers, 32-64 bytes per destination and warp row, reached only a fifth of the NVLink bandwidth
+// on the 3.1 Gbp build; profiles/r01_c3_3p1gbp_8gpu.log).
 // Blocks visit the tiles in a strided order (tile = block * stride mod grid, stride coprime with the grid): when the
 // input is sorted -- the in-edge queries are -- consecutive tiles all go to the same owner, every rank walks the owners
 // in the same order, and all ranks would store into ONE rank's memory at a time (incast on a single NVLink port: the
@@ -344,71 +287,6 @@ __global__ void __launch_bounds__(TPB) flag_slice_kernel(const u64* __restrict__
     if (lane == 0) mo_bits[(p - pos_lo) >> 5] = bal;
 }
 
-__global__ void __launch_bounds__(TPB) patch_bits_slice_kernel(u32* __restrict__ mo_bits, u64 pos_lo, u64 pos_hi,
-                                                              const u64* __restrict__ pos, u64 m) {
-    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (t >= m) return;
-    const u64 p = pos[t];
-    if (p < pos_lo || p >= pos_hi) return;
-    atomicOr(mo_bits + ((p - pos_lo) >> 5), 1u << (p & 31));
-}
-
-__global__ void __launch_bounds__(TPB) emit_codes_slice_kernel(const u64* __restrict__ words, u64 word_lo, u64 nbw,
-                                                              const u32* __restrict__ mo_bits,
-                                                              const u32* __restrict__ word_prefix, u64 code_base,
-                                                              u64* __restrict__ sp_codes) {
-    const u64 wl = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (wl >= nbw) return;
-    u32 bits = mo_bits[wl];
-    if (!bits) return;
-    const u64 w = word_lo + wl;
-    const u64 w0 = words[w], w1 = words[w + 1];
-    u64 c = code_base + word_prefix[wl];
-    u64 acc = 0, acc_word = c >> 5;
-    while (bits) {
-        const int b = __ffs(bits) - 1;
-        bits &= bits - 1;
-        const u64 code = (b == 0) ? (w0 & 3ull) : ((w1 >> (2 * (32 - b))) & 3ull);
-        const u64 cw = c >> 5;
-        if (cw != acc_word) {
-            if (acc) atomicOr(sp_codes + acc_word, acc);
-            acc = 0; acc_word = cw;
-        }
-        acc |= code << (2 * (31 - (c & 31)));
-        ++c;
-    }
-    if (acc) atomicOr(sp_codes + acc_word, acc);
-}
-
-__device__ __forceinline__ u64 slice_sp_index(const u32* __restrict__ mo_bits, const u32* __restrict__ word_prefix,
-                                              u64 pos_lo, u64 code_base, u64 p) {
-    const u64 l = p - pos_lo;
-    return code_base + sp_index_of(mo_bits, word_prefix, l);
-}
-
-// separator codes of the tail positions that fall into this slice; index of each written to out_idx
-// (entries of other slices stay 0)
-__global__ void __launch_bounds__(TPB) mark_sep_slice_kernel(const u32* __restrict__ mo_bits, const u32* __restrict__ word_prefix,
-                                                            u64 pos_lo, u64 pos_hi, u64 code_base,
-                                                            const u64* __restrict__ pos, u64 m, u32* __restrict__ sp_sep,
-                                                            u64* __restrict__ out_idx) {
-    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (t >= m) return;
-    const u64 p = pos[t];
-    if (p < pos_lo || p >= pos_hi) { out_idx[t] = 0; return; }
-    const u64 c = slice_sp_index(mo_bits, word_prefix, pos_lo, code_base, p);
-    atomicOr(sp_sep + (c >> 5), 1u << (c & 31));
-    out_idx[t] = c;
-}
-
-__global__ void __launch_bounds__(TPB) fix_records_kernel(u64* __restrict__ rec_entry, u64 m, const u32* __restrict__ mo_bits,
-                                                         const u32* __restrict__ word_prefix, u64 pos_lo, u64 code_base) {
-    const u64 e = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (e >= m) return;
-    const u64 v = rec_entry[e];
-    rec_entry[e] = (slice_sp_index(mo_bits, word_prefix, pos_lo, code_base, v >> 4) << 4) | (v & 15ull);
-}
-
 __global__ void __launch_bounds__(TPB) scatter_blue_kernel(const u64* __restrict__ rec_entry, const u64* __restrict__ rec_local,
                                                           u64 m, BranchTable bt, u64* __restrict__ blue) {
     const u64 e = (u64)blockIdx.x * TPB + threadIdx.x;
@@ -416,43 +294,6 @@ __global__ void __launch_bounds__(TPB) scatter_blue_kernel(const u64* __restrict
     const u64 b = rec_local[e];
     const u32 slot = atomicAdd(bt.cursor + b, 1u);
     blue[(u64)bt.blue[b] + slot] = rec_entry[e];
-}
-
-// ---- K8 / K11 on a key range --------------------------------------------------------------------
-constexpr int FILL_WORDS_PER_WARP = 8;
-
-__global__ void __launch_bounds__(TPB) fill_range_kernel(const u16* __restrict__ gmask, u64 n_keys, u64 key_base, u64 n,
-                                                        const u64* __restrict__ spec_rows, u64 m, u64 word_lo, u64 word_hi,
-                                                        u64* __restrict__ bwt) {
-    __shared__ u64 s_lo, s_hi;
-    constexpr int WORDS_PER_BLOCK = (TPB / 32) * FILL_WORDS_PER_WARP;
-    const u64 wblock = word_lo + (u64)blockIdx.x * WORDS_PER_BLOCK;
-    if (threadIdx.x == 0) {
-        s_lo = lower_bound_u64(spec_rows, 0, m, wblock * 32);
-        s_hi = lower_bound_u64(spec_rows, 0, m, (wblock + WORDS_PER_BLOCK) * 32);
-    }
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const u64 lo = s_lo, hi = s_hi;
-#pragma unroll
-    for (int q = 0; q < FILL_WORDS_PER_WARP; ++q) {
-        const u64 w = wblock + (u64)warp * FILL_WORDS_PER_WARP + q;
-        if (w >= word_hi) break;
-        const u64 row = w * 32 + lane;
-        u32 code = 0;
-        if (row < n) {
-            const u64 t = lower_bound_u64(spec_rows, lo, hi, row);
-            const bool special = t < m && spec_rows[t] == row;
-            const u64 i = row - t;                                   // global sorted-key index
-            if (!special && i >= key_base && i - key_base < n_keys) {
-                const u32 mk = gmask[i - key_base];
-                if (!gm_multi_in(mk) && (mk & 15u)) code = (u32)__ffs(mk & 15u) - 1u;
-            }
-        }
-        const u32 hi32 = __reduce_or_sync(0xffffffffu, lane < 16 ? code << (2 * (15 - lane)) : 0u);
-        const u32 lo32 = __reduce_or_sync(0xffffffffu, lane >= 16 ? code << (2 * (31 - lane)) : 0u);
-        if (lane == 0) bwt[w] = ((u64)hi32 << 32) | lo32;
-    }
 }
 
 }  // namespace
@@ -463,13 +304,6 @@ __global__ void __launch_bounds__(TPB) fill_range_kernel(const u16* __restrict__
         CUDA_TRY(cudaGetLastError());    \
         return 0;                        \
     } while (0)
-
-int k_extract_range(const u64* words, u64 pos_lo, u64 pos_hi, const u64* d_seps, u64 n_rec, u64 idx_base, u64* keys,
-                    cudaStream_t st) {
-    if (pos_hi <= pos_lo) return 0;
-    extract_range_kernel<<<grid_for(pos_hi - pos_lo, TPB), TPB, 0, st>>>(words, pos_lo, pos_hi, d_seps, n_rec, idx_base, keys);
-    LAUNCHED(1);
-}
 
 int k_owner_of_keys(const u64* items, u64 n, const u64* d_splitters, u32 n_split, u64 mask, bool drop_marker, u8* dest,
                     cudaStream_t st) {
@@ -511,16 +345,12 @@ int k_partition_scatter_p2p(const u64* a, const PartitionBy& by, u64 n, u32 n_ra
     if (n == 0) return 0;
     PeerDst pd;
     for (u32 r = 0; r < MAX_RANKS; ++r) pd.ptr[r] = r < n_ranks ? dst[r] : nullptr;
-    static const bool direct = getenv("DEBWT_P2P_DIRECT") != nullptr;      // the unstaged variant, kept for comparison
-    if (direct) partition_scatter_p2p_kernel<<<grid_for(n, PART_TILE), TPB, 0, st>>>(a, make_owner(by), n, n_ranks, d_cursors, pd);
-    else {
-        const unsigned grid = grid_for(n, PART_TILE);
-        auto gcd = [](unsigned x, unsigned y) { while (y) { const unsigned t = x % y; x = y; y = t; } return x; };
-        unsigned stride = (unsigned)(grid * 0.6180339887) | 1u;            // golden-ratio stride: neighbours in time are far apart in the input
-        while (stride > 1 && gcd(stride, grid) != 1) stride -= 2;
-        if (grid < 8) stride = 1;
-        partition_scatter_p2p_staged_kernel<<<grid, TPB, 0, st>>>(a, make_owner(by), n, n_ranks, d_cursors, pd, stride);
-    }
+    const unsigned grid = grid_for(n, PART_TILE);
+    auto gcd = [](unsigned x, unsigned y) { while (y) { const unsigned t = x % y; x = y; y = t; } return x; };
+    unsigned stride = (unsigned)(grid * 0.6180339887) | 1u;                // golden-ratio stride: neighbours in time are far apart in the input
+    while (stride > 1 && gcd(stride, grid) != 1) stride -= 2;
+    if (grid < 8) stride = 1;
+    partition_scatter_p2p_staged_kernel<<<grid, TPB, 0, st>>>(a, make_owner(by), n, n_ranks, d_cursors, pd, stride);
     LAUNCHED(1);
 }
 
@@ -545,46 +375,9 @@ int k_flag_slice(const u64* words, u64 pos_lo, u64 pos_hi, const u64* d_seps, u6
     LAUNCHED(1);
 }
 
-int k_patch_bits_slice(u32* mo_bits, u64 pos_lo, u64 pos_hi, const u64* positions, u64 m, cudaStream_t st) {
-    if (m == 0) return 0;
-    patch_bits_slice_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, pos_lo, pos_hi, positions, m);
-    LAUNCHED(1);
-}
-
-int k_emit_codes_slice(const u64* words, u64 word_lo, u64 nbw, const u32* mo_bits, const u32* word_prefix, u64 code_base,
-                       u64* sp_codes, cudaStream_t st) {
-    if (nbw == 0) return 0;
-    emit_codes_slice_kernel<<<grid_for(nbw, TPB), TPB, 0, st>>>(words, word_lo, nbw, mo_bits, word_prefix, code_base, sp_codes);
-    LAUNCHED(1);
-}
-
-int k_mark_sep_slice(const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 pos_hi, u64 code_base,
-                     const u64* positions, u64 m, u32* sp_sep, u64* out_idx, cudaStream_t st) {
-    if (m == 0) return 0;
-    mark_sep_slice_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, word_prefix, pos_lo, pos_hi, code_base, positions, m,
-                                                            sp_sep, out_idx);
-    LAUNCHED(1);
-}
-
-int k_fix_records(u64* rec_entry, u64 m, const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 code_base,
-                  cudaStream_t st) {
-    if (m == 0) return 0;
-    fix_records_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(rec_entry, m, mo_bits, word_prefix, pos_lo, code_base);
-    LAUNCHED(1);
-}
-
 int k_scatter_blue(const u64* rec_entry, const u64* rec_local, u64 m, BranchTable bt, u64* blue, cudaStream_t st) {
     if (m == 0) return 0;
     scatter_blue_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(rec_entry, rec_local, m, bt, blue);
-    LAUNCHED(1);
-}
-
-int k_fill_range(const u16* gmask, u64 n_keys, u64 key_base, u64 n, const u64* spec_rows, u64 m, u64 word_lo, u64 word_hi,
-                 u64* bwt, cudaStream_t st) {
-    if (word_hi <= word_lo) return 0;
-    constexpr int WORDS_PER_BLOCK = (TPB / 32) * FILL_WORDS_PER_WARP;
-    fill_range_kernel<<<grid_for(word_hi - word_lo, WORDS_PER_BLOCK), TPB, 0, st>>>(gmask, n_keys, key_base, n, spec_rows, m,
-                                                                                    word_lo, word_hi, bwt);
     LAUNCHED(1);
 }
 

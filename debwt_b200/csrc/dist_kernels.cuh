@@ -4,8 +4,6 @@
 
 namespace debwt {
 
-int k_extract_range(const u64* words, u64 pos_lo, u64 pos_hi, const u64* d_seps, u64 n_rec, u64 idx_base, u64* keys,
-                    cudaStream_t st);
 int k_owner_of_keys(const u64* items, u64 n, const u64* d_splitters, u32 n_split, u64 mask, bool drop_marker, u8* dest,
                     cudaStream_t st);
 int k_owner_of_index(u64* idx, u64 n, const u64* d_bases, u32 n_ranks, u8* dest, cudaStream_t st);
@@ -27,19 +25,6 @@ int k_out_edges_queries(const u64* sorted, u64 n, u16* gmask, u64* queries, cuda
 int k_apply_in_queries(const u64* sorted, u64 n, KeyIndex ki, u16* gmask, const u64* q, u64 m, cudaStream_t st);
 int k_flag_slice(const u64* words, u64 pos_lo, u64 pos_hi, const u64* d_seps, u64 n_rec, BranchTable bt, u32* mo_bits,
                  u64* rec_entry, u64* rec_index, u64* d_rec_count, cudaStream_t st);
-int k_patch_bits_slice(u32* mo_bits, u64 pos_lo, u64 pos_hi, const u64* positions, u64 m, cudaStream_t st);
-int k_emit_codes_slice(const u64* words, u64 word_lo, u64 nbw, const u32* mo_bits, const u32* word_prefix, u64 code_base,
-                       u64* sp_codes, cudaStream_t st);
-int k_mark_sep_slice(const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 pos_hi, u64 code_base,
-                     const u64* positions, u64 m, u32* sp_sep, u64* out_idx, cudaStream_t st);
-int k_fix_records(u64* rec_entry, u64 m, const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 code_base,
-                  cudaStream_t st);
 int k_scatter_blue(const u64* rec_entry, const u64* rec_local, u64 m, BranchTable bt, u64* blue, cudaStream_t st);
-int k_fill_range(const u16* gmask, u64 n_keys, u64 key_base, u64 n, const u64* spec_rows, u64 m, u64 word_lo, u64 word_hi,
-                 u64* bwt, cudaStream_t st);
-int k_emit_blue_base(const u64* blue, BranchTable bt, u64 key_base, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
-                     u32* d_sharp_count, u64* dollar_row, cudaStream_t st);
-// K1 on a slice: packs n symbols into nwords words (T padding for [n, n+32), zeros beyond)
-int k_pack_words(const u8* ascii, u64 n, u64* words, u64 nwords, u32* d_err, cudaStream_t st, PackPolicy pol = PackPolicy());
 
 }  // namespace debwt

@@ -537,7 +537,7 @@ int shard_build_impl(debwt_shard* s, const void* slice, int slice_on_device, u64
     SCUDA(cudaMemsetAsync(mo, 0, (wp + 2) * 4, st));
     SCUDA(cudaMemsetAsync(d_small, 0, 64 * 8, st));
     if (k_flag_slice(W, pos_lo, pos_hi, d_seps, R, gbt, mo, rec_entry, rec_index, d_small, st)) return -1;
-    if (k_patch_bits_slice(mo, pos_lo, pos_hi_al, d_emit, h_emit_pos.size(), st)) return -1;
+    if (k_patch_bits(mo, pos_lo, pos_hi_al, d_emit, h_emit_pos.size(), st)) return -1;
     if (scan_exclusive_u32(mo, wpfx, wp, true, scanws, d_small + 1, st)) return -1;
     u64 h_cnt[2] = {0, 0};
     SCUDA(cudaMemcpyAsync(h_cnt, d_small, 16, cudaMemcpyDeviceToHost, st));
@@ -556,8 +556,8 @@ int shard_build_impl(debwt_shard* s, const void* slice, int slice_on_device, u64
     u32* sep = reinterpret_cast<u32*>(sh + off_sep);
     u64* tail_idx = reinterpret_cast<u64*>(sh + off_tail);
     SCUDA(cudaMemsetAsync(sh, 0, off_tail + R * 8, st));
-    if (k_emit_codes_slice(W, (u64)me * wp, wp, mo, wpfx, code_base, codes, st)) return -1;
-    if (k_mark_sep_slice(mo, wpfx, pos_lo, pos_hi_al, code_base, d_tail, R, sep, tail_idx, st)) return -1;
+    if (k_emit_codes(W, (u64)me * wp, wp, mo, wpfx, code_base, codes, st)) return -1;
+    if (k_mark_sep_codes(mo, wpfx, pos_lo, pos_hi_al, code_base, d_tail, R, sep, tail_idx, st)) return -1;
     if (G > 1) {
         if (sync_all(s)) return -1;                    // every rank's share is written
         u64 base_p = 0;
@@ -583,7 +583,7 @@ int shard_build_impl(debwt_shard* s, const void* slice, int slice_on_device, u64
         if (sync_all(s)) return -1;
     }
     SCUDA(cudaMemcpyAsync(&dollar_index, tail_idx + (R - 1), 8, cudaMemcpyDeviceToHost, st));
-    if (k_fix_records(rec_entry, m_rec, mo, wpfx, pos_lo, code_base, st)) return -1;
+    if (k_blue_fix(rec_entry, m_rec, mo, wpfx, pos_lo, code_base, st)) return -1;
     SCUDA(cudaStreamSynchronize(st));
     pc.tick("codes");
     SCUDA(cudaEventRecord(s->ev[7], st));
@@ -672,12 +672,12 @@ int shard_build_impl(debwt_shard* s, const void* slice, int slice_on_device, u64
     SCUDA(cudaMemsetAsync(d_dollar, 0xff, 16, st));
     u64* bwt_v = seg - w_lo;                           // the emit kernels index with global word numbers
     if (my_hi > my_lo) {
-        if (n_loc && k_fill_range(gmask, n_loc, key_base, N, d_rows, nspec, w_lo, w_hi, bwt_v, st)) return -1;
+        if (n_loc && k_fill_case2(gmask, n_loc, key_base, N, d_rows, nspec, w_lo, w_hi, bwt_v, st)) return -1;
         const u64 t_lo = (u64)(std::lower_bound(h_rows.begin(), h_rows.end(), my_lo) - h_rows.begin());
         const u64 t_hi = (u64)(std::lower_bound(h_rows.begin(), h_rows.end(), my_hi) - h_rows.begin());
         if (t_hi > t_lo && k_emit_special(d_rows + t_lo, d_chr + t_lo, t_hi - t_lo, bwt_v, st)) return -1;
     }
-    if (k_emit_blue_base(blue, bt, key_base, d_ins, nspec, bwt_v, d_sharp, d_scnt, d_dollar, st)) return -1;
+    if (k_emit_blue(blue, bt, key_base, d_ins, nspec, bwt_v, d_sharp, d_scnt, d_dollar, st)) return -1;
     if (G > 1) {
         if (sync_all(s)) return -1;                    // rank 0's result buffer is zeroed
     }

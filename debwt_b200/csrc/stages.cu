@@ -5,7 +5,6 @@
 #include <cstdlib>
 #include "special.cuh"
 #include "stages_dev.cuh"
-#include "dist_kernels.cuh"
 
 namespace debwt {
 
@@ -281,14 +280,6 @@ __global__ void __launch_bounds__(TPB) rle_write_kernel(const u64* __restrict__ 
 }
 
 }  // namespace
-
-int k_pack(const u8* ascii, u64 n, u64* words, u32* d_err, cudaStream_t st, PackPolicy pol) {
-    const u64 nw = text_words(n);
-    pack_kernel<<<grid_for(nw, TPB), TPB, 0, st>>>(ascii, n, words, nw, d_err, pol);
-    DEBWT_COUNT(1);
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-}
 
 int k_pack_words(const u8* ascii, u64 n, u64* words, u64 nwords, u32* d_err, cudaStream_t st, PackPolicy pol) {
     if (nwords == 0) return 0;
@@ -1223,21 +1214,27 @@ __global__ void __launch_bounds__(TPB) blue_keys_strip_kernel(u64* __restrict__ 
     if (e < m) bkeys[e] &= 0xFFFFFFFF7ull;
 }
 
-__global__ void __launch_bounds__(TPB) patch_bits_kernel(u32* __restrict__ mo_bits, const u64* __restrict__ pos, u64 m) {
+// patch_bits, emit_codes, mark_sep_codes and blue_fix see one position slice with codes from code_base (stages.cuh).
+__global__ void __launch_bounds__(TPB) patch_bits_kernel(u32* __restrict__ mo_bits, u64 pos_lo, u64 pos_hi,
+                                                        const u64* __restrict__ pos, u64 m) {
     const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (t < m) atomicOr(mo_bits + (pos[t] >> 5), 1u << (pos[t] & 31));
+    if (t >= m) return;
+    const u64 p = pos[t];
+    if (p < pos_lo || p >= pos_hi) return;
+    atomicOr(mo_bits + ((p - pos_lo) >> 5), 1u << (p & 31));
 }
 
-__global__ void __launch_bounds__(TPB) emit_codes_kernel(const u64* __restrict__ words, u64 nbw,
+__global__ void __launch_bounds__(TPB) emit_codes_kernel(const u64* __restrict__ words, u64 word_lo, u64 nbw,
                                                         const u32* __restrict__ mo_bits, const u32* __restrict__ word_prefix,
-                                                        u64* __restrict__ sp_codes) {
-    const u64 w = (u64)blockIdx.x * TPB + threadIdx.x;
-    if (w >= nbw) return;
-    u32 bits = mo_bits[w];
+                                                        u64 code_base, u64* __restrict__ sp_codes) {
+    const u64 wl = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (wl >= nbw) return;
+    u32 bits = mo_bits[wl];
     if (!bits) return;
     // next symbols of positions 32w+b are text positions 32w+31+b: last symbol of word w, then word w+1
+    const u64 w = word_lo + wl;
     const u64 w0 = words[w], w1 = words[w + 1];
-    u64 c = word_prefix[w];
+    u64 c = code_base + word_prefix[wl];
     u64 acc = 0, acc_word = c >> 5;
     while (bits) {
         const int b = __ffs(bits) - 1;
@@ -1254,22 +1251,27 @@ __global__ void __launch_bounds__(TPB) emit_codes_kernel(const u64* __restrict__
     if (acc) atomicOr(sp_codes + acc_word, acc);
 }
 
+// separator codes of the tail positions that fall into the slice; index of each written to out_idx (entries of other
+// slices get 0)
 __global__ void __launch_bounds__(TPB) mark_sep_codes_kernel(const u32* __restrict__ mo_bits, const u32* __restrict__ word_prefix,
+                                                            u64 pos_lo, u64 pos_hi, u64 code_base,
                                                             const u64* __restrict__ pos, u64 m, u32* __restrict__ sp_sep,
                                                             u64* __restrict__ out_idx) {
     const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
     if (t >= m) return;
-    const u64 c = sp_index_of(mo_bits, word_prefix, pos[t]);
+    const u64 p = pos[t];
+    if (p < pos_lo || p >= pos_hi) { out_idx[t] = 0; return; }
+    const u64 c = code_base + sp_index_of(mo_bits, word_prefix, p - pos_lo);
     atomicOr(sp_sep + (c >> 5), 1u << (c & 31));
     out_idx[t] = c;
 }
 
 __global__ void __launch_bounds__(TPB) blue_fix_kernel(u64* __restrict__ blue, u64 m, const u32* __restrict__ mo_bits,
-                                                      const u32* __restrict__ word_prefix) {
+                                                      const u32* __restrict__ word_prefix, u64 pos_lo, u64 code_base) {
     const u64 e = (u64)blockIdx.x * TPB + threadIdx.x;
     if (e >= m) return;
     const u64 v = blue[e];
-    blue[e] = (sp_index_of(mo_bits, word_prefix, v >> 4) << 4) | (v & 15ull);
+    blue[e] = ((code_base + sp_index_of(mo_bits, word_prefix, (v >> 4) - pos_lo)) << 4) | (v & 15ull);
 }
 
 // The entries sit in their segments, i.e. in no order of position: every one of them reads the bitmap word and the prefix
@@ -1326,26 +1328,28 @@ int k_blue_keys_strip(u64* bkeys, u64 m, cudaStream_t st) {
     return 0;
 }
 
-int k_patch_bits(u32* mo_bits, const u64* positions, u64 m, cudaStream_t st) {
+int k_patch_bits(u32* mo_bits, u64 pos_lo, u64 pos_hi, const u64* positions, u64 m, cudaStream_t st) {
     if (m == 0) return 0;
-    patch_bits_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, positions, m);
+    patch_bits_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, pos_lo, pos_hi, positions, m);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
-int k_emit_codes(const u64* words, u64 n, const u32* mo_bits, const u32* word_prefix, u64* sp_codes, cudaStream_t st) {
-    const u64 nbw = (n + 31) / 32;
-    emit_codes_kernel<<<grid_for(nbw, TPB), TPB, 0, st>>>(words, nbw, mo_bits, word_prefix, sp_codes);
+int k_emit_codes(const u64* words, u64 word_lo, u64 nbw, const u32* mo_bits, const u32* word_prefix, u64 code_base,
+                 u64* sp_codes, cudaStream_t st) {
+    if (nbw == 0) return 0;
+    emit_codes_kernel<<<grid_for(nbw, TPB), TPB, 0, st>>>(words, word_lo, nbw, mo_bits, word_prefix, code_base, sp_codes);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
-int k_mark_sep_codes(const u32* mo_bits, const u32* word_prefix, const u64* positions, u64 m, u32* sp_sep,
-                     u64* d_code_index_out, cudaStream_t st) {
+int k_mark_sep_codes(const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 pos_hi, u64 code_base, const u64* positions,
+                     u64 m, u32* sp_sep, u64* d_code_index_out, cudaStream_t st) {
     if (m == 0) return 0;
-    mark_sep_codes_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, word_prefix, positions, m, sp_sep, d_code_index_out);
+    mark_sep_codes_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(mo_bits, word_prefix, pos_lo, pos_hi, code_base, positions, m, sp_sep,
+                                                            d_code_index_out);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1360,9 +1364,9 @@ int k_blue_fix_interleaved(u64* blue, u64 m, const u32* mo_bits, const u32* word
     return 0;
 }
 
-int k_blue_fix(u64* blue, u64 m, const u32* mo_bits, const u32* word_prefix, cudaStream_t st) {
+int k_blue_fix(u64* blue, u64 m, const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 code_base, cudaStream_t st) {
     if (m == 0) return 0;
-    blue_fix_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(blue, m, mo_bits, word_prefix);
+    blue_fix_kernel<<<grid_for(m, TPB), TPB, 0, st>>>(blue, m, mo_bits, word_prefix, pos_lo, code_base);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1375,12 +1379,13 @@ namespace {
 
 constexpr int FILL_WORDS_PER_WARP = 32;
 
-__global__ void __launch_bounds__(TPB) fill_case2_kernel(const u16* __restrict__ gmask, u64 n_keys, u64 n,
-                                                        const u64* __restrict__ spec_rows, u64 m, u64 nwords,
+// output words [word_lo, word_hi); gmask holds the n_keys sorted keys from global key index key_base on
+__global__ void __launch_bounds__(TPB) fill_case2_kernel(const u16* __restrict__ gmask, u64 n_keys, u64 key_base, u64 n,
+                                                        const u64* __restrict__ spec_rows, u64 m, u64 word_lo, u64 word_hi,
                                                         u64* __restrict__ bwt) {
     __shared__ u64 s_lo, s_hi;
     constexpr int WORDS_PER_BLOCK = (TPB / 32) * FILL_WORDS_PER_WARP;
-    const u64 wblock = (u64)blockIdx.x * WORDS_PER_BLOCK;
+    const u64 wblock = word_lo + (u64)blockIdx.x * WORDS_PER_BLOCK;
     if (threadIdx.x == 0) s_lo = lower_bound_u64(spec_rows, 0, m, wblock * 32);
     if (threadIdx.x == 32) s_hi = lower_bound_u64(spec_rows, 0, m, (wblock + WORDS_PER_BLOCK) * 32);
     __syncthreads();
@@ -1389,13 +1394,14 @@ __global__ void __launch_bounds__(TPB) fill_case2_kernel(const u16* __restrict__
 #pragma unroll 4
     for (int q = 0; q < FILL_WORDS_PER_WARP; ++q) {
         const u64 w = wblock + (u64)warp * FILL_WORDS_PER_WARP + q;
-        if (w >= nwords) break;                       // warp-uniform
+        if (w >= word_hi) break;                      // warp-uniform
         const u64 row = w * 32 + lane;
         u32 code = 0;
         if (row < n) {
             const u64 t = lower_bound_u64(spec_rows, lo, hi, row);   // special rows before this row
             const bool special = t < m && spec_rows[t] == row;
-            const u64 i = row - t;
+            // index into this device's keys; the rows of keys below key_base wrap around to values far above n_keys
+            const u64 i = row - t - key_base;
             if (!special && i < n_keys) {
                 const u32 mk = gmask[i];
                 if (!gm_multi_in(mk) && (mk & 15u)) code = (u32)__ffs(mk & 15u) - 1u;   // the single in-base (src/INandOut.c:367-395)
@@ -1462,28 +1468,25 @@ __global__ void __launch_bounds__(TPB) emit_special_kernel(const u64* __restrict
 
 }  // namespace
 
-int k_fill_case2(const u16* gmask, u64 n_keys, u64 n, const u64* spec_rows, u64 m, u64* bwt, cudaStream_t st) {
-    const u64 nwords = (n + 31) / 32;
+int k_fill_case2(const u16* gmask, u64 n_keys, u64 key_base, u64 n, const u64* spec_rows, u64 m, u64 word_lo, u64 word_hi,
+                 u64* bwt, cudaStream_t st) {
+    if (word_hi <= word_lo) return 0;
     constexpr int WORDS_PER_BLOCK = (TPB / 32) * FILL_WORDS_PER_WARP;
-    fill_case2_kernel<<<grid_for(nwords, WORDS_PER_BLOCK), TPB, 0, st>>>(gmask, n_keys, n, spec_rows, m, nwords, bwt);
+    fill_case2_kernel<<<grid_for(word_hi - word_lo, WORDS_PER_BLOCK), TPB, 0, st>>>(gmask, n_keys, key_base, n, spec_rows, m,
+                                                                                    word_lo, word_hi, bwt);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
-int k_emit_blue_base(const u64* blue, BranchTable bt, u64 key_base, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
-                     u32* d_sharp_count, u64* dollar_row, cudaStream_t st) {
+int k_emit_blue(const u64* blue, BranchTable bt, u64 key_base, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
+                u32* d_sharp_count, u64* dollar_row, cudaStream_t st) {
     if (bt.n_blue == 0) return 0;
     emit_blue_kernel<<<grid_for(bt.n_blue, EB_ITEMS * TPB), TPB, 0, st>>>(blue, bt, key_base, spec_ins, m, bwt, sharp_rows,
                                                                           d_sharp_count, dollar_row);
     DEBWT_COUNT(1);
     CUDA_TRY(cudaGetLastError());
     return 0;
-}
-
-int k_emit_blue(const u64* blue, BranchTable bt, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
-                u32* d_sharp_count, u64* dollar_row, cudaStream_t st) {
-    return k_emit_blue_base(blue, bt, 0, spec_ins, m, bwt, sharp_rows, d_sharp_count, dollar_row, st);
 }
 
 int k_emit_special(const u64* spec_rows, const u8* spec_chr, u64 m, u64* bwt, cudaStream_t st) {

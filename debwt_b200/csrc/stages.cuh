@@ -10,7 +10,7 @@ size_t scan_workspace_bytes(u64 m);
 int scan_exclusive_u32(const u32* in, u32* out, u64 m, bool popc, void* workspace, u64* d_total, cudaStream_t st);
 
 // ---- K1 / K2 ------------------------------------------------------------------------------
-// ascii: n bytes (bases, '#' between records, '$' last).  words: ceil((n+32)/32)+1 u64.
+// ascii: n bytes (bases, '#' between records, '$' last).  A whole text packs into text_words(n) u64.
 // what K1 does with a symbol that is not A, C, G or T: reject (default), or resolve IUPAC ambiguity codes to a seeded
 // pseudo-random compatible base (reference otherTool/transferN.c); pos_base = text position of ascii[0]
 struct PackPolicy {
@@ -18,8 +18,9 @@ struct PackPolicy {
     u64 seed = 0;
     u64 pos_base = 0;
 };
-int k_pack(const u8* ascii, u64 n, u64* words, u32* d_err, cudaStream_t st, PackPolicy pol = PackPolicy());
 inline u64 text_words(u64 n) { return (n + 32 + 31) / 32 + 1; }
+// packs n symbols into nwords words (T padding for [n, n+32), zeros beyond): a whole text, or the slice of one
+int k_pack_words(const u8* ascii, u64 n, u64* words, u64 nwords, u32* d_err, cudaStream_t st, PackPolicy pol = PackPolicy());
 // all in-record 32-mers; key index of window p in record r is p - 32 r.  keys: n - 32 R entries.
 int k_extract(const u64* words, u64 n, const u64* d_seps, u64 n_rec, u64* keys, cudaStream_t st);
 // the same for the positions [pos_lo, pos_hi) only (pos_lo a multiple of 32); key index = p - 32 r - idx_base
@@ -121,13 +122,20 @@ int k_blue_keys_strip(u64* bkeys, u64 m, cudaStream_t st);
 // blue entries: position -> spIndex (k_blue_fix), or the same through an interleaved copy of the bitmap and its prefix
 // (scratch: n_words u64, n_words = words of mo_bits) when there are enough entries to pay for the copy
 int k_blue_fix_interleaved(u64* blue, u64 m, const u32* mo_bits, const u32* word_prefix, u64 n_words, u64* scratch, cudaStream_t st);
-int k_patch_bits(u32* mo_bits, const u64* positions, u64 m, cudaStream_t st);
-// sp_codes: ceil(S/32)+3 u64 zeroed; codes packed 32 per word, code j at bits 2*(31-(j&31))
-int k_emit_codes(const u64* words, u64 n, const u32* mo_bits, const u32* word_prefix, u64* sp_codes, cudaStream_t st);
-// marks separator codes: sp_sep bit per code (u32 words, zeroed); positions = tail positions whose code is '#'/'$'
-int k_mark_sep_codes(const u32* mo_bits, const u32* word_prefix, const u64* positions, u64 m, u32* sp_sep,
-                     u64* d_code_index_out, cudaStream_t st);
-int k_blue_fix(u64* blue, u64 m, const u32* mo_bits, const u32* word_prefix, cudaStream_t st);
+// The calls below also serve the sharded build, which produces the codes of one position slice [pos_lo, pos_hi) (pos_lo a
+// multiple of 32, word_lo = pos_lo / 32) at global code indices from code_base: mo_bits and word_prefix cover the slice
+// only.  The single-GPU build passes pos_lo = word_lo = code_base = 0 and the whole text.
+// sets the bits of the positions inside the slice; the others are skipped
+int k_patch_bits(u32* mo_bits, u64 pos_lo, u64 pos_hi, const u64* positions, u64 m, cudaStream_t st);
+// sp_codes: ceil(S/32)+3 u64 zeroed; codes packed 32 per word, code j at bits 2*(31-(j&31)); nbw: words of the slice
+int k_emit_codes(const u64* words, u64 word_lo, u64 nbw, const u32* mo_bits, const u32* word_prefix, u64 code_base,
+                 u64* sp_codes, cudaStream_t st);
+// marks separator codes: sp_sep bit per code (u32 words, zeroed); positions = tail positions whose code is '#'/'$'.
+// d_code_index_out[t] = global code index of positions[t], or 0 for a position outside the slice
+int k_mark_sep_codes(const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 pos_hi, u64 code_base, const u64* positions,
+                     u64 m, u32* sp_sep, u64* d_code_index_out, cudaStream_t st);
+// every entry's position must lie in the slice
+int k_blue_fix(u64* blue, u64 m, const u32* mo_bits, const u32* word_prefix, u64 pos_lo, u64 code_base, cudaStream_t st);
 
 // ---- K10 segmented sort (bluesort.cu) ------------------------------------------------------
 struct SpView {
@@ -143,10 +151,14 @@ struct SpView {
 int k_sort_blue(u64* blue, BranchTable bt, SpView sp, u32* d_work /* >= 4 B + 16 u32 */, cudaStream_t st);
 
 // ---- K8 / K11 emission ---------------------------------------------------------------------
-// bwt: ceil(n/32) words.  spec_rows: m ascending rows of the special suffixes.
-int k_fill_case2(const u16* gmask, u64 n_keys, u64 n, const u64* spec_rows, u64 m, u64* bwt, cudaStream_t st);
-// scatter sorted blue symbols; '#'/'$' rows appended to sharp_rows (unordered) / dollar_row
-int k_emit_blue(const u64* blue, BranchTable bt, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
+// bwt: ceil(n/32) words, indexed by global word number.  spec_rows: m ascending rows of the special suffixes.
+// A device that owns the sorted keys [key_base, key_base + n_keys) (gmask: their masks) writes the words [word_lo, word_hi)
+// of its rows; the single-GPU build passes key_base = 0 and all ceil(n/32) words.
+int k_fill_case2(const u16* gmask, u64 n_keys, u64 key_base, u64 n, const u64* spec_rows, u64 m, u64 word_lo, u64 word_hi,
+                 u64* bwt, cudaStream_t st);
+// scatter sorted blue symbols; '#'/'$' rows appended to sharp_rows (unordered) / dollar_row.  bt.head is local to the
+// device's keys, which start at global key index key_base.
+int k_emit_blue(const u64* blue, BranchTable bt, u64 key_base, const u64* spec_ins, u64 m, u64* bwt, u64* sharp_rows,
                 u32* d_sharp_count, u64* dollar_row, cudaStream_t st);
 int k_emit_special(const u64* spec_rows, const u8* spec_chr, u64 m, u64* bwt, cudaStream_t st);
 

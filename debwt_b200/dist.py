@@ -212,13 +212,9 @@ class CudaOps:
     def pack(self, ascii_slice, n_valid, words_out, nwords, err):
         self._ck(self.L.debwt_dev_pack(_p(ascii_slice), _u64(n_valid), _p(words_out), _u64(nwords), _p(err), self._st()))
 
-    def extract(self, words, pos_lo, pos_hi, seps, n_rec, idx_base, keys_out, n_symbols=None):
-        if n_symbols is None:
-            self._ck(self.L.debwt_dev_extract(_p(words), _u64(pos_lo), _u64(pos_hi), _p(seps), _u64(n_rec), _u64(idx_base),
-                                              _p(keys_out), self._st()))
-        else:
-            self._ck(self.L.debwt_dev_extract_slice(_p(words), _u64(n_symbols), _u64(pos_lo), _u64(pos_hi), _p(seps), _u64(n_rec),
-                                                    _u64(idx_base), _p(keys_out), self._st()))
+    def extract(self, words, pos_lo, pos_hi, seps, n_rec, idx_base, keys_out, n_symbols):
+        self._ck(self.L.debwt_dev_extract_slice(_p(words), _u64(n_symbols), _u64(pos_lo), _u64(pos_hi), _p(seps), _u64(n_rec),
+                                                _u64(idx_base), _p(keys_out), self._st()))
 
     def sort(self, keys, timed: bool = False):
         n = keys.numel()

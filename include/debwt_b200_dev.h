@@ -25,11 +25,9 @@ int debwt_dev_init(int device);
 /* K1 on a text slice: n ASCII symbols -> nwords packed words (T padding for [n, n+32), zeros beyond);
    *d_err (u32, device) is OR-ed with 1 on a non-ACGT symbol (src/collect#$.c:66-90). */
 int debwt_dev_pack(const void* d_ascii, uint64_t n, void* d_words, uint64_t nwords, void* d_err, void* stream);
-/* K2 on positions [pos_lo, pos_hi): key of window p in record r goes to keys[p - 32 r - idx_base]. */
-int debwt_dev_extract(const void* d_words, uint64_t pos_lo, uint64_t pos_hi, const void* d_seps, uint64_t n_rec,
-                      uint64_t idx_base, void* d_keys, void* stream);
-/* The same through the tiled kernel of the single-GPU path (packed words staged in shared memory, one record lookup per
-   tile); pos_lo must be a multiple of 32, d_words must hold the whole packed text of n_symbols symbols. */
+/* K2 on positions [pos_lo, pos_hi): key of window p in record r goes to keys[p - 32 r - idx_base].  Runs the tiled
+   kernel of the single-GPU path (packed words staged in shared memory, one record lookup per tile); pos_lo must be a
+   multiple of 32, d_words must hold the whole packed text of n_symbols symbols. */
 int debwt_dev_extract_slice(const void* d_words, uint64_t n_symbols, uint64_t pos_lo, uint64_t pos_hi, const void* d_seps,
                             uint64_t n_rec, uint64_t idx_base, void* d_keys, void* stream);
 /* Workspaces are provided by the caller (device memory, sizes in bytes from the *_workspace_bytes calls):

@@ -88,7 +88,7 @@ class NumpyOps:
         sh = (U(2) * (U(31) - (np.arange(nwords * 32, dtype=np.uint64) & U(31))))
         u(words_out)[:nwords] = np.bitwise_or.reduce((code << sh).reshape(nwords, 32), axis=1)
 
-    def extract(self, words, pos_lo, pos_hi, seps, n_rec, idx_base, keys_out, n_symbols=None):
+    def extract(self, words, pos_lo, pos_hi, seps, n_rec, idx_base, keys_out, n_symbols):
         w, s = u(words), u(seps)
         p = np.arange(pos_lo, pos_hi, dtype=np.uint64)
         r = np.searchsorted(s, p, side="left")
