@@ -290,6 +290,17 @@ def k_group_masks(text: np.ndarray, seps: np.ndarray, device: int = 0) -> np.nda
     return out
 
 
+def k_branch_kmers(text: np.ndarray, seps: np.ndarray, device: int = 0):
+    """K7: the branch table, (entries u64[B] = k-mer << 2 | multi_in << 1 | multi_out ascending, group head key index u64[B])"""
+    text = np.ascontiguousarray(text, dtype=np.uint8)
+    seps = np.ascontiguousarray(seps, dtype=np.uint64)
+    cap = max(text.size - 32 * seps.size, 1)
+    kmer, head = np.empty(cap, dtype=np.uint64), np.empty(cap, dtype=np.uint64)
+    nb = c_u64()
+    check(lib().debwt_k_branch_kmers(device, _ptr(text), text.size, _ptr(seps), seps.size, _ptr(kmer), _ptr(head), cap, ctypes.byref(nb)))
+    return kmer[:nb.value].copy(), head[:nb.value].copy()
+
+
 def bench_sort(n: int, device: int = 0, cfg: int = 0, iters: int = 5) -> float:
     ms = ctypes.c_float()
     check(lib().debwt_bench_sort(device, n, cfg, iters, ctypes.byref(ms)))

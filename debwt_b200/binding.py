@@ -94,6 +94,7 @@ _SIGS = {
     "debwt_k_radix_sort_u64": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, ctypes.c_int, ctypes.POINTER(ctypes.c_float)]),
     "debwt_k_rle": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_p, ctypes.POINTER(c_u64)]),
     "debwt_k_group_masks": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_p]),
+    "debwt_k_branch_kmers": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_p, c_p, c_u64, ctypes.POINTER(c_u64)]),
     "debwt_k_codes": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_p, c_u64, ctypes.POINTER(c_u64), c_p, c_p, c_p, c_u64,
                                       ctypes.POINTER(c_u64)]),
     "debwt_k_sort_blue": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_p, c_p]),

@@ -389,6 +389,10 @@ int debwt_build(debwt_ctx* c, int k) {
     if (k_branch_count(d_keys, nk, d_gmask, true, d_brws, d_tot, st)) return -1;
     u64 h_tot[2] = {0, 0};
     CUDA_TRY(cudaMemcpyAsync(h_tot, d_tot, 16, cudaMemcpyDeviceToHost, st));
+    if (c->cap.on) {
+        c->cap.gmask.resize(nk);
+        CUDA_TRY(cudaMemcpyAsync(c->cap.gmask.data(), d_gmask, nk * 2, cudaMemcpyDeviceToHost, st));
+    }
     CUDA_TRY(cudaStreamSynchronize(st));
     if (h_err[0]) FAIL(c->resolve_ambiguous ? "input contains a symbol that is neither a base nor an IUPAC ambiguity code"
                                             : "input contains a symbol other than A, C, G, T (either case)");
@@ -789,6 +793,18 @@ int open_scratch(Scratch& s, int device) {
     CUDA_TRY(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking));
     return 0;
 }
+// one production build of the text with the capture on; `take` reads what it needs from the capture
+template <typename F>
+int captured_build(int device, const char* text, uint64_t n, const uint64_t* seps, uint64_t R, F take) {
+    debwt_ctx* c = nullptr;
+    if (debwt_create(&c, device)) return -1;
+    c->cap.on = true;
+    int rc = debwt_set_text(c, text, n, seps, R);
+    if (!rc) rc = debwt_build(c, 32);
+    if (!rc) rc = take(c->cap);
+    debwt_destroy(c);
+    return rc;
+}
 }  // namespace
 
 extern "C" {
@@ -870,34 +886,25 @@ int debwt_k_rle(int device, const uint64_t* sorted, uint64_t n, uint64_t* kmers_
     return 0;
 }
 
+// K5-K7 through the production build: the masks as K7's count pass leaves them (key index marked by the sort, text-derived
+// digit histogram when it applies, masks propagated inside the branch-count kernel)
 int debwt_k_group_masks(int device, const char* text, uint64_t n, const uint64_t* seps, uint64_t R, uint16_t* masks_out) {
-    if (check_seps(seps, R, n)) return -1;
-    Scratch s;
-    if (open_scratch(s, device)) return -1;
-    const u64 nk = n - 32 * R;
-    u8* d_a; u64 *d_w, *d_s, *d_ka, *d_kb; u32* d_e; u16* d_g; void* d_ws;
-    KeyIndex ki;
-    ki.bits = key_index_bits(nk);
-    if (s.get(&d_a, n + 64) || s.get(&d_w, text_words(n)) || s.get(&d_e, 4) || s.get(&d_s, R) || s.get(&d_ka, nk + 2) ||
-        s.get(&d_kb, nk + 2) || s.get(&d_g, nk + 2) || s.get(&ki.idx, (1ull << ki.bits) + 2))
-        return -1;
-    CUDA_TRY(cudaMalloc(&d_ws, sort_workspace_bytes(nk, 0)));
-    s.ptrs.push_back(d_ws);
-    SortWorkspace ws;
-    sort_workspace_bind(ws, d_ws, nk, 0);
-    CUDA_TRY(cudaMemcpyAsync(d_a, text, n, cudaMemcpyHostToDevice, s.st));
-    CUDA_TRY(cudaMemcpyAsync(d_s, seps, R * 8, cudaMemcpyHostToDevice, s.st));
-    CUDA_TRY(cudaMemsetAsync(d_e, 0, 16, s.st));
-    CUDA_TRY(cudaMemsetAsync(d_g, 0, (nk + 2) * 2, s.st));
-    u64* d_keys = nullptr;
-    if (k_pack_words(d_a, n, d_w, text_words(n), d_e, s.st) || k_extract(d_w, n, d_s, R, d_ka, s.st) ||
-        radix_sort_u64(d_ka, d_kb, nk, ws, s.st, &d_keys) || k_build_key_index(d_keys, nk, ki, s.st) ||
-        k_mark_edges(d_keys, nk, ki, d_g, s.st) || k_mark_heads_tails(d_w, d_s, R, d_keys, nk, ki, d_g, s.st) ||
-        k_propagate(d_keys, nk, d_g, s.st))
-        return -1;
-    CUDA_TRY(cudaMemcpyAsync(masks_out, d_g, nk * 2, cudaMemcpyDeviceToHost, s.st));
-    CUDA_TRY(cudaStreamSynchronize(s.st));
-    return 0;
+    return captured_build(device, text, n, seps, R, [&](const debwt_ctx::Capture& q) {
+        std::copy(q.gmask.begin(), q.gmask.end(), masks_out);
+        return 0;
+    });
+}
+
+// K7 through the production build: the branch table (k-mer << 2 | multi_in << 1 | multi_out, group head key index)
+int debwt_k_branch_kmers(int device, const char* text, uint64_t n, const uint64_t* seps, uint64_t R, uint64_t* kmer_out,
+                         uint64_t* head_out, uint64_t cap, uint64_t* n_branch_out) {
+    return captured_build(device, text, n, seps, R, [&](const debwt_ctx::Capture& q) {
+        if (n_branch_out) *n_branch_out = q.seg_kmer.size();
+        if (q.seg_kmer.size() > cap) { set_error("debwt_k_branch_kmers: output buffers too small"); return -1; }
+        std::copy(q.seg_kmer.begin(), q.seg_kmer.end(), kmer_out);
+        std::copy(q.seg_head.begin(), q.seg_head.end(), head_out);
+        return 0;
+    });
 }
 
 
@@ -905,19 +912,10 @@ int debwt_k_group_masks(int device, const char* text, uint64_t n, const uint64_t
 int debwt_k_codes(int device, const char* text, uint64_t n, const uint64_t* seps, uint64_t R, uint8_t* codes_out, uint64_t codes_cap,
                   uint64_t* n_codes_out, uint64_t* blue_head_out, uint64_t* blue_spindex_out, uint8_t* blue_prev_out, uint64_t blue_cap,
                   uint64_t* n_blue_out) {
-    debwt_ctx* c = nullptr;
-    if (debwt_create(&c, device)) return -1;
-    c->cap.on = true;
-    int rc = debwt_set_text(c, text, n, seps, R);
-    if (!rc) rc = debwt_build(c, 32);
-    if (!rc) {
-        const auto& q = c->cap;
+    return captured_build(device, text, n, seps, R, [&](const debwt_ctx::Capture& q) {
         if (n_codes_out) *n_codes_out = q.n_codes;
         if (n_blue_out) *n_blue_out = q.blue.size();
-        if (q.n_codes > codes_cap || q.blue.size() > blue_cap) { set_error("debwt_k_codes: output buffers too small"); rc = -1; }
-    }
-    if (!rc) {
-        const auto& q = c->cap;
+        if (q.n_codes > codes_cap || q.blue.size() > blue_cap) { set_error("debwt_k_codes: output buffers too small"); return -1; }
         for (u64 i = 0; i < q.n_codes; ++i) {
             u8 code = (u8)((q.codes[i >> 5] >> (2 * (31 - (i & 31)))) & 3ull);
             if ((q.sep[i >> 5] >> (i & 31)) & 1u) code = i == q.dollar_index ? 5 : 4;
@@ -929,9 +927,8 @@ int debwt_k_codes(int device, const char* text, uint64_t n, const uint64_t* seps
                 blue_spindex_out[e] = q.blue[e] >> 4;
                 blue_prev_out[e] = (u8)(q.blue[e] & 15ull);
             }
-    }
-    debwt_destroy(c);
-    return rc;
+        return 0;
+    });
 }
 
 // K10 alone: codes (one byte per code, 0..3, 4 = '#', 5 = '$' which must be the last code and unique), segments of

@@ -102,9 +102,11 @@ struct debwt_ctx {
         u64 n = 0;                                 // symbols packed so far (a multiple of 32 until the end)
         u64 cap_words = 0;
     } ing;
-    // debwt_k_codes: the build copies the K9 products to the host right before K10 (test entry point only)
+    // debwt_k_group_masks / debwt_k_branch_kmers / debwt_k_codes: the build copies the K5-K7 masks and the K9 products to
+    // the host right before K10 (test entry points only)
     struct Capture {
         bool on = false;
+        std::vector<u16> gmask;        // per sorted key: its group's mask, as K7's count pass leaves it (propagated)
         std::vector<u64> codes;        // packed 2-bit SP codes
         std::vector<u32> sep;          // 1 bit per code: '#' / '$'
         u64 dollar_index = 0, n_codes = 0;

@@ -236,10 +236,15 @@ int debwt_k_radix_sort_u64(int device, uint64_t* keys, uint64_t n, int cfg, floa
 /* K4: count-by-sort of sorted keys -> {kmer, count} (kmerInfo, src/mySort.c:76-77,194); returns D. */
 int debwt_k_rle(int device, const uint64_t* sorted, uint64_t n, uint64_t* kmers_out, uint64_t* counts_out,
                 uint64_t* n_distinct_out);
-/* K5-K7: per sorted key the in/out mask of its k-mer group (src/INandOut.c:253-343):
+/* K5-K7 through the production build: per sorted key the in/out mask of its k-mer group (src/INandOut.c:253-343):
    bits 0-3 in-bases, bit 4 '#'/'$' predecessor, bits 8-11 out-bases, bit 12 precedes a separator. */
 int debwt_k_group_masks(int device, const char* text, uint64_t n_symbols, const uint64_t* seps, uint64_t n_records,
                         uint16_t* masks_out /* n - 32 R */);
+/* K7 through the production build: the branch k-mers (src/INandOut.c:396-417) in ascending order, each as
+   (k-mer << 2) | multi_in << 1 | multi_out with the sorted-key index of its group's first key.  *n_branch_out is set
+   even when it exceeds `cap` (then the call fails and writes nothing). */
+int debwt_k_branch_kmers(int device, const char* text, uint64_t n_symbols, const uint64_t* seps, uint64_t n_records,
+                         uint64_t* kmer_out, uint64_t* head_out, uint64_t cap, uint64_t* n_branch_out);
 
 /* K9 through the production build (src/generateSP.c:534-683): the branch ("SP") codes, one byte each -- 0..3 the next
    base, 4 = '#', 5 = '$' -- and the blue entries as K10 receives them: for entry e the sorted-key index of its k-mer's
