@@ -159,7 +159,7 @@ class BwtBuilder:
 
     def set_result(self, words: np.ndarray, n_symbols: int, sharp: np.ndarray, dollar):
         """Load a finished result (the reference's three outputs, e.g. from `read_outputs` or `build_multi`) in place of a
-        build, to query it with count / sample_sa / sa / locate / verify."""
+        build, to query it with count / sample_sa / sa / locate / extract / verify."""
         words = np.ascontiguousarray(words, dtype=np.uint64)
         sharp = np.ascontiguousarray(sharp, dtype=np.uint64)
         if words.size != (n_symbols + 31) // 32:
@@ -193,6 +193,39 @@ class BwtBuilder:
         if pos.size:
             check(lib().debwt_index_locate(self._h, _ptr(blob), _ptr(offs), len(pats), _ptr(hits), _ptr(pos), pos.size))
         return hits, pos
+
+    def _sizes(self) -> tuple[int, int]:
+        """(N, R) of the result"""
+        n, nw, ns = c_u64(), c_u64(), c_u64()
+        check(lib().debwt_result_sizes(self._h, ctypes.byref(n), ctypes.byref(nw), ctypes.byref(ns)))
+        return int(n.value), int(ns.value) + 1
+
+    def extract(self, starts, ends) -> tuple[np.ndarray, np.ndarray]:
+        """(offsets u64[m + 1], symbols u8[total]): T[starts[i]:ends[i]] as ASCII (A, C, G, T upper case, '#', '$') is
+        symbols[offsets[i]:offsets[i+1]], decoded from the index alone; needs sample_sa"""
+        starts = np.ascontiguousarray(starts, dtype=np.uint64).reshape(-1)
+        ends = np.ascontiguousarray(ends, dtype=np.uint64).reshape(-1)
+        if starts.size != ends.size:
+            raise DebwtError(f"extract: {starts.size} starts but {ends.size} ends")
+        n, _ = self._sizes()
+        # an interval the library will refuse counts 0 here, so that the buffer stays small and the call names it
+        lens = np.where((starts <= ends) & (ends <= np.uint64(n)), ends - starts, np.uint64(0))
+        offs = np.zeros(starts.size + 1, dtype=np.uint64)
+        np.cumsum(lens, out=offs[1:])
+        out = np.empty(int(offs[-1]), dtype=np.uint8)
+        check(lib().debwt_index_extract(self._h, _ptr(starts), _ptr(ends), starts.size, _ptr(out), out.size))
+        return offs, out
+
+    def text(self) -> np.ndarray:
+        """the whole text T (u8[N], ASCII) inverted from the index; needs sample_sa"""
+        n, _ = self._sizes()
+        return self.extract([0], [n])[1]
+
+    def separators(self) -> np.ndarray:
+        """the R separator positions of T ('#' ... '$', ascending; the `seps` of join_records) from the index alone: the
+        rows [N - R, N) hold the suffixes that start with a separator; needs sample_sa"""
+        n, r = self._sizes()
+        return np.sort(self.sa(np.arange(n - r, n, dtype=np.uint64)))
 
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""

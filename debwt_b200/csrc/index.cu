@@ -144,12 +144,14 @@ __device__ __forceinline__ u32 row_symbol(const FmView& f, u64 r) {
     return (u32)(f.bwt[r >> 5] >> (2 * (31 - (r & 31)))) & 3u;
 }
 
-__device__ __forceinline__ u64 lf_of(const FmView& f, u64 r) {
-    const u32 c = row_symbol(f, r);
+// LF(r) for a row r whose symbol c = row_symbol(f, r) is already known
+__device__ __forceinline__ u64 lf_with(const FmView& f, u64 r, u32 c) {
     if (c == 5u) return f.n - 1;                                                  // '$' is the largest suffix
     if (c == 4u) return f.C[4] + lower_bound_u64(f.sharp, 0, f.n_sharp, r);       // src/LFsearch.c:131
     return f.C[c] + occ_before(f, c, r);
 }
+
+__device__ __forceinline__ u64 lf_of(const FmView& f, u64 r) { return lf_with(f, r, row_symbol(f, r)); }
 
 // list node of row r: successor (LF) in the high half, distance to it in the low half; the row whose LF is the start
 // row (the row of suffix 0, which holds '$') ends the list
@@ -402,6 +404,41 @@ __global__ void __launch_bounds__(TPB) locate_kernel(FmView f, SaView s, const u
     positions[h] = sa_of(f, s, sp[i] + (h - hit_offsets[i]));
 }
 
+// ---- extract ------------------------------------------------------------------------------------------------------
+// Inverse samples: isa[v / rate] = r for every sampled row r with SA[r] = v.  The samples are exactly the multiples of
+// the rate below N, so every slot is written once; isa[0] is the '$' row.
+__global__ void __launch_bounds__(TPB) isa_from_sa_kernel(SaView s, u64 n, u32* __restrict__ isa) {
+    const u64 r = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (r >= n) return;
+    const u64 b = s.bits[r >> 5];
+    const u32 m = (u32)b, bit = 1u << (r & 31);
+    if (m & bit) isa[s.vals[(b >> 32) + __popc(m & (bit - 1u))] >> (__ffs(s.rate) - 1)] = (u32)r;
+}
+
+// One thread per rate-aligned block q of interval i = [a, b): it writes T[lo, hi) with lo = max(a, q rate),
+// hi = min(b, (q + 1) rate).  It starts in the row of suffix s = min((q + 1) rate, N) -- the sampled row isa[s / rate], or
+// the '$' row when s = N (suffix N is suffix 0 cyclically) -- and each LF step reads the symbol before the current
+// suffix, so it reads s - lo <= rate symbols to reach lo.  out_off[i] is where T[a] goes; b = a + out_off[i + 1] - out_off[i].
+__global__ void __launch_bounds__(TPB) extract_kernel(FmView f, SaView s, const u32* __restrict__ isa, const u64* __restrict__ starts,
+                                                     const u64* __restrict__ blk_off, const u64* __restrict__ out_off, u64 m,
+                                                     u64 n_blocks, u8* __restrict__ out) {
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (t >= n_blocks) return;
+    const u64 i = upper_bound_u64(blk_off, 0, m + 1, t) - 1;                     // last interval whose blocks start at or before t
+    const u32 sh = __ffs(s.rate) - 1;
+    const u64 a = starts[i], b = a + (out_off[i + 1] - out_off[i]);
+    const u64 q = (a >> sh) + (t - blk_off[i]);
+    const u64 lo = max(a, q << sh), hi = min(b, (q + 1) << sh), top = min((q + 1) << sh, f.n);
+    u8* o = out + out_off[i];                                                     // o[p - a] receives T[p]
+    u64 r = top == f.n ? f.dollar_row : isa[top >> sh];
+    for (u64 p = top - 1;; --p) {                                                 // r is the row of suffix p + 1
+        const u32 c = row_symbol(f, r);
+        if (p < hi) o[p - a] = (u8)"ACGT#$"[c];
+        if (p == lo) break;
+        r = lf_with(f, r, c);
+    }
+}
+
 FmView view_of(const debwt_ctx* c) {
     FmView f;
     f.bwt = c->d_bwt; f.spec = c->d_spec_bits; f.occ = c->d_occ; f.sharp = c->d_sharp_sorted;
@@ -417,7 +454,8 @@ SaView sa_view_of(const debwt_ctx* c) { return SaView{c->d_sa_bits, c->d_sa_vals
 void drop_samples(debwt_ctx* c) {
     if (c->d_sa_bits) cudaFree(c->d_sa_bits);
     if (c->d_sa_vals) cudaFree(c->d_sa_vals);
-    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr;
+    if (c->d_isa_vals) cudaFree(c->d_isa_vals);
+    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr; c->d_isa_vals = nullptr;
     c->sa_rate = 0;
 }
 
@@ -802,6 +840,58 @@ int debwt_index_locate(debwt_ctx* c, const char* patterns, const uint64_t* offse
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
     cudaFree(d); cudaFree(d_pos);
+    return 0;
+}
+
+int debwt_index_extract(debwt_ctx* c, const uint64_t* starts, const uint64_t* ends, uint64_t n_intervals, char* out, uint64_t out_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (n_intervals == 0) return 0;
+    if (!starts || !ends) FAIL("null argument");
+    const u64 m = n_intervals, n = c->n, rate = c->sa_rate;
+    // what the device reads: starts (m) | block offsets (m + 1) | output offsets (m + 1)
+    std::vector<u64> h(3 * m + 2);
+    u64 *blk = h.data() + m, *off = blk + m + 1;
+    blk[0] = off[0] = 0;
+    for (u64 i = 0; i < m; ++i) {
+        const u64 a = starts[i], b = ends[i];
+        if (a > b || b > n)
+            FAIL("index_extract: interval " + std::to_string(i) + " = [" + std::to_string(a) + ", " + std::to_string(b) +
+                 ") does not satisfy 0 <= start <= end <= N = " + std::to_string(n));
+        h[i] = a;
+        blk[i + 1] = blk[i] + (b > a ? (b + rate - 1) / rate - a / rate : 0);
+        off[i + 1] = off[i] + (b - a);
+    }
+    const u64 total = off[m], n_blocks = blk[m];
+    if (total > out_cap)
+        FAIL("index_extract: the intervals hold " + std::to_string(total) + " symbols; out holds " + std::to_string(out_cap));
+    if (total == 0) return 0;
+    if (!out) FAIL("null argument");
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t st = c->st;
+    if (!c->d_isa_vals) {
+        if (cudaMalloc(reinterpret_cast<void**>(&c->d_isa_vals), c->n_sa_samples * 4) != cudaSuccess) {
+            cudaGetLastError();
+            c->d_isa_vals = nullptr;
+            FAIL("index_extract: out of device memory for the inverse samples");
+        }
+        isa_from_sa_kernel<<<grid_for(n), TPB, 0, st>>>(sa_view_of(c), n, c->d_isa_vals);
+        DEBWT_COUNT(1);
+    }
+    u64* d = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d), h.size() * 8 + total) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL("index_extract: out of device memory for " + std::to_string(total) + " symbols");
+    }
+    u64 *d_starts = d, *d_blk = d + m, *d_off = d_blk + m + 1;
+    u8* d_out = reinterpret_cast<u8*>(d + h.size());
+    CUDA_TRY(cudaMemcpyAsync(d, h.data(), h.size() * 8, cudaMemcpyHostToDevice, st));
+    extract_kernel<<<grid_for(n_blocks), TPB, 0, st>>>(view_of(c), sa_view_of(c), c->d_isa_vals, d_starts, d_blk, d_off, m, n_blocks,
+                                                       d_out);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(out, d_out, total, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    cudaFree(d);
     return 0;
 }
 

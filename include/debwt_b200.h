@@ -195,6 +195,14 @@ int debwt_index_sa(debwt_ctx* ctx, const uint64_t* rows, uint64_t n_rows, uint64
    positions_cap fails and names the number needed.  Needs debwt_index_sample_sa. */
 int debwt_index_locate(debwt_ctx* ctx, const char* patterns, const uint64_t* offsets, uint64_t n_patterns, uint64_t* hit_offsets,
                        uint64_t* positions, uint64_t positions_cap);
+/* Extract: T[starts[i] .. ends[i]) for every i -- the text the result is the BWT of -- as ASCII (A, C, G, T upper case,
+   '#', '$'), concatenated in order into `out` (sum of ends[i] - starts[i] bytes, no terminator).  Needs
+   debwt_index_sample_sa; the first call after it derives the inverse samples from the SA samples (4 ceil(N / rate) more
+   bytes of HBM, kept with the samples).  Each rate-aligned block is decoded by at most `rate` LF steps, one thread per
+   block, so [0, N) inverts the whole BWT.  Fails, writing nothing, when some 0 <= starts[i] <= ends[i] <= N does not hold
+   (the message names i) or the total exceeds out_cap (the message names the total).  n_intervals = 0 does nothing. */
+int debwt_index_extract(debwt_ctx* ctx, const uint64_t* starts, const uint64_t* ends, uint64_t n_intervals,
+                        char* out, uint64_t out_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
