@@ -227,6 +227,22 @@ class BwtBuilder:
         n, r = self._sizes()
         return np.sort(self.sa(np.arange(n - r, n, dtype=np.uint64)))
 
+    def smem(self, reads: Sequence, min_len: int = 19) -> tuple[np.ndarray, np.ndarray]:
+        """(offsets u64[m + 1], smems SMEM_DTYPE[total]): the super-maximal exact matches of at least `min_len` bases of read
+        i are smems[offsets[i]:offsets[i+1]], in ascending qbeg.  The text must hold both strands (`both_strands`); rows
+        [row, row + count) are the suffixes that start with the match, for `sa`.  Builds the index tables if needed."""
+        check(lib().debwt_index_build(self._h))
+        rs = [r.encode() if isinstance(r, str) else bytes(r) for r in reads]
+        offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(r) for r in rs])
+        blob = np.frombuffer(b"".join(rs) + b"\0", dtype=np.uint8)
+        so = np.zeros(len(rs) + 1, dtype=np.uint64)
+        check(lib().debwt_index_smem(self._h, _ptr(blob), _ptr(offs), len(rs), min_len, _ptr(so), c_p(0), 0))
+        out = np.zeros(int(so[-1]), dtype=SMEM_DTYPE)
+        if out.size:
+            check(lib().debwt_index_smem(self._h, _ptr(blob), _ptr(offs), len(rs), min_len, _ptr(so), _ptr(out), out.size))
+        return so, out
+
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""
         bad, ms = c_u64(), ctypes.c_float()
@@ -281,6 +297,44 @@ def record_offsets(positions, seps) -> tuple[np.ndarray, np.ndarray]:
     rec = np.searchsorted(seps, pos, side="left")
     starts = np.concatenate(([0], seps[:-1] + 1)).astype(np.uint64)
     return rec.astype(np.int64), pos - starts[rec]
+
+
+# ---- SMEM seeding over both strands (debwt_index_smem) ---------------------------------------------------------------
+SMEM_DTYPE = np.dtype([("row", np.uint64), ("rc_row", np.uint64), ("count", np.uint64), ("qbeg", np.uint32), ("qend", np.uint32)],
+                      align=True)                      # debwt_smem of include/debwt_b200.h
+
+_COMP = bytes.maketrans(b"ACGT", b"TGCA")
+
+
+def both_strands(records: Sequence) -> list[bytes]:
+    """records + their reverse complements, upper case, in that order: a text closed under reverse complement, which SMEM
+    search needs (Li 2012's FMD-index).  Only A, C, G, T (either case) are accepted; ambiguity codes resolved at random
+    per position would break the closure."""
+    fwd = []
+    for i, r in enumerate(records):
+        b = (r.encode() if isinstance(r, str) else bytes(np.asarray(r, dtype=np.uint8)) if isinstance(r, np.ndarray) else bytes(r)).upper()
+        bad = b.translate(None, b"ACGT")
+        if bad:
+            raise DebwtError(f"both_strands: record {i} holds {bad[:1]!r}; only A, C, G and T have a reverse complement here")
+        fwd.append(b)
+    return fwd + [b.translate(_COMP)[::-1] for b in fwd]
+
+
+def strand_offsets(positions, length: int, seps) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """Hits of `length` symbols at text positions of a `both_strands` text (separators `seps`, 2 R records) to (record in
+    0..R-1, strand 0 forward / 1 reverse, offset of the hit's first base on the forward strand).  A hit at offset o of the
+    reverse copy of record i covers forward bases [len_i - o - length, len_i - o)."""
+    seps = np.asarray(seps, dtype=np.uint64)
+    if seps.size % 2:
+        raise ValueError(f"{seps.size} records: a both_strands text has an even number")
+    rec, off = record_offsets(positions, seps)
+    off = off.astype(np.int64)
+    R = seps.size // 2
+    lens = (seps - np.concatenate(([0], seps[:-1] + 1)).astype(np.uint64)).astype(np.int64)
+    if rec.size and (off + length > lens[rec]).any():
+        raise ValueError(f"a hit of {length} symbols runs past the end of its record")
+    rev = rec >= R
+    return rec % R, rev.astype(np.int8), np.where(rev, lens[rec] - off - length, off)
 
 
 # ---- per-kernel entry points (parity tests) -------------------------------------------------------

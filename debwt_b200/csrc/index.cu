@@ -439,6 +439,142 @@ __global__ void __launch_bounds__(TPB) extract_kernel(FmView f, SaView s, const 
     }
 }
 
+// ---- SMEM search (FMD-index, Li 2012) ----------------------------------------------------------------------------
+// Over a text closed under reverse complement the rows of rc(P) are the reverse interval of P: a bi-interval (k, l, s)
+// holds the rows [k, k + s) of P and [l, l + s) of rc(P).  Here '#' and '$' sort after T, so inside [l, l + s) the suffixes
+// rc(P)T, rc(P)G, rc(P)C, rc(P)A come first, in that order, and rc(P)# / rc(P)$ last: the reverse starts need no sentinel
+// term (BWA's bwt_extend has its sentinel first and does not carry over).
+
+// counts of A, C, G, T in the rows < r: one 32-byte occ checkpoint, the BWT word and the '#'/'$' mask word
+__device__ __forceinline__ void occ4_before(const FmView& f, u64 r, u64 o[4]) {
+    const u64 w = r >> 5;
+    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(f.occ + w * 4);
+    const ulonglong2 a = p[0], b = p[1];
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+    const u32 below = (1u << (r & 31)) - 1u;
+    if (below) {                                                                  // r = N on a word edge reads no word
+        const u64 x = f.bwt[w];
+        const u32 ok = ~f.spec[w] & below;
+#pragma unroll
+        for (u32 c = 0; c < 4; ++c) o[c] += __popc(symbol_mask(x, c) & ok);
+    }
+}
+
+__device__ __forceinline__ u64 pick4(const u64 v[4], u32 c) { return c == 0 ? v[0] : c == 1 ? v[1] : c == 2 ? v[2] : v[3]; }
+
+struct BiIv {
+    u64 k, l, s;   // rows [k, k + s) start with P, [l, l + s) with rc(P)
+    u64 end;       // read position one past P
+};
+
+// P -> aP: k_a = C[a] + occ(a, k), s_a = occ(a, k + s) - occ(a, k); l_T = l, l_G = l_T + s_T, l_C = l_G + s_G, l_A = l_C + s_C
+__device__ __forceinline__ BiIv backward_ext(const FmView& f, const BiIv& p, u32 a) {
+    u64 lo[4], hi[4];
+    occ4_before(f, p.k, lo);
+    occ4_before(f, p.k + p.s, hi);
+    u64 l = p.l;
+#pragma unroll
+    for (u32 c = 3; c > 0; --c)
+        if (c > a) l += hi[c] - lo[c];
+    const u64 k_a = (a == 0 ? f.C[0] : a == 1 ? f.C[1] : a == 2 ? f.C[2] : f.C[3]) + pick4(lo, a);
+    return BiIv{k_a, l, pick4(hi, a) - pick4(lo, a), p.end};
+}
+
+// P -> Pa: backward extension of rc(P) by comp(a), starts swapped back
+__device__ __forceinline__ BiIv forward_ext(const FmView& f, const BiIv& p, u32 a) {
+    const BiIv r = backward_ext(f, BiIv{p.l, p.k, p.s, p.end}, 3u - a);
+    return BiIv{r.l, r.k, r.s, p.end};
+}
+
+// One thread per scratch slot; slots take reads from the work counter `next`.  Slot t owns two interval lists of
+// `list_cap` entries (the longest read + 1), entry j of list h at scratch[(h list_cap + j) n_slots + t], so that the
+// threads of a warp that stand at the same entry touch neighbouring 32-byte entries.  Li's outer loop: x = 0; x = smem1(x)
+// at A/C/G/T that occurs in T, x + 1 past any other symbol.  The count pass (out == nullptr) writes the number of SMEMs
+// of at least min_len per read; the write pass writes them at out_off.
+__global__ void __launch_bounds__(TPB) smem_kernel(FmView f, const u8* __restrict__ reads, const u64* __restrict__ offs, u64 n_reads,
+                                                  u32 min_len, BiIv* __restrict__ scratch, u64 n_slots, u64 list_cap,
+                                                  unsigned long long* __restrict__ next, u64* __restrict__ counts,
+                                                  const u64* __restrict__ out_off, debwt_smem* __restrict__ out) {
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (t >= n_slots) return;
+    BiIv* const list0 = scratch + t;
+    BiIv* const list1 = scratch + list_cap * n_slots + t;
+    for (;;) {
+        const u64 rd = atomicAdd(next, 1ull);
+        if (rd >= n_reads) break;
+        const u8* q = reads + offs[rd];
+        const u32 m = (u32)(offs[rd + 1] - offs[rd]);
+        debwt_smem* o = out ? out + out_off[rd] : nullptr;
+        u64 n_out = 0;
+        u32 x = 0;
+        while (x < m) {
+            const u32 a = pattern_symbol(q[x]);
+            const u64 ca = a > 3u ? 0 : (a == 0 ? f.C[1] - f.C[0] : a == 1 ? f.C[2] - f.C[1] : a == 2 ? f.C[3] - f.C[2] : f.C[4] - f.C[3]);
+            if (ca == 0) { ++x; continue; }                                       // no match covers x
+            // forward from x: push the interval before each change of size, at the end of the read or before a non-ACGT;
+            // pushed at descending entries of list 1 so that they read back longest-match first
+            BiIv ik{a == 0 ? f.C[0] : a == 1 ? f.C[1] : a == 2 ? f.C[2] : f.C[3],
+                    a == 3 ? f.C[0] : a == 2 ? f.C[1] : a == 1 ? f.C[2] : f.C[3], ca, (u64)x + 1};
+            u64 top = list_cap;
+            u32 i = x + 1;
+            for (; i < m; ++i) {
+                const u32 c = pattern_symbol(q[i]);
+                if (c > 3u) { list1[--top * n_slots] = ik; break; }
+                BiIv ok = forward_ext(f, ik, c);
+                if (ok.s != ik.s) {
+                    list1[--top * n_slots] = ik;
+                    if (ok.s == 0) break;
+                }
+                ik = ok;
+                ik.end = (u64)i + 1;
+            }
+            if (i == m) list1[--top * n_slots] = ik;
+            const BiIv* prev = list1 + top * n_slots;
+            u64 n_prev = list_cap - top;
+            const u32 ret = (u32)prev[0].end;
+            // backward: extend every interval by q[i]; the first that cannot be extended ends an SMEM at i + 1 unless a longer
+            // one ended there; equal sizes are kept once
+            const u64 first = n_out;
+            u32 last_beg = 0xFFFFFFFFu;
+            BiIv* curr = list0;
+            for (long long i2 = (long long)x - 1; i2 >= -1; --i2) {
+                const u32 c = i2 < 0 ? 4u : pattern_symbol(q[i2]);
+                u64 n_curr = 0, last_s = 0;
+                for (u64 j = 0; j < n_prev; ++j) {
+                    const BiIv p = prev[j * n_slots];
+                    BiIv ok{0, 0, 0, 0};
+                    if (c < 4u) ok = backward_ext(f, p, c);
+                    if (ok.s == 0) {
+                        const u32 beg = (u32)(i2 + 1);
+                        if (n_curr == 0 && beg < last_beg) {
+                            last_beg = beg;
+                            if (p.end - beg >= min_len) {
+                                if (o) o[n_out] = debwt_smem{p.k, p.l, p.s, beg, (u32)p.end};
+                                ++n_out;
+                            }
+                        }
+                    } else if (n_curr == 0 || ok.s != last_s) {
+                        curr[n_curr++ * n_slots] = ok;
+                        last_s = ok.s;
+                    }
+                }
+                if (n_curr == 0) break;
+                prev = curr;
+                n_prev = n_curr;
+                curr = curr == list0 ? list1 : list0;
+            }
+            if (o)                                                                // one smem1 call finds them by descending qbeg
+                for (u64 lo = first, hi = n_out; lo + 1 < hi; ++lo, --hi) {
+                    const debwt_smem tmp = o[lo];
+                    o[lo] = o[hi - 1];
+                    o[hi - 1] = tmp;
+                }
+            x = ret;
+        }
+        if (!o) counts[rd] = n_out;
+    }
+}
+
 FmView view_of(const debwt_ctx* c) {
     FmView f;
     f.bwt = c->d_bwt; f.spec = c->d_spec_bits; f.occ = c->d_occ; f.sharp = c->d_sharp_sorted;
@@ -892,6 +1028,90 @@ int debwt_index_extract(debwt_ctx* c, const uint64_t* starts, const uint64_t* en
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
     cudaFree(d);
+    return 0;
+}
+
+static_assert(sizeof(debwt_smem) == 32, "debwt_smem is 3 u64 + 2 u32");
+static_assert(sizeof(BiIv) == 32, "one scratch entry is one 32-byte sector");
+
+// Scratch of the SMEM lists: each read in flight holds two lists of (longest read + 1) entries of 32 bytes
+constexpr u64 kSmemScratchBytes = 1ull << 30;
+
+int debwt_index_smem(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, uint32_t min_len,
+                     uint64_t* smem_offsets, debwt_smem* smems, uint64_t smems_cap) {
+    if (!c || !c->indexed) FAIL("no index: call debwt_index_build first");
+    if (!offsets || !smem_offsets || (n_reads && !reads)) FAIL("null argument");
+    if (min_len == 0) FAIL("index_smem: min_len must be at least 1");
+    const u64* C = c->c_array;
+    const u64 nA = C[1] - C[0], nC = C[2] - C[1], nG = C[3] - C[2], nT = C[4] - C[3];
+    if (nA != nT || nC != nG)
+        FAIL("index_smem: the text is not closed under reverse complement: it holds A = " + std::to_string(nA) + ", C = " +
+             std::to_string(nC) + ", G = " + std::to_string(nG) + ", T = " + std::to_string(nT) +
+             " bases; build it from every record and its reverse complement (api.both_strands)");
+    const u64 m = n_reads;
+    u64 max_len = 0, longest = 0;
+    for (u64 i = 0; i < m; ++i) {
+        if (offsets[i + 1] < offsets[i]) FAIL("index_smem: offsets decrease at read " + std::to_string(i));
+        if (offsets[i + 1] - offsets[i] > max_len) { max_len = offsets[i + 1] - offsets[i]; longest = i; }
+    }
+    const u64 list_cap = max_len + 1, slot_bytes = 2 * list_cap * sizeof(BiIv);
+    if (slot_bytes > kSmemScratchBytes)
+        FAIL("index_smem: read " + std::to_string(longest) + " has " + std::to_string(max_len) + " symbols; its interval lists need " +
+             std::to_string(slot_bytes) + " bytes, more than the " + std::to_string(kSmemScratchBytes) + " bytes of scratch (reads up to " +
+             std::to_string(kSmemScratchBytes / (2 * sizeof(BiIv)) - 1) + " symbols)");
+    smem_offsets[0] = 0;
+    if (m == 0) return 0;
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t st = c->st;
+    int sms = 0, per_sm = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxThreadsPerMultiProcessor, c->device));
+    const u64 n_slots = std::min<u64>({(u64)sms * (u64)per_sm, kSmemScratchBytes / slot_bytes, m});
+    const u64 bytes = offsets[m], nb = (m + TPB - 1) / TPB, words = (bytes + 16 + 7) / 8;
+    // one block: reads | offsets (m + 1) | counts (m) | SMEM offsets (m + 1) | block totals (nb) | their scan (nb + 1) | counter
+    u64* d = nullptr;
+    BiIv* d_scratch = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d), (words + 3 * m + 2 * nb + 4) * 8));
+    if (cudaMalloc(reinterpret_cast<void**>(&d_scratch), n_slots * slot_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d);
+        FAIL("index_smem: out of device memory for " + std::to_string(n_slots * slot_bytes) + " bytes of scratch");
+    }
+    u8* d_r = reinterpret_cast<u8*>(d);
+    u64 *d_o = d + words, *d_cnt = d_o + m + 1, *d_off = d_cnt + m, *d_tot = d_off + m + 1, *d_base = d_tot + nb;
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(d_base + nb + 1);
+    CUDA_TRY(cudaMemcpyAsync(d_r, reads, bytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_o, offsets, (m + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
+    const FmView f = view_of(c);
+    const unsigned grid = grid_for(n_slots);
+    smem_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, min_len, d_scratch, n_slots, list_cap, d_next, d_cnt, nullptr, nullptr);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_base, d_off);
+    DEBWT_COUNT(4);
+    CUDA_TRY(cudaMemcpyAsync(smem_offsets, d_off, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    const u64 total = smem_offsets[m];
+    if (!smems || total == 0) { cudaFree(d); cudaFree(d_scratch); return 0; }   // size query
+    if (total > smems_cap) {
+        cudaFree(d); cudaFree(d_scratch);
+        FAIL("index_smem: the reads have " + std::to_string(total) + " SMEMs; smems holds " + std::to_string(smems_cap));
+    }
+    debwt_smem* d_out = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_out), total * sizeof(debwt_smem)) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d); cudaFree(d_scratch);
+        FAIL("index_smem: out of device memory for " + std::to_string(total) + " SMEMs");
+    }
+    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
+    smem_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, min_len, d_scratch, n_slots, list_cap, d_next, nullptr, d_off, d_out);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(smems, d_out, total * sizeof(debwt_smem), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    cudaFree(d); cudaFree(d_scratch); cudaFree(d_out);
     return 0;
 }
 

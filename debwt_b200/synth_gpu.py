@@ -48,6 +48,14 @@ def mutate(seq: torch.Tensor, seed: int, rate: float) -> torch.Tensor:
     return out
 
 
+def reverse_complement(seq: torch.Tensor) -> torch.Tensor:
+    """the reverse complement of an upper-case ACGT sequence on the device (api.both_strands on the device)"""
+    lut = torch.zeros(256, dtype=torch.uint8, device=seq.device)
+    for x, y in (b"AT", b"CG", b"GC", b"TA"):
+        lut[x] = y
+    return lut[seq.long()].flip(0)
+
+
 def join_records_device(records) -> tuple[torch.Tensor, np.ndarray]:
     """T = S1 # S2 # ... Sn $ in one device buffer + separator offsets (what api.join_records does on the host)"""
     n = sum(int(r.numel()) for r in records) + len(records)

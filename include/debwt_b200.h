@@ -203,6 +203,26 @@ int debwt_index_locate(debwt_ctx* ctx, const char* patterns, const uint64_t* off
    (the message names i) or the total exceeds out_cap (the message names the total).  n_intervals = 0 does nothing. */
 int debwt_index_extract(debwt_ctx* ctx, const uint64_t* starts, const uint64_t* ends, uint64_t n_intervals,
                         char* out, uint64_t out_cap);
+/* Super-maximal exact matches (SMEMs, the seeds of BWA-MEM) of reads against a text that holds both strands, by the
+   bidirectional FMD-index search of Li (2012) over the occ / C tables.  The text must be closed under reverse complement:
+   every record's reverse complement is a record too (python: api.both_strands).  That is the caller's duty; the call only
+   checks the necessary count(A) = count(T) and count(C) = count(G) from the C-array.
+   Read i = reads[offsets[i] .. offsets[i+1]).  A match is a piece read[s, e) of A, C, G, T (either case) that occurs in
+   T; with start(e) the smallest s for which read[s, e) matches (e if none does), the SMEMs are the [start(e), e) with
+   start(e) < e and (e = len or start(e+1) > start(e)) -- the matches not contained in another maximal match.  Those with
+   qend - qbeg >= min_len (>= 1) are written, read by read, in ascending qbeg (and qend): smems[smem_offsets[i] + j].
+   Rows [row, row + count) hold the suffixes that start with read[qbeg, qend) (locate them with debwt_index_sa), rc_row
+   the first row of its reverse complement; count covers both strands.  smem_offsets[n_reads + 1] is always written;
+   smems == NULL is a size query; more SMEMs than smems_cap fails and names the number needed.  Needs debwt_index_build,
+   not the SA samples.  Fails, writing nothing, on an unbalanced text (the message names the four base counts), min_len = 0,
+   decreasing offsets, NULL arguments, or a read too long for the 1 GiB of scratch (64 (len + 1) bytes per read in flight;
+   reads up to 16 Mbp; the message names the read).  n_reads = 0 only writes smem_offsets[0] = 0. */
+typedef struct debwt_smem {
+    uint64_t row, rc_row, count;   /* rows [row, row + count) start with read[qbeg, qend); rc_row: its reverse complement */
+    uint32_t qbeg, qend;
+} debwt_smem;
+int debwt_index_smem(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads, uint32_t min_len,
+                     uint64_t* smem_offsets /* n_reads + 1 */, debwt_smem* smems, uint64_t smems_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
