@@ -243,6 +243,31 @@ class BwtBuilder:
             check(lib().debwt_index_smem(self._h, _ptr(blob), _ptr(offs), len(rs), min_len, _ptr(so), _ptr(out), out.size))
         return so, out
 
+    def seeds(self, reads: Sequence, min_len: int = 19, split_factor: float = 1.5, split_width: int = 10, max_mem_intv: int = 20,
+              max_occ: int = 500) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(offsets u64[m + 1], seeds SEED_DTYPE[total], hits HIT_DTYPE[all hits]): BWA-MEM's seeds of read i (bwa's -k, -r,
+        split_width, -y, -c; SMEMs, re-seeded SMEMs and LAST-like seeds, `round` 1 / 2 / 3) are seeds[offsets[i]:offsets[i+1]],
+        in ascending (qbeg, qend, round); seed s has hits[s.hit_begin : s.hit_begin + s.n_hits], at most max_occ evenly
+        spaced rows of its interval, each with its text position, record, strand and forward offset (`strand_offsets`).
+        The text must hold both strands (`both_strands`); needs sample_sa."""
+        rs = [r.encode() if isinstance(r, str) else bytes(r) for r in reads]
+        offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(r) for r in rs])
+        blob = np.frombuffer(b"".join(rs) + b"\0", dtype=np.uint8)
+        for name, v in (("min_len", min_len), ("split_width", split_width), ("max_mem_intv", max_mem_intv), ("max_occ", max_occ)):
+            if not 0 <= v < 1 << 32:
+                raise DebwtError(f"seeds: {name} = {v} is not a 32-bit unsigned integer")
+        opts = SeedOpts(min_len, split_width, max_mem_intv, max_occ, split_factor)
+        so = np.zeros(len(rs) + 1, dtype=np.uint64)
+        nh = c_u64()
+        args = (self._h, _ptr(blob), _ptr(offs), len(rs), ctypes.addressof(opts), _ptr(so), ctypes.addressof(nh))
+        check(lib().debwt_index_seeds(*args, c_p(0), 0, c_p(0), 0))
+        seeds = np.zeros(int(so[-1]), dtype=SEED_DTYPE)
+        hits = np.zeros(int(nh.value), dtype=HIT_DTYPE)
+        if seeds.size:
+            check(lib().debwt_index_seeds(*args, _ptr(seeds), seeds.size, _ptr(hits), hits.size))
+        return so, seeds, hits
+
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""
         bad, ms = c_u64(), ctypes.c_float()
@@ -302,6 +327,18 @@ def record_offsets(positions, seps) -> tuple[np.ndarray, np.ndarray]:
 # ---- SMEM seeding over both strands (debwt_index_smem) ---------------------------------------------------------------
 SMEM_DTYPE = np.dtype([("row", np.uint64), ("rc_row", np.uint64), ("count", np.uint64), ("qbeg", np.uint32), ("qend", np.uint32)],
                       align=True)                      # debwt_smem of include/debwt_b200.h
+
+# ---- BWA-MEM seed collection over both strands (debwt_index_seeds) ---------------------------------------------------
+SEED_DTYPE = np.dtype([("row", np.uint64), ("rc_row", np.uint64), ("count", np.uint64), ("qbeg", np.uint32), ("qend", np.uint32),
+                       ("hit_begin", np.uint64), ("n_hits", np.uint32), ("round", np.uint32)], align=True)    # debwt_seed
+HIT_DTYPE = np.dtype([("pos", np.uint64), ("offset", np.uint64), ("record", np.uint32), ("strand", np.uint32)], align=True)  # debwt_seed_hit
+
+
+class SeedOpts(ctypes.Structure):
+    """debwt_seed_opts of include/debwt_b200.h"""
+    _fields_ = [("min_seed_len", ctypes.c_uint32), ("split_width", ctypes.c_uint32), ("max_mem_intv", ctypes.c_uint32),
+                ("max_occ", ctypes.c_uint32), ("split_factor", ctypes.c_float)]
+
 
 _COMP = bytes.maketrans(b"ACGT", b"TGCA")
 

@@ -142,6 +142,7 @@ struct debwt_ctx {
     u32 sa_rate = 0;                  // 0 = not sampled
     u64 n_sa_samples = 0;
     u32* d_isa_vals = nullptr;        // [n_sa_samples]: [k] = row of suffix k * rate (the first debwt_index_extract after sampling)
+    u64* d_seps_sorted = nullptr;     // [n_rec]: the separator positions, ascending (the first debwt_index_seeds after sampling)
     bool loaded = false;              // the result came from debwt_set_result, not from a build
 };
 

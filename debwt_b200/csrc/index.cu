@@ -11,10 +11,12 @@
 //     its distance to the end of the walk, i.e. its text position.  The BWT is the BWT of T iff the permutation is ONE
 //     cycle and the symbol of row r equals T[position(r) - 1] for every r -- checked against the caller's ASCII text.
 #include <algorithm>
+#include <cmath>
 #include <string>
 #include <vector>
 
 #include "ctx.cuh"
+#include "radix_sort.cuh"
 
 namespace debwt {
 
@@ -486,6 +488,72 @@ __device__ __forceinline__ BiIv forward_ext(const FmView& f, const BiIv& p, u32 
     return BiIv{r.l, r.k, r.s, p.end};
 }
 
+__device__ __forceinline__ u64 base_count(const FmView& f, u32 a) {                  // occurrences of base a (0 past T)
+    return a > 3u ? 0 : (a == 0 ? f.C[1] - f.C[0] : a == 1 ? f.C[2] - f.C[1] : a == 2 ? f.C[3] - f.C[2] : f.C[4] - f.C[3]);
+}
+
+// the bi-interval of the one base a (count ca) at read position x
+__device__ __forceinline__ BiIv single_base(const FmView& f, u32 a, u64 ca, u32 x) {
+    return BiIv{a == 0 ? f.C[0] : a == 1 ? f.C[1] : a == 2 ? f.C[2] : f.C[3],
+                a == 3 ? f.C[0] : a == 2 ? f.C[1] : a == 1 ? f.C[2] : f.C[3], ca, (u64)x + 1};
+}
+
+// Li's smem1 from q[x], a base a that occurs ca >= 1 times in T: BWA's bwt_smem1a(x, min_intv = t, max_intv = 0).  Every
+// SMEM it finds goes to emit(interval, qbeg) by descending qbeg (qend = interval.end); returns the end of the longest match
+// from x.  list0 / list1: the slot's two interval lists of list_cap entries, entry j at [j n_slots].
+template <class Emit>
+__device__ __forceinline__ u32 smem1(const FmView& f, const u8* __restrict__ q, u32 m, u32 x, u32 a, u64 ca, u64 t, BiIv* list0,
+                                     BiIv* list1, u64 n_slots, u64 list_cap, Emit&& emit) {
+    // forward from x: push the interval before each change of size, at the end of the read or before a non-ACGT;
+    // pushed at descending entries of list 1 so that they read back longest-match first
+    BiIv ik = single_base(f, a, ca, x);
+    u64 top = list_cap;
+    u32 i = x + 1;
+    for (; i < m; ++i) {
+        const u32 c = pattern_symbol(q[i]);
+        if (c > 3u) { list1[--top * n_slots] = ik; break; }
+        BiIv ok = forward_ext(f, ik, c);
+        if (ok.s != ik.s) {
+            list1[--top * n_slots] = ik;
+            if (ok.s < t) break;
+        }
+        ik = ok;
+        ik.end = (u64)i + 1;
+    }
+    if (i == m) list1[--top * n_slots] = ik;
+    const BiIv* prev = list1 + top * n_slots;
+    u64 n_prev = list_cap - top;
+    const u32 ret = (u32)prev[0].end;
+    // backward: extend every interval by q[i]; the first that falls below t ends an SMEM at i + 1 unless a longer one
+    // ended there; equal sizes are kept once
+    u32 last_beg = 0xFFFFFFFFu;
+    BiIv* curr = list0;
+    for (long long i2 = (long long)x - 1; i2 >= -1; --i2) {
+        const u32 c = i2 < 0 ? 4u : pattern_symbol(q[i2]);
+        u64 n_curr = 0, last_s = 0;
+        for (u64 j = 0; j < n_prev; ++j) {
+            const BiIv p = prev[j * n_slots];
+            BiIv ok{0, 0, 0, 0};
+            if (c < 4u) ok = backward_ext(f, p, c);
+            if (ok.s < t) {
+                const u32 beg = (u32)(i2 + 1);
+                if (n_curr == 0 && beg < last_beg) {
+                    last_beg = beg;
+                    emit(p, beg);
+                }
+            } else if (n_curr == 0 || ok.s != last_s) {
+                curr[n_curr++ * n_slots] = ok;
+                last_s = ok.s;
+            }
+        }
+        if (n_curr == 0) break;
+        prev = curr;
+        n_prev = n_curr;
+        curr = curr == list0 ? list1 : list0;
+    }
+    return ret;
+}
+
 // One thread per scratch slot; slots take reads from the work counter `next`.  Slot t owns two interval lists of
 // `list_cap` entries (the longest read + 1), entry j of list h at scratch[(h list_cap + j) n_slots + t], so that the
 // threads of a warp that stand at the same entry touch neighbouring 32-byte entries.  Li's outer loop: x = 0; x = smem1(x)
@@ -509,70 +577,153 @@ __global__ void __launch_bounds__(TPB) smem_kernel(FmView f, const u8* __restric
         u32 x = 0;
         while (x < m) {
             const u32 a = pattern_symbol(q[x]);
-            const u64 ca = a > 3u ? 0 : (a == 0 ? f.C[1] - f.C[0] : a == 1 ? f.C[2] - f.C[1] : a == 2 ? f.C[3] - f.C[2] : f.C[4] - f.C[3]);
+            const u64 ca = base_count(f, a);
             if (ca == 0) { ++x; continue; }                                       // no match covers x
-            // forward from x: push the interval before each change of size, at the end of the read or before a non-ACGT;
-            // pushed at descending entries of list 1 so that they read back longest-match first
-            BiIv ik{a == 0 ? f.C[0] : a == 1 ? f.C[1] : a == 2 ? f.C[2] : f.C[3],
-                    a == 3 ? f.C[0] : a == 2 ? f.C[1] : a == 1 ? f.C[2] : f.C[3], ca, (u64)x + 1};
-            u64 top = list_cap;
-            u32 i = x + 1;
-            for (; i < m; ++i) {
-                const u32 c = pattern_symbol(q[i]);
-                if (c > 3u) { list1[--top * n_slots] = ik; break; }
-                BiIv ok = forward_ext(f, ik, c);
-                if (ok.s != ik.s) {
-                    list1[--top * n_slots] = ik;
-                    if (ok.s == 0) break;
-                }
-                ik = ok;
-                ik.end = (u64)i + 1;
-            }
-            if (i == m) list1[--top * n_slots] = ik;
-            const BiIv* prev = list1 + top * n_slots;
-            u64 n_prev = list_cap - top;
-            const u32 ret = (u32)prev[0].end;
-            // backward: extend every interval by q[i]; the first that cannot be extended ends an SMEM at i + 1 unless a longer
-            // one ended there; equal sizes are kept once
             const u64 first = n_out;
-            u32 last_beg = 0xFFFFFFFFu;
-            BiIv* curr = list0;
-            for (long long i2 = (long long)x - 1; i2 >= -1; --i2) {
-                const u32 c = i2 < 0 ? 4u : pattern_symbol(q[i2]);
-                u64 n_curr = 0, last_s = 0;
-                for (u64 j = 0; j < n_prev; ++j) {
-                    const BiIv p = prev[j * n_slots];
-                    BiIv ok{0, 0, 0, 0};
-                    if (c < 4u) ok = backward_ext(f, p, c);
-                    if (ok.s == 0) {
-                        const u32 beg = (u32)(i2 + 1);
-                        if (n_curr == 0 && beg < last_beg) {
-                            last_beg = beg;
-                            if (p.end - beg >= min_len) {
-                                if (o) o[n_out] = debwt_smem{p.k, p.l, p.s, beg, (u32)p.end};
-                                ++n_out;
-                            }
-                        }
-                    } else if (n_curr == 0 || ok.s != last_s) {
-                        curr[n_curr++ * n_slots] = ok;
-                        last_s = ok.s;
-                    }
+            x = smem1(f, q, m, x, a, ca, 1, list0, list1, n_slots, list_cap, [&](const BiIv& p, u32 beg) {
+                if (p.end - beg >= min_len) {
+                    if (o) o[n_out] = debwt_smem{p.k, p.l, p.s, beg, (u32)p.end};
+                    ++n_out;
                 }
-                if (n_curr == 0) break;
-                prev = curr;
-                n_prev = n_curr;
-                curr = curr == list0 ? list1 : list0;
-            }
+            });
             if (o)                                                                // one smem1 call finds them by descending qbeg
                 for (u64 lo = first, hi = n_out; lo + 1 < hi; ++lo, --hi) {
                     const debwt_smem tmp = o[lo];
                     o[lo] = o[hi - 1];
                     o[hi - 1] = tmp;
                 }
-            x = ret;
         }
         if (!o) counts[rd] = n_out;
     }
+}
+
+// ---- BWA-MEM seed collection (mem_collect_intv) -----------------------------------------------------------------------
+struct SeedParams {
+    u32 min_len, max_occ;
+    u64 split_len, split_width, max_mem_intv;
+};
+
+__device__ __forceinline__ bool seed_less(const debwt_seed& a, const debwt_seed& b) {
+    return a.qbeg != b.qbeg ? a.qbeg < b.qbeg : a.qend != b.qend ? a.qend < b.qend : a.round < b.round;
+}
+
+// heapsort of one read's seeds into (qbeg, qend, round): O(n log n) in place; seeds with the same key are the same piece
+// and bi-interval, so the order between them does not show
+__device__ void sort_seeds(debwt_seed* a, u64 n) {
+    auto sift = [&](u64 r, u64 end) {
+        for (u64 ch; (ch = 2 * r + 1) < end; r = ch) {
+            if (ch + 1 < end && seed_less(a[ch], a[ch + 1])) ++ch;
+            if (!seed_less(a[r], a[ch])) return;
+            const debwt_seed tmp = a[r]; a[r] = a[ch]; a[ch] = tmp;
+        }
+    };
+    for (u64 r = n / 2; r-- > 0;) sift(r, n);
+    for (u64 end = n; end-- > 1;) {
+        const debwt_seed tmp = a[0]; a[0] = a[end]; a[end] = tmp;
+        sift(0, end);
+    }
+}
+
+// The three rounds of BWA-MEM's seeding per read, with the slots, lists and work counter of smem_kernel.  Round 1: Li's
+// outer loop with t = 1, seeds of at least min_len; each one of at least split_len bases and at most split_width
+// occurrences leaves (its middle << 32 | count) in the slot's `mids` list (entry j at [j n_slots]; one per qbeg, so at
+// most the read's length).  Round 2: smem1(middle, count + 1) for each, seeds of at least min_len.  Round 3 (max_mem_intv
+// > 0): from x, forward extension until the first piece [x, i + 1) of more than min_len bases with fewer than
+// max_mem_intv occurrences, a seed if it occurs; on at i + 1 (also after a non-ACGT at i).  The count pass (out ==
+// nullptr) writes the seeds and hits per read; the write pass writes the seeds at out_off, sorts them and gives each its
+// first hit, also into seed_hit.
+__global__ void __launch_bounds__(TPB) seed_kernel(FmView f, const u8* __restrict__ reads, const u64* __restrict__ offs, u64 n_reads,
+                                                  SeedParams o, BiIv* __restrict__ scratch, u64* __restrict__ mids, u64 n_slots,
+                                                  u64 list_cap, unsigned long long* __restrict__ next, u64* __restrict__ counts,
+                                                  u64* __restrict__ hit_counts, const u64* __restrict__ out_off,
+                                                  const u64* __restrict__ hit_off, debwt_seed* __restrict__ out,
+                                                  u64* __restrict__ seed_hit) {
+    const u64 t = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (t >= n_slots) return;
+    BiIv* const list0 = scratch + t;
+    BiIv* const list1 = scratch + list_cap * n_slots + t;
+    u64* const mid = mids + t;
+    for (;;) {
+        const u64 rd = atomicAdd(next, 1ull);
+        if (rd >= n_reads) break;
+        const u8* q = reads + offs[rd];
+        const u32 m = (u32)(offs[rd + 1] - offs[rd]);
+        debwt_seed* w = out ? out + out_off[rd] : nullptr;
+        u64 n = 0, hits = 0, n_mid = 0;
+        auto put = [&](const BiIv& p, u32 beg, u32 end, u32 round) {
+            const u32 nh = (u32)min(p.s, (u64)o.max_occ);
+            if (w) w[n] = debwt_seed{p.k, p.l, p.s, beg, end, 0, nh, round};
+            ++n;
+            hits += nh;
+        };
+        for (u32 x = 0; x < m;) {                                                 // round 1
+            const u32 a = pattern_symbol(q[x]);
+            const u64 ca = base_count(f, a);
+            if (ca == 0) { ++x; continue; }
+            x = smem1(f, q, m, x, a, ca, 1, list0, list1, n_slots, list_cap, [&](const BiIv& p, u32 beg) {
+                const u32 len = (u32)p.end - beg;
+                if (len < o.min_len) return;
+                put(p, beg, (u32)p.end, 1);
+                if (len >= o.split_len && p.s <= o.split_width) mid[n_mid++ * n_slots] = ((u64)((beg + (u32)p.end) >> 1) << 32) | p.s;
+            });
+        }
+        for (u64 j = 0; j < n_mid; ++j) {                                         // round 2
+            const u64 v = mid[j * n_slots];
+            const u32 x = (u32)(v >> 32), a = pattern_symbol(q[x]);
+            smem1(f, q, m, x, a, base_count(f, a), (u64)(u32)v + 1, list0, list1, n_slots, list_cap, [&](const BiIv& p, u32 beg) {
+                if ((u32)p.end - beg >= o.min_len) put(p, beg, (u32)p.end, 2);
+            });
+        }
+        if (o.max_mem_intv > 0)                                                   // round 3
+            for (u32 x = 0; x < m;) {
+                const u32 a = pattern_symbol(q[x]);
+                const u64 ca = base_count(f, a);
+                if (ca == 0) { ++x; continue; }
+                BiIv ik = single_base(f, a, ca, x);
+                u32 next_x = m;
+                for (u32 i = x + 1; i < m; ++i) {
+                    const u32 c = pattern_symbol(q[i]);
+                    if (c > 3u) { next_x = i + 1; break; }
+                    if (ik.s) ik = forward_ext(f, ik, c);                         // an empty interval stays empty
+                    if (ik.s < o.max_mem_intv && i - x >= o.min_len) {
+                        if (ik.s) put(ik, x, i + 1, 3);
+                        next_x = i + 1;
+                        break;
+                    }
+                }
+                x = next_x;
+            }
+        if (w) {
+            sort_seeds(w, n);
+            u64 h = hit_off[rd];
+            for (u64 j = 0; j < n; ++j) {
+                w[j].hit_begin = h;
+                seed_hit[out_off[rd] + j] = h;
+                h += w[j].n_hits;
+            }
+        } else {
+            counts[rd] = n;
+            hit_counts[rd] = hits;
+        }
+    }
+}
+
+// One thread per hit: its seed by binary search over seed_hit (n_seeds + 1 entries), then SA of row + j step (BWA's
+// mem_chain sampling: step = count / max_occ when count > max_occ), then record, strand and forward offset from the R
+// ascending separator positions `seps` of the both-strands text (records R / 2 .. R - 1 are the reverse copies).
+__global__ void __launch_bounds__(TPB) seed_hits_kernel(FmView f, SaView s, const debwt_seed* __restrict__ seeds,
+                                                       const u64* __restrict__ seed_hit, u64 n_seeds, u64 total, u32 max_occ,
+                                                       const u64* __restrict__ seps, u64 R, debwt_seed_hit* __restrict__ out) {
+    const u64 h = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (h >= total) return;
+    const u64 i = upper_bound_u64(seed_hit, 0, n_seeds + 1, h) - 1;
+    const debwt_seed sd = seeds[i];
+    const u64 step = sd.count > max_occ ? sd.count / max_occ : 1;
+    const u64 pos = sa_of(f, s, sd.row + (h - seed_hit[i]) * step);
+    const u64 rec = lower_bound_u64(seps, 0, R, pos);                            // records that end before pos
+    const u64 start = rec ? seps[rec - 1] + 1 : 0, off = pos - start, half = R / 2;
+    const bool rev = rec >= half;
+    out[h] = debwt_seed_hit{pos, rev ? seps[rec] - start - off - (sd.qend - sd.qbeg) : off, (u32)(rev ? rec - half : rec), rev ? 1u : 0u};
 }
 
 FmView view_of(const debwt_ctx* c) {
@@ -591,7 +742,8 @@ void drop_samples(debwt_ctx* c) {
     if (c->d_sa_bits) cudaFree(c->d_sa_bits);
     if (c->d_sa_vals) cudaFree(c->d_sa_vals);
     if (c->d_isa_vals) cudaFree(c->d_isa_vals);
-    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr; c->d_isa_vals = nullptr;
+    if (c->d_seps_sorted) cudaFree(c->d_seps_sorted);
+    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr; c->d_isa_vals = nullptr; c->d_seps_sorted = nullptr;
     c->sa_rate = 0;
 }
 
@@ -1112,6 +1264,160 @@ int debwt_index_smem(debwt_ctx* c, const char* reads, const uint64_t* offsets, u
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
     cudaFree(d); cudaFree(d_scratch); cudaFree(d_out);
+    return 0;
+}
+
+static_assert(sizeof(debwt_seed) == 48, "debwt_seed is 3 u64 + 2 u32 + u64 + 2 u32");
+static_assert(sizeof(debwt_seed_hit) == 24, "debwt_seed_hit is 2 u64 + 2 u32");
+
+// The R separator positions of T, ascending, kept with the SA samples: SA of the rows [N - R, N), which hold the suffixes
+// that start with '#' or '$', sorted on the device.
+static int sorted_separators(debwt_ctx* c) {
+    if (c->d_seps_sorted) return 0;
+    cudaStream_t st = c->st;
+    const u64 R = c->n_rec, n = c->n;
+    std::vector<u64> rows(R);
+    for (u64 i = 0; i < R; ++i) rows[i] = n - R + i;
+    u64 *d_a = nullptr, *d_b = nullptr;
+    void* d_ws = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_a), (R + 2) * 8) != cudaSuccess || cudaMalloc(reinterpret_cast<void**>(&d_b), (R + 2) * 8) != cudaSuccess ||
+        cudaMalloc(&d_ws, sort_workspace_bytes(R, c->sort_cfg)) != cudaSuccess) {
+        cudaGetLastError();
+        if (d_a) cudaFree(d_a);
+        if (d_b) cudaFree(d_b);
+        FAIL("index_seeds: out of device memory for the separator positions");
+    }
+    SortWorkspace ws;
+    sort_workspace_bind(ws, d_ws, R, c->sort_cfg);
+    CUDA_TRY(cudaMemcpyAsync(d_b, rows.data(), R * 8, cudaMemcpyHostToDevice, st));
+    sa_lookup_kernel<<<grid_for(R), TPB, 0, st>>>(view_of(c), sa_view_of(c), d_b, R, d_a);
+    DEBWT_COUNT(1);
+    u64* res = nullptr;
+    const int rc = radix_sort_u64(d_a, d_b, R, ws, st, &res);
+    if (!rc) CUDA_TRY(cudaStreamSynchronize(st));
+    cudaFree(d_ws);
+    cudaFree(res == d_a ? d_b : d_a);
+    if (rc) { cudaFree(res ? res : d_a); return -1; }
+    c->d_seps_sorted = res;
+    return 0;
+}
+
+int debwt_index_seeds(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* opts,
+                      uint64_t* seed_offsets, uint64_t* n_hits_out, debwt_seed* seeds, uint64_t seeds_cap, debwt_seed_hit* hits,
+                      uint64_t hits_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !seed_offsets || !n_hits_out || !opts || (n_reads && !reads) || (seeds && !hits)) FAIL("null argument");
+    const debwt_seed_opts op = *opts;
+    if (op.min_seed_len == 0) FAIL("index_seeds: min_seed_len must be at least 1");
+    if (op.max_occ == 0) FAIL("index_seeds: max_occ must be at least 1");
+    if (!std::isfinite(op.split_factor) || op.split_factor < 0)
+        FAIL("index_seeds: split_factor must be finite and not negative, not " + std::to_string(op.split_factor));
+    const u64* C = c->c_array;
+    const u64 nA = C[1] - C[0], nC = C[2] - C[1], nG = C[3] - C[2], nT = C[4] - C[3];
+    if (nA != nT || nC != nG)
+        FAIL("index_seeds: the text is not closed under reverse complement: it holds A = " + std::to_string(nA) + ", C = " +
+             std::to_string(nC) + ", G = " + std::to_string(nG) + ", T = " + std::to_string(nT) +
+             " bases; build it from every record and its reverse complement (api.both_strands)");
+    if (c->n_rec % 2)
+        FAIL("index_seeds: the text holds " + std::to_string(c->n_rec) +
+             " records; one built from every record and its reverse complement (api.both_strands) holds an even number");
+    const u64 m = n_reads;
+    u64 max_len = 0, longest = 0;
+    for (u64 i = 0; i < m; ++i) {
+        if (offsets[i + 1] < offsets[i]) FAIL("index_seeds: offsets decrease at read " + std::to_string(i));
+        if (offsets[i + 1] - offsets[i] > max_len) { max_len = offsets[i + 1] - offsets[i]; longest = i; }
+    }
+    // per read in flight: two interval lists of len + 1 entries and the middles of the round-1 seeds to split (one per qbeg)
+    const u64 list_cap = max_len + 1, slot_bytes = 2 * list_cap * sizeof(BiIv) + max_len * 8;
+    if (slot_bytes > kSmemScratchBytes)
+        FAIL("index_seeds: read " + std::to_string(longest) + " has " + std::to_string(max_len) + " symbols; its interval lists need " +
+             std::to_string(slot_bytes) + " bytes, more than the " + std::to_string(kSmemScratchBytes) + " bytes of scratch (reads up to " +
+             std::to_string((kSmemScratchBytes - 2 * sizeof(BiIv)) / (2 * sizeof(BiIv) + 8)) + " symbols)");
+    seed_offsets[0] = 0;
+    *n_hits_out = 0;
+    if (m == 0) return 0;
+    SeedParams prm;
+    prm.min_len = op.min_seed_len;
+    prm.max_occ = op.max_occ;
+    const double split = (double)(op.min_seed_len * op.split_factor) + .499;    // bwa: (int)(min_seed_len * split_factor + .499)
+    prm.split_len = split >= 18446744073709551615.0 ? ~0ull : (u64)split;
+    prm.split_width = op.split_width;
+    prm.max_mem_intv = op.max_mem_intv;
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t st = c->st;
+    int sms = 0, per_sm = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxThreadsPerMultiProcessor, c->device));
+    const u64 n_slots = std::min<u64>({(u64)sms * (u64)per_sm, kSmemScratchBytes / slot_bytes, m});
+    const u64 bytes = offsets[m], nb = (m + TPB - 1) / TPB, words = (bytes + 16 + 7) / 8;
+    // one block: reads | offsets (m + 1) | seed counts (m) | seed offsets (m + 1) | hit counts (m) | hit offsets (m + 1) |
+    // block totals (nb) | their scan (nb + 1) | counter
+    u64* d = nullptr;
+    BiIv* d_scratch = nullptr;
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d), (words + 5 * m + 2 * nb + 5) * 8));
+    if (cudaMalloc(reinterpret_cast<void**>(&d_scratch), n_slots * slot_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d);
+        FAIL("index_seeds: out of device memory for " + std::to_string(n_slots * slot_bytes) + " bytes of scratch");
+    }
+    u64* d_mids = reinterpret_cast<u64*>(d_scratch + 2 * list_cap * n_slots);
+    u8* d_r = reinterpret_cast<u8*>(d);
+    u64 *d_o = d + words, *d_cnt = d_o + m + 1, *d_off = d_cnt + m, *d_hcnt = d_off + m + 1, *d_hoff = d_hcnt + m, *d_tot = d_hoff + m + 1,
+        *d_base = d_tot + nb;
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(d_base + nb + 1);
+    auto release = [&]() { cudaFree(d); cudaFree(d_scratch); };
+    CUDA_TRY(cudaMemcpyAsync(d_r, reads, bytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_o, offsets, (m + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
+    const FmView f = view_of(c);
+    const unsigned grid = grid_for(n_slots);
+    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, prm, d_scratch, d_mids, n_slots, list_cap, d_next, d_cnt, d_hcnt, nullptr, nullptr,
+                                      nullptr, nullptr);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_base, d_off);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, d_base, d_hoff);
+    DEBWT_COUNT(7);
+    u64 total_hits = 0;
+    CUDA_TRY(cudaMemcpyAsync(seed_offsets, d_off, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&total_hits, d_hoff + m, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    *n_hits_out = total_hits;
+    const u64 total = seed_offsets[m];
+    if (!seeds || total == 0) { release(); return 0; }                         // size query
+    if (total > seeds_cap || total_hits > hits_cap) {
+        release();
+        FAIL("index_seeds: the reads have " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits; seeds holds " +
+             std::to_string(seeds_cap) + " and hits " + std::to_string(hits_cap));
+    }
+    if (sorted_separators(c)) { release(); return -1; }
+    // the seeds | their first hits (total + 1) | the hits
+    char* d_out = nullptr;
+    const u64 out_bytes = total * sizeof(debwt_seed) + (total + 1) * 8 + total_hits * sizeof(debwt_seed_hit);
+    if (cudaMalloc(reinterpret_cast<void**>(&d_out), out_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        release();
+        FAIL("index_seeds: out of device memory for " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits");
+    }
+    debwt_seed* d_seeds = reinterpret_cast<debwt_seed*>(d_out);
+    u64* d_seed_hit = reinterpret_cast<u64*>(d_seeds + total);
+    debwt_seed_hit* d_hits = reinterpret_cast<debwt_seed_hit*>(d_seed_hit + total + 1);
+    CUDA_TRY(cudaMemcpyAsync(d_seed_hit + total, d_hoff + m, 8, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
+    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, prm, d_scratch, d_mids, n_slots, list_cap, d_next, nullptr, nullptr, d_off, d_hoff,
+                                      d_seeds, d_seed_hit);
+    seed_hits_kernel<<<grid_for(total_hits), TPB, 0, st>>>(f, sa_view_of(c), d_seeds, d_seed_hit, total, total_hits, op.max_occ,
+                                                           c->d_seps_sorted, c->n_rec, d_hits);
+    DEBWT_COUNT(2);
+    CUDA_TRY(cudaMemcpyAsync(seeds, d_seeds, total * sizeof(debwt_seed), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(hits, d_hits, total_hits * sizeof(debwt_seed_hit), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    release();
+    cudaFree(d_out);
     return 0;
 }
 

@@ -223,6 +223,48 @@ typedef struct debwt_smem {
 } debwt_smem;
 int debwt_index_smem(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads, uint32_t min_len,
                      uint64_t* smem_offsets /* n_reads + 1 */, debwt_smem* smems, uint64_t smems_cap);
+/* BWA-MEM's whole seeding step (bwa's mem_collect_intv and the SA sampling of mem_chain) over a text that holds both
+   strands, as for debwt_index_smem, from reads to located seed hits.  Options are bwa's -k, -r, split_width, -y and -c
+   (defaults 19, 1.5, 10, 20, 500).  smem1(x, t) is bwa's bwt_smem1a(x, min_intv = t, max_intv = 0); a base that does not
+   occur in T is stepped over (x + 1) in every round.  Per read of length m:
+     round 1: Li's loop x = smem1(x, 1) (the SMEMs of debwt_index_smem); seeds of at least min_seed_len bases;
+     round 2: with split_len = (int)(min_seed_len * split_factor + .499) (float product), for every round-1 seed [b, e)
+              with e - b >= split_len and count <= split_width, smem1((b + e) >> 1, count + 1); seeds of at least
+              min_seed_len bases (duplicates stay, as in bwa);
+     round 3 (only when max_mem_intv > 0): from x, extend forward to the first i with i - x >= min_seed_len and
+              count(read[x, i + 1)) < max_mem_intv: [x, i + 1) is a seed if its count is > 0; go on at i + 1.  A non-ACGT
+              at i ends the attempt without a seed (on at i + 1); the end of the read ends the round.
+   A read's seeds are seeds[seed_offsets[i] .. seed_offsets[i + 1]), in ascending (qbeg, qend, round).  Seed rows
+   [row, row + count) start with read[qbeg, qend) (count covers both strands), rc_row is the first row of its reverse
+   complement.  A seed has n_hits = min(count, max_occ) hits, hits[hit_begin .. hit_begin + n_hits): hit j is
+   SA[row + j step], step = count > max_occ ? count / max_occ : 1, with the record (0 .. R/2 - 1 of the R records), the
+   strand (0 forward, 1 reverse: records R/2 .. R - 1) and the offset of the hit's first base on the forward strand
+   (python: api.strand_offsets).  Seeds hold A, C, G, T only, so no hit spans a separator.
+   seed_offsets[n_reads + 1] and *n_hits_out (all hits) are always written; seeds == NULL is a size query.  More seeds
+   than seeds_cap or more hits than hits_cap fails, writes nothing into seeds / hits, and names both totals.  Needs
+   debwt_index_sample_sa (the first call after sampling also sorts the separator positions on the device and keeps them
+   with the samples).  Fails, writing nothing, on: no samples, an unbalanced text (as debwt_index_smem) or an odd number
+   of records, min_seed_len = 0, max_occ = 0, a negative or non-finite split_factor, decreasing offsets, NULL arguments
+   (hits may be NULL only with seeds), or a read too long for the 1 GiB of scratch (72 len + 64 bytes per read in flight;
+   reads up to 14.9 Mbp; the message names the read and the limit).  n_reads = 0 only writes seed_offsets[0] = 0 and
+   *n_hits_out = 0. */
+typedef struct debwt_seed_opts {
+    uint32_t min_seed_len, split_width, max_mem_intv, max_occ;
+    float split_factor;
+} debwt_seed_opts;
+typedef struct debwt_seed {
+    uint64_t row, rc_row, count;   /* as debwt_smem */
+    uint32_t qbeg, qend;
+    uint64_t hit_begin;            /* its hits are hits[hit_begin, hit_begin + n_hits) */
+    uint32_t n_hits, round;        /* min(count, max_occ); 1, 2 or 3 */
+} debwt_seed;                      /* 48 bytes */
+typedef struct debwt_seed_hit {
+    uint64_t pos, offset;          /* text position; offset of the hit's first base on the forward strand of its record */
+    uint32_t record, strand;       /* record 0 .. R/2 - 1; strand 0 forward, 1 reverse */
+} debwt_seed_hit;                  /* 24 bytes */
+int debwt_index_seeds(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* opts,
+                      uint64_t* seed_offsets /* n_reads + 1 */, uint64_t* n_hits_out, debwt_seed* seeds, uint64_t seeds_cap,
+                      debwt_seed_hit* hits, uint64_t hits_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
