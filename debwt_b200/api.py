@@ -268,6 +268,37 @@ class BwtBuilder:
             check(lib().debwt_index_seeds(*args, _ptr(seeds), seeds.size, _ptr(hits), hits.size))
         return so, seeds, hits
 
+    def chains(self, reads: Sequence, min_len: int = 19, split_factor: float = 1.5, split_width: int = 10, max_mem_intv: int = 20,
+               max_occ: int = 500, w: int = 100, max_chain_gap: int = 10000, min_chain_weight: int = 0, mask_level: float = 0.5,
+               drop_ratio: float = 0.5, max_chain_extend: int = 1 << 30) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(offsets u64[m + 1], chains CHAIN_DTYPE[total], chain_seeds CHAIN_SEED_DTYPE[all chain seeds]): BWA-MEM's chains of
+        read i (bwa's mem_chain and mem_chain_flt over the seeds of `seeds` with the same seed options; bwa's w,
+        max_chain_gap, -W, mask_level, -D, max_chain_extend) are chains[offsets[i]:offsets[i+1]], in the filter's order;
+        chain c has chain_seeds[c.seed_begin : c.seed_begin + c.n_seeds] in insertion order, in bwa's coordinate
+        (`bwa_rbeg`).  The text must hold both strands (`both_strands`); needs sample_sa."""
+        rs = [r.encode() if isinstance(r, str) else bytes(r) for r in reads]
+        offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(r) for r in rs])
+        blob = np.frombuffer(b"".join(rs) + b"\0", dtype=np.uint8)
+        for name, v in (("min_len", min_len), ("split_width", split_width), ("max_mem_intv", max_mem_intv), ("max_occ", max_occ)):
+            if not 0 <= v < 1 << 32:
+                raise DebwtError(f"chains: {name} = {v} is not a 32-bit unsigned integer")
+        for name, v in (("w", w), ("max_chain_gap", max_chain_gap), ("min_chain_weight", min_chain_weight),
+                        ("max_chain_extend", max_chain_extend)):
+            if not -(1 << 31) <= v < 1 << 31:
+                raise DebwtError(f"chains: {name} = {v} is not a 32-bit signed integer")
+        so = SeedOpts(min_len, split_width, max_mem_intv, max_occ, split_factor)
+        co = ChainOpts(w, max_chain_gap, min_chain_weight, max_chain_extend, mask_level, drop_ratio)
+        co_offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        ns = c_u64()
+        args = (self._h, _ptr(blob), _ptr(offs), len(rs), ctypes.addressof(so), ctypes.addressof(co), _ptr(co_offs), ctypes.addressof(ns))
+        check(lib().debwt_index_chains(*args, c_p(0), 0, c_p(0), 0))
+        chains = np.zeros(int(co_offs[-1]), dtype=CHAIN_DTYPE)
+        seeds = np.zeros(int(ns.value), dtype=CHAIN_SEED_DTYPE)
+        if chains.size:
+            check(lib().debwt_index_chains(*args, _ptr(chains), chains.size, _ptr(seeds), seeds.size))
+        return co_offs, chains, seeds
+
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""
         bad, ms = c_u64(), ctypes.c_float()
@@ -340,6 +371,19 @@ class SeedOpts(ctypes.Structure):
                 ("max_occ", ctypes.c_uint32), ("split_factor", ctypes.c_float)]
 
 
+# ---- BWA-MEM seed chaining over both strands (debwt_index_chains) ----------------------------------------------------
+CHAIN_DTYPE = np.dtype([("pos", np.uint64), ("seed_begin", np.uint64), ("n_seeds", np.uint32), ("weight", np.uint32),
+                        ("record", np.uint32), ("strand", np.uint32), ("kept", np.uint32), ("frac_rep", np.float32)],
+                       align=True)                     # debwt_chain
+CHAIN_SEED_DTYPE = np.dtype([("rbeg", np.uint64), ("qbeg", np.uint32), ("len", np.uint32)], align=True)  # debwt_chain_seed
+
+
+class ChainOpts(ctypes.Structure):
+    """debwt_chain_opts of include/debwt_b200.h"""
+    _fields_ = [("w", ctypes.c_int32), ("max_chain_gap", ctypes.c_int32), ("min_chain_weight", ctypes.c_int32),
+                ("max_chain_extend", ctypes.c_int32), ("mask_level", ctypes.c_float), ("drop_ratio", ctypes.c_float)]
+
+
 _COMP = bytes.maketrans(b"ACGT", b"TGCA")
 
 
@@ -372,6 +416,21 @@ def strand_offsets(positions, length: int, seps) -> tuple[np.ndarray, np.ndarray
         raise ValueError(f"a hit of {length} symbols runs past the end of its record")
     rev = rec >= R
     return rec % R, rev.astype(np.int8), np.where(rev, lens[rec] - off - length, off)
+
+
+def bwa_rbeg(record, strand, offset, length, seps) -> np.ndarray:
+    """bwa's forward-reverse coordinate (int64) of hits of `length` bases at (record, strand, forward offset) of a
+    `both_strands` text with separators `seps`: with l_pac = (N - R) / 2 forward bases and F[r] the bases of the forward
+    records before r, F[r] + offset on strand 0 (the text position - r), 2 l_pac - (F[r] + offset + length) on strand 1."""
+    seps = np.asarray(seps, dtype=np.int64)
+    if seps.size % 2:
+        raise ValueError(f"{seps.size} records: a both_strands text has an even number")
+    R = seps.size
+    l_pac = (int(seps[-1]) + 1 - R) // 2
+    F = np.concatenate(([0], seps[:R // 2 - 1] + 1 - np.arange(1, R // 2))).astype(np.int64)
+    rec = np.asarray(record, dtype=np.int64)
+    f = F[rec] + np.asarray(offset, dtype=np.int64)
+    return np.where(np.asarray(strand) != 0, 2 * l_pac - (f + np.asarray(length, dtype=np.int64)), f)
 
 
 # ---- per-kernel entry points (parity tests) -------------------------------------------------------

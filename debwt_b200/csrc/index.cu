@@ -13,6 +13,8 @@
 #include <algorithm>
 #include <cmath>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "ctx.cuh"
@@ -726,6 +728,291 @@ __global__ void __launch_bounds__(TPB) seed_hits_kernel(FmView f, SaView s, cons
     out[h] = debwt_seed_hit{pos, rev ? seps[rec] - start - off - (sd.qend - sd.qbeg) : off, (u32)(rev ? rec - half : rec), rev ? 1u : 0u};
 }
 
+// ---- BWA-MEM seed chaining (mem_chain, mem_chain_flt) ----------------------------------------------------------------
+struct ChainParams {
+    long long w, max_chain_gap, max_chain_extend, min_seed_len;
+    u32 min_chain_weight, max_occ;
+    float mask_level, drop_ratio;
+    u64 l_pac;
+};
+
+// One chain after the weight pass, at its ordinal in chain-set order: query span, weight, seeds, slot, bwa's first and kept
+struct ChainRec {
+    u32 beg, end, w, n, slot;
+    int first;
+    u32 kept;
+};
+
+// Per-hit scratch; a read with hits [hb, hb + H) owns entries [hb, hb + H) of each array (indices inside are read-local
+// u32: a read's hits stay below 2^32, whose 24-byte hits alone would not fit the device) and bitmap words from
+// hb / 64 + read, summary words from hb / 4096 + read.
+struct ChainScratch {
+    debwt_chain_seed* cs;   // hit h as a chain seed, in hit order
+    u64* key;               // slot p: the p-th smallest (rbeg, hit) pair's rbeg; after chaining the filter's sort keys
+    u32* idx;               // slot p: that pair's hit, the hit that creates the chain of slot p
+    u32* nxt;               // hit h: the next seed of its chain (NIL at the end)
+    u32* tail;              // slot p: the last seed of its chain
+    u32* list;              // the filter's kept list
+    ChainRec* rec;          // chains in chain-set order
+    u64* bits;              // bit p: slot p holds a chain
+    u64* summary;           // bit w: bitmap word w is not zero
+};
+
+// bwa's coordinate of a hit of `len` bases: F[r] + o forward, 2 l_pac - (F[r] + o + len) reverse (F[r] = seps[r-1] + 1 - r)
+__device__ __forceinline__ u64 bwa_rbeg(const debwt_seed_hit& h, u32 len, const u64* __restrict__ seps, u64 l_pac) {
+    const u64 f = (h.record ? seps[h.record - 1] + 1 - h.record : 0) + h.offset;
+    return h.strand ? 2 * l_pac - (f + len) : f;
+}
+
+// heapsort of (key, idx) pairs by (key, idx); the pairs are distinct
+__device__ void sort_pairs(u64* key, u32* idx, u64 n) {
+    auto less = [&](u64 a, u64 b) { return key[a] != key[b] ? key[a] < key[b] : idx[a] < idx[b]; };
+    auto swap = [&](u64 a, u64 b) {
+        const u64 k = key[a]; key[a] = key[b]; key[b] = k;
+        const u32 i = idx[a]; idx[a] = idx[b]; idx[b] = i;
+    };
+    auto sift = [&](u64 r, u64 end) {
+        for (u64 ch; (ch = 2 * r + 1) < end; r = ch) {
+            if (ch + 1 < end && less(ch, ch + 1)) ++ch;
+            if (!less(r, ch)) return;
+            swap(r, ch);
+        }
+    };
+    for (u64 r = n / 2; r-- > 0;) sift(r, n);
+    for (u64 end = n; end-- > 1;) {
+        swap(0, end);
+        sift(0, end);
+    }
+}
+
+// heapsort of distinct u64 keys
+__device__ void sort_keys(u64* a, u64 n) {
+    auto sift = [&](u64 r, u64 end) {
+        for (u64 ch; (ch = 2 * r + 1) < end; r = ch) {
+            if (ch + 1 < end && a[ch] < a[ch + 1]) ++ch;
+            if (a[r] >= a[ch]) return;
+            const u64 t = a[r]; a[r] = a[ch]; a[ch] = t;
+        }
+    };
+    for (u64 r = n / 2; r-- > 0;) sift(r, n);
+    for (u64 end = n; end-- > 1;) {
+        const u64 t = a[0]; a[0] = a[end]; a[end] = t;
+        sift(0, end);
+    }
+}
+
+__device__ __forceinline__ int top_bit(u64 x) { return 63 - __clzll((long long)x); }
+__device__ __forceinline__ int low_bit(u64 x) { return __ffsll((long long)x) - 1; }
+
+// the greatest occupied slot below x, or -1; bits / summary are the read's words
+__device__ long long slot_before(const u64* __restrict__ bits, const u64* __restrict__ summary, u64 x) {
+    if (x == 0) return -1;
+    const u64 q = x - 1, w = q >> 6;
+    const u64 m = bits[w] & (~0ull >> (63 - (q & 63)));
+    if (m) return (long long)(w * 64 + top_bit(m));
+    for (long long sw = (long long)(w >> 6), below = (long long)(w & 63); sw >= 0; --sw, below = 64) {
+        const u64 s = summary[sw] & (below == 64 ? ~0ull : (1ull << below) - 1);
+        if (s) {
+            const u64 w2 = (u64)sw * 64 + top_bit(s);
+            return (long long)(w2 * 64 + top_bit(bits[w2]));
+        }
+    }
+    return -1;
+}
+
+// the least occupied slot at or above x (one exists)
+__device__ u64 slot_from(const u64* __restrict__ bits, const u64* __restrict__ summary, u64 x) {
+    const u64 w = x >> 6;
+    const u64 m = bits[w] & (~0ull << (x & 63));
+    if (m) return w * 64 + low_bit(m);
+    for (u64 sw = w >> 6, from = (w & 63) + 1;; ++sw, from = 0) {
+        const u64 s = from == 64 ? 0 : summary[sw] & (~0ull << from);
+        if (s) {
+            const u64 w2 = sw * 64 + low_bit(s);
+            return w2 * 64 + low_bit(bits[w2]);
+        }
+    }
+}
+
+// One thread per read in flight, reads from the work counter `next`: the read's hits become chain seeds, its (rbeg, hit)
+// pairs are sorted once, and a chain lives in the slot of the hit that created it, so `lower` is the chain of the first
+// occupied slot of the rbeg group of the greatest occupied slot below upper_bound(rbeg).  Then the weights, the sort and
+// bwa's filter.  Writes per read the kept chains and their seeds (for the scans), the chains after the weight pass and
+// frac_rep; the chains and the filter's order stay in the scratch for chain_write_kernel.
+__global__ void __launch_bounds__(TPB) chain_kernel(const u64* __restrict__ offs, u64 n_reads, const debwt_seed* __restrict__ seeds,
+                                                   const u64* __restrict__ seed_off, const debwt_seed_hit* __restrict__ hits,
+                                                   const u64* __restrict__ hit_off, const u64* __restrict__ seps, ChainParams o,
+                                                   ChainScratch s, unsigned long long* __restrict__ next, u64* __restrict__ chain_cnt,
+                                                   u64* __restrict__ seed_cnt, u32* __restrict__ n_sorted, float* __restrict__ frac) {
+    for (;;) {
+        const u64 rd = atomicAdd(next, 1ull);
+        if (rd >= n_reads) break;
+        const u64 hb = hit_off[rd], H = hit_off[rd + 1] - hb, len = offs[rd + 1] - offs[rd];
+        const debwt_seed* sd = seeds + seed_off[rd];
+        const u64 n_sd = seed_off[rd + 1] - seed_off[rd];
+        // frac_rep: bwa's sweep over the seeds above max_occ
+        u64 b = 0, e = 0, l_rep = 0;
+        for (u64 j = 0; j < n_sd; ++j) {
+            if (sd[j].count <= o.max_occ) continue;
+            if (sd[j].qbeg > e) { l_rep += e - b; b = sd[j].qbeg; e = sd[j].qend; }
+            else e = max(e, (u64)sd[j].qend);
+        }
+        l_rep += e - b;
+        frac[rd] = len ? (float)l_rep / (float)len : 0.f;
+        debwt_chain_seed* cs = s.cs + hb;
+        u64* key = s.key + hb;
+        u32 *idx = s.idx + hb, *nxt = s.nxt + hb, *tail = s.tail + hb;
+        const debwt_seed_hit* ht = hits + hb;
+        for (u64 j = 0, h = 0; j < n_sd; ++j) {
+            const u32 l = sd[j].qend - sd[j].qbeg;
+            for (u32 k = 0; k < sd[j].n_hits; ++k, ++h) {
+                const u64 r = bwa_rbeg(ht[h], l, seps, o.l_pac);
+                cs[h] = debwt_chain_seed{r, sd[j].qbeg, l};
+                key[h] = r;
+                idx[h] = (u32)h;
+            }
+        }
+        sort_pairs(key, idx, H);
+        const u64 nw = (H + 63) / 64;
+        u64* bits = s.bits + hb / 64 + rd;
+        u64* summary = s.summary + hb / 4096 + rd;
+        for (u64 w = 0; w < nw; ++w) bits[w] = 0;
+        for (u64 w = 0; w < (nw + 63) / 64; ++w) summary[w] = 0;
+        // mem_chain
+        for (u32 h = 0; h < H; ++h) {
+            const debwt_chain_seed p = cs[h];
+            const u64 lb = lower_bound_u64(key, 0, H, p.rbeg), ub = upper_bound_u64(key, lb, H, p.rbeg);
+            const long long pred = slot_before(bits, summary, ub);
+            bool merged = false;
+            if (pred >= 0) {
+                const u64 pk = key[pred];
+                const u64 c = slot_from(bits, summary, pk == p.rbeg ? lb : lower_bound_u64(key, 0, (u64)pred, pk));
+                const debwt_chain_seed first = cs[idx[c]], last = cs[tail[c]];
+                if (ht[h].record == ht[idx[c]].record) {
+                    if (p.qbeg >= first.qbeg && p.qbeg + p.len <= last.qbeg + last.len && p.rbeg >= first.rbeg &&
+                        p.rbeg + p.len <= last.rbeg + last.len) {
+                        merged = true;                                            // contained: not added
+                    } else if (!((last.rbeg < o.l_pac || first.rbeg < o.l_pac) && p.rbeg >= o.l_pac)) {
+                        const long long x = (long long)p.qbeg - (long long)last.qbeg, y = (long long)(p.rbeg - last.rbeg);
+                        if (y >= 0 && x - y <= o.w && y - x <= o.w && x - (long long)last.len < o.max_chain_gap &&
+                            y - (long long)last.len < o.max_chain_gap) {
+                            nxt[tail[c]] = h;
+                            nxt[h] = NIL;
+                            tail[c] = h;
+                            merged = true;
+                        }
+                    }
+                }
+            }
+            if (!merged) {                                                        // a new chain in the slot of (rbeg, h)
+                u64 lo = lb, hi = ub;
+                while (lo < hi) {
+                    const u64 mid = lo + ((hi - lo) >> 1);
+                    if (idx[mid] < h) lo = mid + 1; else hi = mid;
+                }
+                bits[lo >> 6] |= 1ull << (lo & 63);
+                summary[lo >> 12] |= 1ull << ((lo >> 6) & 63);
+                tail[lo] = h;
+                nxt[h] = NIL;
+            }
+        }
+        // mem_chain_weight in chain-set order; chains below min_chain_weight are dropped
+        ChainRec* rec = s.rec + hb;
+        u32 nc = 0;
+        for (u64 w = 0; w < nw; ++w)
+            for (u64 m = bits[w]; m; m &= m - 1) {
+                const u32 p = (u32)(w * 64 + low_bit(m));
+                u64 qe = 0, re = 0, wq = 0, wr = 0;
+                u32 n = 0;
+                for (u32 h = idx[p]; h != NIL; h = nxt[h], ++n) {
+                    const debwt_chain_seed q = cs[h];
+                    wq += q.qbeg >= qe ? q.len : (q.qbeg + (u64)q.len > qe ? q.qbeg + (u64)q.len - qe : 0);
+                    qe = max(qe, q.qbeg + (u64)q.len);
+                    wr += q.rbeg >= re ? q.len : (q.rbeg + q.len > re ? q.rbeg + q.len - re : 0);
+                    re = max(re, (u64)(q.rbeg + q.len));
+                }
+                const u32 wt = (u32)min(wq, wr);
+                if (wt < o.min_chain_weight) continue;
+                const debwt_chain_seed f = cs[idx[p]], l = cs[tail[p]];
+                rec[nc] = ChainRec{f.qbeg, l.qbeg + l.len, wt, n, p, -1, 0};
+                key[nc] = (u64)(0xFFFFFFFFu - wt) << 32 | nc;                   // weight descending, then chain-set order
+                ++nc;
+            }
+        sort_keys(key, nc);
+        // mem_chain_flt
+        u32* list = s.list + hb;
+        u64 n_list = 0;
+        if (nc) {
+            rec[(u32)key[0]].kept = 3;
+            list[n_list++] = 0;
+        }
+        for (u32 i = 1; i < nc; ++i) {
+            ChainRec& a = rec[(u32)key[i]];
+            bool large = false;
+            u64 k = 0;
+            for (; k < n_list; ++k) {
+                const u32 j = list[k];
+                ChainRec& c = rec[(u32)key[j]];
+                const u32 bm = max(a.beg, c.beg), em = min(a.end, c.end);
+                if (em <= bm) continue;
+                const long long min_l = min(a.end - a.beg, c.end - c.beg);
+                if ((float)(em - bm) >= (float)min_l * o.mask_level && min_l < o.max_chain_gap) {
+                    large = true;
+                    if (c.first < 0) c.first = (int)i;
+                    if ((float)a.w < (float)c.w * o.drop_ratio && (long long)c.w - (long long)a.w >= 2 * o.min_seed_len) break;
+                }
+            }
+            if (k == n_list) {
+                list[n_list++] = i;
+                a.kept = large ? 2 : 3;
+            }
+        }
+        for (u64 k = 0; k < n_list; ++k) {
+            const int f = rec[(u32)key[list[k]]].first;
+            if (f >= 0) rec[(u32)key[f]].kept = 1;
+        }
+        u32 i = 0;
+        for (long long cnt = 0; i < nc; ++i) {
+            const u32 kp = rec[(u32)key[i]].kept;
+            if (kp == 0 || kp == 3) continue;
+            if (++cnt >= o.max_chain_extend) break;
+        }
+        for (; i < nc; ++i)
+            if (rec[(u32)key[i]].kept < 3) rec[(u32)key[i]].kept = 0;
+        u64 kept = 0, kept_seeds = 0;
+        for (u32 j = 0; j < nc; ++j) {
+            const ChainRec& a = rec[(u32)key[j]];
+            if (a.kept) { ++kept; kept_seeds += a.n; }
+        }
+        chain_cnt[rd] = kept;
+        seed_cnt[rd] = kept_seeds;
+        n_sorted[rd] = nc;
+    }
+}
+
+// One thread per read: its kept chains in filter order at chain_off, their seeds (list order) at cseed_off
+__global__ void __launch_bounds__(TPB) chain_write_kernel(u64 n_reads, const debwt_seed_hit* __restrict__ hits, const u64* __restrict__ hit_off,
+                                                         ChainScratch s, const u32* __restrict__ n_sorted, const float* __restrict__ frac,
+                                                         const u64* __restrict__ chain_off, const u64* __restrict__ cseed_off,
+                                                         debwt_chain* __restrict__ chains, debwt_chain_seed* __restrict__ chain_seeds) {
+    const u64 rd = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (rd >= n_reads) return;
+    const u64 hb = hit_off[rd];
+    const debwt_chain_seed* cs = s.cs + hb;
+    const u64* key = s.key + hb;
+    const u32 *idx = s.idx + hb, *nxt = s.nxt + hb;
+    const ChainRec* rec = s.rec + hb;
+    u64 o = chain_off[rd], so = cseed_off[rd];
+    for (u32 i = 0; i < n_sorted[rd]; ++i) {
+        const ChainRec a = rec[(u32)key[i]];
+        if (!a.kept) continue;
+        const u32 h0 = idx[a.slot];
+        const debwt_seed_hit& ht = hits[hb + h0];
+        chains[o++] = debwt_chain{cs[h0].rbeg, so, a.n, a.w, ht.record, ht.strand, a.kept, frac[rd]};
+        for (u32 h = h0; h != NIL; h = nxt[h]) chain_seeds[so++] = cs[h];
+    }
+}
+
 FmView view_of(const debwt_ctx* c) {
     FmView f;
     f.bwt = c->d_bwt; f.spec = c->d_spec_bits; f.occ = c->d_occ; f.sharp = c->d_sharp_sorted;
@@ -1272,7 +1559,7 @@ static_assert(sizeof(debwt_seed_hit) == 24, "debwt_seed_hit is 2 u64 + 2 u32");
 
 // The R separator positions of T, ascending, kept with the SA samples: SA of the rows [N - R, N), which hold the suffixes
 // that start with '#' or '$', sorted on the device.
-static int sorted_separators(debwt_ctx* c) {
+static int sorted_separators(debwt_ctx* c, const char* name) {
     if (c->d_seps_sorted) return 0;
     cudaStream_t st = c->st;
     const u64 R = c->n_rec, n = c->n;
@@ -1285,7 +1572,7 @@ static int sorted_separators(debwt_ctx* c) {
         cudaGetLastError();
         if (d_a) cudaFree(d_a);
         if (d_b) cudaFree(d_b);
-        FAIL("index_seeds: out of device memory for the separator positions");
+        FAIL(std::string(name) + ": out of device memory for the separator positions");
     }
     SortWorkspace ws;
     sort_workspace_bind(ws, d_ws, R, c->sort_cfg);
@@ -1302,40 +1589,67 @@ static int sorted_separators(debwt_ctx* c) {
     return 0;
 }
 
-int debwt_index_seeds(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* opts,
-                      uint64_t* seed_offsets, uint64_t* n_hits_out, debwt_seed* seeds, uint64_t seeds_cap, debwt_seed_hit* hits,
-                      uint64_t hits_cap) {
-    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
-    if (!offsets || !seed_offsets || !n_hits_out || !opts || (n_reads && !reads) || (seeds && !hits)) FAIL("null argument");
-    const debwt_seed_opts op = *opts;
-    if (op.min_seed_len == 0) FAIL("index_seeds: min_seed_len must be at least 1");
-    if (op.max_occ == 0) FAIL("index_seeds: max_occ must be at least 1");
+}  // extern "C"
+
+// The device buffers of one seeding run, freed with it
+struct SeedRun {
+    u64* d = nullptr;                 // reads | offsets | seed counts | seed offsets | hit counts | hit offsets | block sums
+    BiIv* scratch = nullptr;
+    char* out = nullptr;              // the seeds | their first hits (total + 1) | the hits
+    u64 *d_o = nullptr, *d_off = nullptr, *d_hoff = nullptr, *d_tot = nullptr, *d_base = nullptr;
+    unsigned long long* d_next = nullptr;
+    debwt_seed* seeds = nullptr;
+    debwt_seed_hit* hits = nullptr;
+    u64 total = 0, total_hits = 0;
+    SeedRun() = default;
+    SeedRun(const SeedRun&) = delete;
+    ~SeedRun() {
+        if (d) cudaFree(d);
+        if (scratch) cudaFree(scratch);
+        if (out) cudaFree(out);
+    }
+};
+
+// The input checks of debwt_index_seeds after its NULL checks; `name` starts the messages.  max_len: the longest read.
+static int check_seed_input(const debwt_ctx* c, const char* name, const uint64_t* offsets, u64 m, const debwt_seed_opts& op,
+                            u64& max_len) {
+    const std::string nm(name);
+    if (op.min_seed_len == 0) FAIL(nm + ": min_seed_len must be at least 1");
+    if (op.max_occ == 0) FAIL(nm + ": max_occ must be at least 1");
     if (!std::isfinite(op.split_factor) || op.split_factor < 0)
-        FAIL("index_seeds: split_factor must be finite and not negative, not " + std::to_string(op.split_factor));
+        FAIL(nm + ": split_factor must be finite and not negative, not " + std::to_string(op.split_factor));
     const u64* C = c->c_array;
     const u64 nA = C[1] - C[0], nC = C[2] - C[1], nG = C[3] - C[2], nT = C[4] - C[3];
     if (nA != nT || nC != nG)
-        FAIL("index_seeds: the text is not closed under reverse complement: it holds A = " + std::to_string(nA) + ", C = " +
+        FAIL(nm + ": the text is not closed under reverse complement: it holds A = " + std::to_string(nA) + ", C = " +
              std::to_string(nC) + ", G = " + std::to_string(nG) + ", T = " + std::to_string(nT) +
              " bases; build it from every record and its reverse complement (api.both_strands)");
     if (c->n_rec % 2)
-        FAIL("index_seeds: the text holds " + std::to_string(c->n_rec) +
+        FAIL(nm + ": the text holds " + std::to_string(c->n_rec) +
              " records; one built from every record and its reverse complement (api.both_strands) holds an even number");
-    const u64 m = n_reads;
-    u64 max_len = 0, longest = 0;
+    u64 longest = 0;
+    max_len = 0;
     for (u64 i = 0; i < m; ++i) {
-        if (offsets[i + 1] < offsets[i]) FAIL("index_seeds: offsets decrease at read " + std::to_string(i));
+        if (offsets[i + 1] < offsets[i]) FAIL(nm + ": offsets decrease at read " + std::to_string(i));
         if (offsets[i + 1] - offsets[i] > max_len) { max_len = offsets[i + 1] - offsets[i]; longest = i; }
     }
     // per read in flight: two interval lists of len + 1 entries and the middles of the round-1 seeds to split (one per qbeg)
-    const u64 list_cap = max_len + 1, slot_bytes = 2 * list_cap * sizeof(BiIv) + max_len * 8;
+    const u64 slot_bytes = 2 * (max_len + 1) * sizeof(BiIv) + max_len * 8;
     if (slot_bytes > kSmemScratchBytes)
-        FAIL("index_seeds: read " + std::to_string(longest) + " has " + std::to_string(max_len) + " symbols; its interval lists need " +
+        FAIL(nm + ": read " + std::to_string(longest) + " has " + std::to_string(max_len) + " symbols; its interval lists need " +
              std::to_string(slot_bytes) + " bytes, more than the " + std::to_string(kSmemScratchBytes) + " bytes of scratch (reads up to " +
              std::to_string((kSmemScratchBytes - 2 * sizeof(BiIv)) / (2 * sizeof(BiIv) + 8)) + " symbols)");
-    seed_offsets[0] = 0;
-    *n_hits_out = 0;
-    if (m == 0) return 0;
+    return 0;
+}
+
+// The seeding of debwt_index_seeds for m >= 1 checked reads, leaving everything in r: the count pass and the two scans
+// (seed_offsets, when given, receives the seed offsets), then proceed(total seeds, total hits): 1 goes on to the write
+// pass and the hit lookups, 0 stops there, -1 fails the call.
+template <class Proceed>
+static int run_seeds(debwt_ctx* c, const char* name, const char* reads, const uint64_t* offsets, u64 m, const debwt_seed_opts& op,
+                     u64 max_len, uint64_t* seed_offsets, SeedRun& r, Proceed&& proceed) {
+    const std::string nm(name);
+    const u64 list_cap = max_len + 1, slot_bytes = 2 * list_cap * sizeof(BiIv) + max_len * 8;
     SeedParams prm;
     prm.min_len = op.min_seed_len;
     prm.max_occ = op.max_occ;
@@ -1350,74 +1664,208 @@ int debwt_index_seeds(debwt_ctx* c, const char* reads, const uint64_t* offsets, 
     CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxThreadsPerMultiProcessor, c->device));
     const u64 n_slots = std::min<u64>({(u64)sms * (u64)per_sm, kSmemScratchBytes / slot_bytes, m});
     const u64 bytes = offsets[m], nb = (m + TPB - 1) / TPB, words = (bytes + 16 + 7) / 8;
-    // one block: reads | offsets (m + 1) | seed counts (m) | seed offsets (m + 1) | hit counts (m) | hit offsets (m + 1) |
-    // block totals (nb) | their scan (nb + 1) | counter
-    u64* d = nullptr;
-    BiIv* d_scratch = nullptr;
-    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&d), (words + 5 * m + 2 * nb + 5) * 8));
-    if (cudaMalloc(reinterpret_cast<void**>(&d_scratch), n_slots * slot_bytes) != cudaSuccess) {
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&r.d), (words + 5 * m + 2 * nb + 5) * 8));
+    if (cudaMalloc(reinterpret_cast<void**>(&r.scratch), n_slots * slot_bytes) != cudaSuccess) {
         cudaGetLastError();
-        cudaFree(d);
-        FAIL("index_seeds: out of device memory for " + std::to_string(n_slots * slot_bytes) + " bytes of scratch");
+        r.scratch = nullptr;
+        FAIL(nm + ": out of device memory for " + std::to_string(n_slots * slot_bytes) + " bytes of scratch");
     }
-    u64* d_mids = reinterpret_cast<u64*>(d_scratch + 2 * list_cap * n_slots);
-    u8* d_r = reinterpret_cast<u8*>(d);
-    u64 *d_o = d + words, *d_cnt = d_o + m + 1, *d_off = d_cnt + m, *d_hcnt = d_off + m + 1, *d_hoff = d_hcnt + m, *d_tot = d_hoff + m + 1,
-        *d_base = d_tot + nb;
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(d_base + nb + 1);
-    auto release = [&]() { cudaFree(d); cudaFree(d_scratch); };
+    u64* d_mids = reinterpret_cast<u64*>(r.scratch + 2 * list_cap * n_slots);
+    u8* d_r = reinterpret_cast<u8*>(r.d);
+    r.d_o = r.d + words;
+    u64 *d_cnt = r.d_o + m + 1, *d_hcnt;
+    r.d_off = d_cnt + m;
+    d_hcnt = r.d_off + m + 1;
+    r.d_hoff = d_hcnt + m;
+    r.d_tot = r.d_hoff + m + 1;
+    r.d_base = r.d_tot + nb;
+    r.d_next = reinterpret_cast<unsigned long long*>(r.d_base + nb + 1);
     CUDA_TRY(cudaMemcpyAsync(d_r, reads, bytes, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(d_o, offsets, (m + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
+    CUDA_TRY(cudaMemcpyAsync(r.d_o, offsets, (m + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(r.d_next, 0, 8, st));
     const FmView f = view_of(c);
     const unsigned grid = grid_for(n_slots);
-    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, prm, d_scratch, d_mids, n_slots, list_cap, d_next, d_cnt, d_hcnt, nullptr, nullptr,
-                                      nullptr, nullptr);
-    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_tot);
-    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
-    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, d_base, d_off);
-    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, d_tot);
-    scan_u64_kernel<<<1, TPB, 0, st>>>(d_tot, nb, d_base);
-    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, d_base, d_hoff);
+    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, r.d_o, m, prm, r.scratch, d_mids, n_slots, list_cap, r.d_next, d_cnt, d_hcnt, nullptr,
+                                      nullptr, nullptr, nullptr);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, r.d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_cnt, m, r.d_base, r.d_off);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, r.d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_hcnt, m, r.d_base, r.d_hoff);
     DEBWT_COUNT(7);
-    u64 total_hits = 0;
-    CUDA_TRY(cudaMemcpyAsync(seed_offsets, d_off, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(&total_hits, d_hoff + m, 8, cudaMemcpyDeviceToHost, st));
+    if (seed_offsets) CUDA_TRY(cudaMemcpyAsync(seed_offsets, r.d_off, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&r.total, r.d_off + m, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&r.total_hits, r.d_hoff + m, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
-    *n_hits_out = total_hits;
-    const u64 total = seed_offsets[m];
-    if (!seeds || total == 0) { release(); return 0; }                         // size query
-    if (total > seeds_cap || total_hits > hits_cap) {
-        release();
-        FAIL("index_seeds: the reads have " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits; seeds holds " +
-             std::to_string(seeds_cap) + " and hits " + std::to_string(hits_cap));
-    }
-    if (sorted_separators(c)) { release(); return -1; }
-    // the seeds | their first hits (total + 1) | the hits
-    char* d_out = nullptr;
+    const int go = proceed(r.total, r.total_hits);
+    if (go <= 0) return go;
+    if (sorted_separators(c, name)) return -1;
+    const u64 total = r.total, total_hits = r.total_hits;
     const u64 out_bytes = total * sizeof(debwt_seed) + (total + 1) * 8 + total_hits * sizeof(debwt_seed_hit);
-    if (cudaMalloc(reinterpret_cast<void**>(&d_out), out_bytes) != cudaSuccess) {
+    if (cudaMalloc(reinterpret_cast<void**>(&r.out), out_bytes) != cudaSuccess) {
         cudaGetLastError();
-        release();
-        FAIL("index_seeds: out of device memory for " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits");
+        r.out = nullptr;
+        FAIL(nm + ": out of device memory for " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits");
     }
-    debwt_seed* d_seeds = reinterpret_cast<debwt_seed*>(d_out);
-    u64* d_seed_hit = reinterpret_cast<u64*>(d_seeds + total);
-    debwt_seed_hit* d_hits = reinterpret_cast<debwt_seed_hit*>(d_seed_hit + total + 1);
-    CUDA_TRY(cudaMemcpyAsync(d_seed_hit + total, d_hoff + m, 8, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaMemsetAsync(d_next, 0, 8, st));
-    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, d_o, m, prm, d_scratch, d_mids, n_slots, list_cap, d_next, nullptr, nullptr, d_off, d_hoff,
-                                      d_seeds, d_seed_hit);
-    seed_hits_kernel<<<grid_for(total_hits), TPB, 0, st>>>(f, sa_view_of(c), d_seeds, d_seed_hit, total, total_hits, op.max_occ,
-                                                           c->d_seps_sorted, c->n_rec, d_hits);
+    r.seeds = reinterpret_cast<debwt_seed*>(r.out);
+    u64* d_seed_hit = reinterpret_cast<u64*>(r.seeds + total);
+    r.hits = reinterpret_cast<debwt_seed_hit*>(d_seed_hit + total + 1);
+    CUDA_TRY(cudaMemcpyAsync(d_seed_hit + total, r.d_hoff + m, 8, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(r.d_next, 0, 8, st));
+    seed_kernel<<<grid, TPB, 0, st>>>(f, d_r, r.d_o, m, prm, r.scratch, d_mids, n_slots, list_cap, r.d_next, nullptr, nullptr, r.d_off,
+                                      r.d_hoff, r.seeds, d_seed_hit);
+    seed_hits_kernel<<<grid_for(total_hits), TPB, 0, st>>>(f, sa_view_of(c), r.seeds, d_seed_hit, total, total_hits, op.max_occ,
+                                                           c->d_seps_sorted, c->n_rec, r.hits);
     DEBWT_COUNT(2);
-    CUDA_TRY(cudaMemcpyAsync(seeds, d_seeds, total * sizeof(debwt_seed), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(hits, d_hits, total_hits * sizeof(debwt_seed_hit), cudaMemcpyDeviceToHost, st));
+    return 1;
+}
+
+extern "C" {
+
+int debwt_index_seeds(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* opts,
+                      uint64_t* seed_offsets, uint64_t* n_hits_out, debwt_seed* seeds, uint64_t seeds_cap, debwt_seed_hit* hits,
+                      uint64_t hits_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !seed_offsets || !n_hits_out || !opts || (n_reads && !reads) || (seeds && !hits)) FAIL("null argument");
+    const debwt_seed_opts op = *opts;
+    const u64 m = n_reads;
+    u64 max_len = 0;
+    if (check_seed_input(c, "index_seeds", offsets, m, op, max_len)) return -1;
+    seed_offsets[0] = 0;
+    *n_hits_out = 0;
+    if (m == 0) return 0;
+    SeedRun r;
+    const int rc = run_seeds(c, "index_seeds", reads, offsets, m, op, max_len, seed_offsets, r, [&](u64 total, u64 total_hits) -> int {
+        *n_hits_out = total_hits;
+        if (!seeds || total == 0) return 0;                                     // size query
+        if (total > seeds_cap || total_hits > hits_cap)
+            FAIL("index_seeds: the reads have " + std::to_string(total) + " seeds and " + std::to_string(total_hits) + " hits; seeds holds " +
+                 std::to_string(seeds_cap) + " and hits " + std::to_string(hits_cap));
+        return 1;
+    });
+    if (rc <= 0) return rc;
+    cudaStream_t st = c->st;
+    CUDA_TRY(cudaMemcpyAsync(seeds, r.seeds, r.total * sizeof(debwt_seed), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(hits, r.hits, r.total_hits * sizeof(debwt_seed_hit), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
-    release();
-    cudaFree(d_out);
+    return 0;
+}
+
+static_assert(sizeof(debwt_chain) == 40, "debwt_chain is 2 u64 + 5 u32 + float");
+static_assert(sizeof(debwt_chain_seed) == 16, "debwt_chain_seed is u64 + 2 u32");
+
+int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* seed_opts,
+                       const debwt_chain_opts* chain_opts, uint64_t* chain_offsets, uint64_t* n_chain_seeds_out, debwt_chain* chains,
+                       uint64_t chains_cap, debwt_chain_seed* chain_seeds, uint64_t chain_seeds_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !chain_offsets || !n_chain_seeds_out || !seed_opts || !chain_opts || (n_reads && !reads) || (chains && !chain_seeds))
+        FAIL("null argument");
+    const debwt_seed_opts op = *seed_opts;
+    const debwt_chain_opts co = *chain_opts;
+    const std::pair<int32_t, const char*> ints[] = {{co.w, "w"}, {co.max_chain_gap, "max_chain_gap"}, {co.min_chain_weight, "min_chain_weight"},
+                                                     {co.max_chain_extend, "max_chain_extend"}};
+    for (const auto& [v, nm] : ints)
+        if (v < 0) FAIL(std::string("index_chains: ") + nm + " must not be negative, not " + std::to_string(v));
+    const std::pair<float, const char*> reals[] = {{co.mask_level, "mask_level"}, {co.drop_ratio, "drop_ratio"}};
+    for (const auto& [v, nm] : reals)
+        if (!std::isfinite(v) || v < 0) FAIL(std::string("index_chains: ") + nm + " must be finite and not negative, not " + std::to_string(v));
+    const u64 m = n_reads;
+    u64 max_len = 0;
+    if (check_seed_input(c, "index_chains", offsets, m, op, max_len)) return -1;
+    if (m == 0) {
+        chain_offsets[0] = 0;
+        *n_chain_seeds_out = 0;
+        return 0;
+    }
+    SeedRun r;
+    const int rc = run_seeds(c, "index_chains", reads, offsets, m, op, max_len, nullptr, r, [](u64, u64 total_hits) { return total_hits ? 1 : 0; });
+    if (rc < 0) return -1;
+    if (rc == 0) {                                                                // no hits: no chains
+        std::fill(chain_offsets, chain_offsets + m + 1, 0ull);
+        *n_chain_seeds_out = 0;
+        return 0;
+    }
+    cudaStream_t st = c->st;
+    const u64 H = r.total_hits, nb = (m + TPB - 1) / TPB;
+    ChainParams prm;
+    prm.w = co.w;
+    prm.max_chain_gap = co.max_chain_gap;
+    prm.max_chain_extend = co.max_chain_extend;
+    prm.min_seed_len = op.min_seed_len;
+    prm.min_chain_weight = (u32)co.min_chain_weight;
+    prm.max_occ = op.max_occ;
+    prm.mask_level = co.mask_level;
+    prm.drop_ratio = co.drop_ratio;
+    prm.l_pac = (c->n - c->n_rec) / 2;
+    // per hit: chain seed, sort key, ChainRec, slot hit, next, tail, kept list (68 bytes); per read: kept chains and their
+    // seeds, the offsets of both, chains after the weight pass, frac_rep; the slot bitmap and its summary
+    const u64 n_bits = H / 64 + m + 1, n_summary = H / 4096 + m + 1;
+    ChainScratch s;
+    u64 *d_ccnt, *d_scnt, *d_coff, *d_soff;
+    u32* d_nsorted;
+    float* d_frac;
+    char* p = nullptr;
+    auto take = [&](auto*& dst, u64 n) {
+        dst = reinterpret_cast<std::remove_reference_t<decltype(dst)>>(p);
+        p += (n * sizeof(*dst) + 15) / 16 * 16;
+    };
+    auto lay_out = [&]() {
+        take(s.cs, H); take(s.key, H); take(s.rec, H); take(s.idx, H); take(s.nxt, H); take(s.tail, H); take(s.list, H);
+        take(s.bits, n_bits); take(s.summary, n_summary);
+        take(d_ccnt, m); take(d_scnt, m); take(d_coff, m + 1); take(d_soff, m + 1); take(d_nsorted, m); take(d_frac, m);
+    };
+    lay_out();
+    const u64 scratch_bytes = (u64)reinterpret_cast<uintptr_t>(p);
+    char* d_c = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_c), scratch_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL("index_chains: out of device memory for " + std::to_string(scratch_bytes) + " bytes of chaining scratch (" + std::to_string(H) + " hits)");
+    }
+    struct Free { char* p; ~Free() { cudaFree(p); } } free_c{d_c};
+    p = d_c;
+    lay_out();
+    int sms = 0, per_sm = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxThreadsPerMultiProcessor, c->device));
+    const u64 n_threads = std::min<u64>((u64)sms * (u64)per_sm, m);
+    CUDA_TRY(cudaMemsetAsync(r.d_next, 0, 8, st));
+    chain_kernel<<<grid_for(n_threads), TPB, 0, st>>>(r.d_o, m, r.seeds, r.d_off, r.hits, r.d_hoff, c->d_seps_sorted, prm, s, r.d_next,
+                                                      d_ccnt, d_scnt, d_nsorted, d_frac);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_ccnt, m, r.d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_ccnt, m, r.d_base, d_coff);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_scnt, m, r.d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_scnt, m, r.d_base, d_soff);
+    DEBWT_COUNT(7);
+    u64 total_seeds = 0;
+    CUDA_TRY(cudaMemcpyAsync(chain_offsets, d_coff, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&total_seeds, d_soff + m, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    *n_chain_seeds_out = total_seeds;
+    const u64 total = chain_offsets[m];
+    if (!chains || total == 0) return 0;                                          // size query
+    if (total > chains_cap || total_seeds > chain_seeds_cap)
+        FAIL("index_chains: the reads have " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds; chains holds " +
+             std::to_string(chains_cap) + " and chain_seeds " + std::to_string(chain_seeds_cap));
+    char* d_out = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_out), total * sizeof(debwt_chain) + total_seeds * sizeof(debwt_chain_seed)) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL("index_chains: out of device memory for " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds");
+    }
+    Free free_out{d_out};
+    debwt_chain* d_chains = reinterpret_cast<debwt_chain*>(d_out);
+    debwt_chain_seed* d_cseeds = reinterpret_cast<debwt_chain_seed*>(d_chains + total);
+    chain_write_kernel<<<grid_for(m), TPB, 0, st>>>(m, r.hits, r.d_hoff, s, d_nsorted, d_frac, d_coff, d_soff, d_chains, d_cseeds);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(chains, d_chains, total * sizeof(debwt_chain), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(chain_seeds, d_cseeds, total_seeds * sizeof(debwt_chain_seed), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
     return 0;
 }
 

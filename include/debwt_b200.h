@@ -265,6 +265,66 @@ typedef struct debwt_seed_hit {
 int debwt_index_seeds(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* opts,
                       uint64_t* seed_offsets /* n_reads + 1 */, uint64_t* n_hits_out, debwt_seed* seeds, uint64_t seeds_cap,
                       debwt_seed_hit* hits, uint64_t hits_cap);
+/* BWA-MEM's seed chaining (bwa 0.7.17's mem_chain and mem_chain_flt) from reads to filtered chains, with the seeding of
+   debwt_index_seeds inside (seed_opts as there).  Options are bwa's w, max_chain_gap, -W, max_chain_extend, mask_level
+   and -D (defaults 100, 10000, 0, 1 << 30, 0.50, 0.50).
+   bwa's coordinate: with l_pac = (N - R) / 2 (the forward bases) and F[r] = the bases of the forward records before r, a
+   hit of length len at (record r, strand, forward offset o) has rbeg = F[r] + o on strand 0 (its text position - r) and
+   rbeg = 2 l_pac - (F[r] + o + len) on strand 1 (python: api.bwa_rbeg).
+   Per read, its hits are visited in the order of debwt_index_seeds (seed by seed, hit j ascending); each is a seed
+   s = (rbeg, qbeg, len = qend - qbeg) with rid = its record.
+     frac_rep: the union length of [qbeg, qend) over the read's seeds with count > max_occ, swept in seed order as bwa
+       does, over the read length (float).  A read of length 0 has no chains.
+     chain set: chains are ordered by pos.  For each hit, lower = the chain with the greatest pos <= s.rbeg; among chains
+       with that pos the one created first (bwa's kbtree orders equal keys by its node layout).  If there is no lower or
+       test_and_merge(lower, s) is 0, a new chain {pos = s.rbeg, seeds = [s], rid} is created.
+     test_and_merge(c, p), first / last = c's first / last seed: 0 if p.rid != c.rid; 1 without adding p if p.qbeg >=
+       first.qbeg, p.qbeg + p.len <= last.qbeg + last.len, p.rbeg >= first.rbeg and p.rbeg + p.len <= last.rbeg +
+       last.len (contained); 0 if (last.rbeg < l_pac or first.rbeg < l_pac) and p.rbeg >= l_pac; with x = p.qbeg -
+       last.qbeg, y = p.rbeg - last.rbeg (64-bit): p is appended and 1 returned if y >= 0, x - y <= w, y - x <= w,
+       x - last.len < max_chain_gap and y - last.len < max_chain_gap; 0 otherwise.
+     weight: a sweep over the chain's seeds in order with end = 0: a seed adds len if qbeg >= end, else max(0, qbeg + len
+       - end), then end = max(end, qbeg + len); the same over rbeg; the weight is the smaller sweep.
+     filter: chains with weight < min_chain_weight are dropped; the rest sorted by weight descending, ties in chain-set
+       order (pos, then creation; bwa's sort is unstable).  a[0].kept = 3, kept list [0], first = -1 everywhere.  For
+       each i >= 1 and each j of the kept list in order, over query spans (beg = first seed's qbeg, end = last seed's
+       qbeg + len): b = max(beg_i, beg_j), e = min(end_i, end_j); if e > b, min_l = min(end_i - beg_i, end_j - beg_j),
+       and e - b >= min_l * mask_level (float) and min_l < max_chain_gap: large_ovlp = 1, first_j = i if first_j < 0,
+       and if also w_i < w_j * drop_ratio (float) and w_j - w_i >= 2 min_seed_len, i is dropped (the loop stops).  An i
+       no j drops joins the kept list with kept = large_ovlp ? 2 : 3.  Then a[first_j].kept = 1 for every j of the kept
+       list with first_j >= 0 (over a 2, or reviving a dropped chain).  Counting the kept-1/2 chains in order, at the
+       chain where the count reaches max_chain_extend and after it every chain with kept < 3 becomes 0.  Chains with
+       kept 0 are removed.
+   A read's chains are chains[chain_offsets[i] .. chain_offsets[i + 1]) in that filter order; a chain's seeds are
+   chain_seeds[seed_begin .. seed_begin + n_seeds) in insertion order; record and strand are its first seed's (every
+   seed of a chain has them).  chain_offsets[n_reads + 1] and *n_chain_seeds_out are always written; chains == NULL is
+   a size query.  More chains than chains_cap or more chain seeds than chain_seeds_cap fails, writes nothing into chains
+   / chain_seeds, and names both totals.  Needs debwt_index_sample_sa.  Fails, writing nothing, on every input that
+   debwt_index_seeds refuses (the messages name index_chains), on a negative w, max_chain_gap, min_chain_weight or
+   max_chain_extend, on a negative or non-finite mask_level or drop_ratio (the message names the option), and on NULL
+   arguments (chain_seeds may be NULL only with chains).  Besides the seeding scratch the call holds 68 bytes of device
+   memory per hit.  n_reads = 0 only writes chain_offsets[0] = 0 and *n_chain_seeds_out = 0.  Not done here: bwa's
+   mem_flt_chained_seeds (it needs the extension's scores) and ALT contigs (is_alt is 0). */
+typedef struct debwt_chain_opts {
+    int32_t w, max_chain_gap, min_chain_weight, max_chain_extend;  /* bwa: 100, 10000, 0 (-W), 1 << 30 */
+    float mask_level, drop_ratio;                                   /* bwa: 0.50, 0.50 (-D) */
+} debwt_chain_opts;
+typedef struct debwt_chain {
+    uint64_t pos;           /* rbeg of its first seed (bwa's coordinate) */
+    uint64_t seed_begin;    /* its seeds are chain_seeds[seed_begin, seed_begin + n_seeds) */
+    uint32_t n_seeds, weight;
+    uint32_t record, strand;
+    uint32_t kept;          /* 1, 2 or 3 as bwa sets it */
+    float frac_rep;         /* the read's, as bwa copies it into every chain */
+} debwt_chain;              /* 40 bytes */
+typedef struct debwt_chain_seed {
+    uint64_t rbeg;          /* bwa's coordinate */
+    uint32_t qbeg, len;
+} debwt_chain_seed;         /* 16 bytes */
+int debwt_index_chains(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads,
+                       const debwt_seed_opts* seed_opts, const debwt_chain_opts* chain_opts,
+                       uint64_t* chain_offsets /* n_reads + 1 */, uint64_t* n_chain_seeds_out,
+                       debwt_chain* chains, uint64_t chains_cap, debwt_chain_seed* chain_seeds, uint64_t chain_seeds_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
