@@ -299,6 +299,42 @@ class BwtBuilder:
             check(lib().debwt_index_chains(*args, _ptr(chains), chains.size, _ptr(seeds), seeds.size))
         return co_offs, chains, seeds
 
+    def regions(self, reads: Sequence, min_len: int = 19, split_factor: float = 1.5, split_width: int = 10, max_mem_intv: int = 20,
+                max_occ: int = 500, w: int = 100, max_chain_gap: int = 10000, min_chain_weight: int = 0, mask_level: float = 0.5,
+                drop_ratio: float = 0.5, max_chain_extend: int = 1 << 30, a: int = 1, b: int = 4, o_del: int = 6, e_del: int = 1,
+                o_ins: int = 6, e_ins: int = 1, pen_clip5: int = 5, pen_clip3: int = 5, zdrop: int = 100) -> tuple[np.ndarray, np.ndarray]:
+        """(offsets u64[m + 1], regions REGION_DTYPE[total]): BWA-MEM's alignment regions of read i (bwa's
+        mem_flt_chained_seeds and mem_chain2aln over the chains of `chains` with the same seed and chain options; w is
+        also the band; bwa's -A, -B, -O, -E, -L and -d) are regions[offsets[i]:offsets[i+1]], chain by chain in the
+        order of extension, in bwa's coordinate.  One device pass per call: the regions land in a buffer the builder
+        keeps, and only a batch with more regions than it holds runs a second time.  Needs sample_sa."""
+        rs = [r.encode() if isinstance(r, str) else bytes(r) for r in reads]
+        offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        offs[1:] = np.cumsum([len(r) for r in rs])
+        blob = np.frombuffer(b"".join(rs) + b"\0", dtype=np.uint8)
+        for name, v in (("min_len", min_len), ("split_width", split_width), ("max_mem_intv", max_mem_intv), ("max_occ", max_occ)):
+            if not 0 <= v < 1 << 32:
+                raise DebwtError(f"regions: {name} = {v} is not a 32-bit unsigned integer")
+        ints = dict(w=w, max_chain_gap=max_chain_gap, min_chain_weight=min_chain_weight, max_chain_extend=max_chain_extend, a=a, b=b,
+                    o_del=o_del, e_del=e_del, o_ins=o_ins, e_ins=e_ins, pen_clip5=pen_clip5, pen_clip3=pen_clip3, zdrop=zdrop)
+        for name, v in ints.items():
+            if not -(1 << 31) <= v < 1 << 31:
+                raise DebwtError(f"regions: {name} = {v} is not a 32-bit signed integer")
+        so = SeedOpts(min_len, split_width, max_mem_intv, max_occ, split_factor)
+        co = ChainOpts(w, max_chain_gap, min_chain_weight, max_chain_extend, mask_level, drop_ratio)
+        eo = ExtOpts(a, b, o_del, e_del, o_ins, e_ins, pen_clip5, pen_clip3, zdrop)
+        r_offs = np.zeros(len(rs) + 1, dtype=np.uint64)
+        args = (self._h, _ptr(blob), _ptr(offs), len(rs), ctypes.addressof(so), ctypes.addressof(co), ctypes.addressof(eo), _ptr(r_offs))
+        buf = getattr(self, "_regions_buf", None)
+        if buf is None:
+            buf = self._regions_buf = np.zeros(1 << 16, dtype=REGION_DTYPE)
+        rc = lib().debwt_index_regions(*args, _ptr(buf), buf.size)
+        if rc != 0 and int(r_offs[-1]) > buf.size:                    # too small: grow once, run again
+            buf = self._regions_buf = np.zeros(int(r_offs[-1]) * 5 // 4, dtype=REGION_DTYPE)
+            rc = lib().debwt_index_regions(*args, _ptr(buf), buf.size)
+        check(rc)
+        return r_offs, buf[:int(r_offs[-1])].copy()
+
     def verify(self, text=None, device_ptr: int | None = None, n_symbols: int | None = None):
         """LF-inversion check of the last build against T; returns (bad rows, device ms).  0 bad rows <=> BWT(T)."""
         bad, ms = c_u64(), ctypes.c_float()
@@ -382,6 +418,18 @@ class ChainOpts(ctypes.Structure):
     """debwt_chain_opts of include/debwt_b200.h"""
     _fields_ = [("w", ctypes.c_int32), ("max_chain_gap", ctypes.c_int32), ("min_chain_weight", ctypes.c_int32),
                 ("max_chain_extend", ctypes.c_int32), ("mask_level", ctypes.c_float), ("drop_ratio", ctypes.c_float)]
+
+
+# ---- BWA-MEM seed extension over both strands (debwt_index_regions) --------------------------------------------------
+REGION_DTYPE = np.dtype([("rb", np.uint64), ("re", np.uint64), ("qb", np.uint32), ("qe", np.uint32), ("score", np.int32),
+                         ("truesc", np.int32), ("w", np.uint32), ("seedcov", np.uint32), ("seedlen0", np.uint32), ("chain", np.uint32),
+                         ("record", np.uint32), ("strand", np.uint32), ("frac_rep", np.float32), ("pad_", np.uint32)],
+                        align=True)                    # debwt_region
+
+
+class ExtOpts(ctypes.Structure):
+    """debwt_ext_opts of include/debwt_b200.h"""
+    _fields_ = [(n, ctypes.c_int32) for n in ("a", "b", "o_del", "e_del", "o_ins", "e_ins", "pen_clip5", "pen_clip3", "zdrop")]
 
 
 _COMP = bytes.maketrans(b"ACGT", b"TGCA")

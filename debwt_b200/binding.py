@@ -85,6 +85,7 @@ _SIGS = {
     "debwt_index_smem": (ctypes.c_int, [c_p, c_p, c_p, c_u64, ctypes.c_uint32, c_p, c_p, c_u64]),
     "debwt_index_seeds": (ctypes.c_int, [c_p, c_p, c_p, c_u64, c_p, c_p, c_p, c_p, c_u64, c_p, c_u64]),
     "debwt_index_chains": (ctypes.c_int, [c_p, c_p, c_p, c_u64, c_p, c_p, c_p, c_p, c_p, c_u64, c_p, c_u64]),
+    "debwt_index_regions": (ctypes.c_int, [c_p, c_p, c_p, c_u64, c_p, c_p, c_p, c_p, c_p, c_u64]),
     "debwt_verify_text": (ctypes.c_int, [c_p, c_p, c_u64, ctypes.POINTER(c_u64), ctypes.POINTER(ctypes.c_float)]),
     "debwt_verify_text_device": (ctypes.c_int, [c_p, c_p, c_u64, ctypes.POINTER(c_u64), ctypes.POINTER(ctypes.c_float)]),
     "debwt_verify_bwt_device": (ctypes.c_int, [ctypes.c_int, c_p, c_u64, c_p, c_u64, c_u64, c_p, ctypes.POINTER(c_u64),

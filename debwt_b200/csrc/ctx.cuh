@@ -143,6 +143,7 @@ struct debwt_ctx {
     u64 n_sa_samples = 0;
     u32* d_isa_vals = nullptr;        // [n_sa_samples]: [k] = row of suffix k * rate (the first debwt_index_extract after sampling)
     u64* d_seps_sorted = nullptr;     // [n_rec]: the separator positions, ascending (the first debwt_index_seeds after sampling)
+    u32* d_pac = nullptr;             // bwa's pac, 16 forward bases per word, base x at bits 2 (x & 15) (the first debwt_index_regions after sampling)
     bool loaded = false;              // the result came from debwt_set_result, not from a build
 };
 

@@ -1013,6 +1013,449 @@ __global__ void __launch_bounds__(TPB) chain_write_kernel(u64 n_reads, const deb
     }
 }
 
+// ---- BWA-MEM seed extension (mem_flt_chained_seeds, mem_chain2aln) ------------------------------------------------
+// bwa's pac from the index: one thread per rate-aligned block of the forward half T[0, fwd_end) (records 0 .. R/2 - 1),
+// walking LF from a sampled row as extract_kernel does.  Base T[p] goes to pac index p - (separators before p); `below`
+// counts the separators at or before the current p.  Blocks share boundary words, so words are merged with atomicOr.
+__global__ void __launch_bounds__(TPB) pac_kernel(FmView f, SaView s, const u32* __restrict__ isa, const u64* __restrict__ seps, u64 R,
+                                                 u64 fwd_end, u64 n_blocks, u32* __restrict__ pac) {
+    const u64 q = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (q >= n_blocks) return;
+    const u32 sh = __ffs(s.rate) - 1;
+    const u64 lo = q << sh, hi = min(fwd_end, (q + 1) << sh), top = min((q + 1) << sh, f.n);
+    u64 r = top == f.n ? f.dollar_row : isa[top >> sh];
+    u64 below = upper_bound_u64(seps, 0, R, top - 1);
+    u64 word = ~0ull;
+    u32 acc = 0;
+    for (u64 p = top - 1;; --p) {                                                 // r is the row of suffix p + 1
+        const u32 c = row_symbol(f, r);
+        if (c >= 4) {
+            --below;
+        } else if (p < hi) {
+            const u64 x = p - below;
+            if (x >> 4 != word) {
+                if (acc) atomicOr(pac + word, acc);
+                word = x >> 4;
+                acc = 0;
+            }
+            acc |= c << (2 * (x & 15));
+        }
+        if (p == lo) break;
+        r = lf_with(f, r, c);
+    }
+    if (acc) atomicOr(pac + word, acc);
+}
+
+struct ExtParams {
+    int a, b, o_del, e_del, o_ins, e_ins, pen_clip5, pen_clip3, zdrop, w, min_chain_weight;
+    u32 ring;               // int2 entries per warp: the DP window of the widest band, and seed SW's 199 columns
+    u64 l_pac;
+};
+
+// Per chain seed (indexed as chain_seeds): the seeds a chain keeps after mem_flt_chained_seeds with their scores, bwa's
+// srt, and the read's region slots (a read has at most as many regions as chain seeds); per chain: its kept seeds.
+struct ExtScratch {
+    debwt_chain_seed* fs;
+    int* sc;
+    u64* srt;
+    debwt_region* reg;
+    u32* fn;
+};
+
+struct ExtOut {
+    int score, qle, tle, gtle, gscore, max_off;
+};
+
+constexpr int EXT_WARPS = 4;
+constexpr int kMaxExtW = 1024;          // widest w: a retry's band w << 1 needs 2 (w << 1) + 3 ring entries per warp
+constexpr unsigned FULL = 0xFFFFFFFFu;
+constexpr long long NEG = -(1ll << 62);
+
+__device__ __forceinline__ u32 nt4(u8 c) {
+    const u32 l = c | 0x20u;
+    return l == 'a' ? 0u : l == 'c' ? 1u : l == 'g' ? 2u : l == 't' ? 3u : 4u;
+}
+
+__device__ __forceinline__ u32 ref_base(const u32* __restrict__ pac, u64 l_pac, u64 x) {
+    const u64 y = x < l_pac ? x : 2 * l_pac - 1 - x;
+    const u32 v = (pac[y >> 4] >> (2 * (y & 15))) & 3u;
+    return x < l_pac ? v : 3u - v;
+}
+
+__device__ __forceinline__ int cal_max_gap(const ExtParams& o, int qlen) {
+    const int l_del = (int)((double)(qlen * o.a - o.o_del) / o.e_del + 1.);
+    const int l_ins = (int)((double)(qlen * o.a - o.o_ins) / o.e_ins + 1.);
+    const int l = max(max(l_del, l_ins), 1);
+    return min(l, o.w << 1);
+}
+
+__device__ __forceinline__ long long warp_incl_max(long long v, u32 lane) {
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const long long u = __shfl_up_sync(FULL, v, d);
+        if ((int)lane >= d) v = max(v, u);
+    }
+    return v;
+}
+
+// ksw_extend2 for one warp: rows i over the target, lanes over 32 columns j of the query at a time.  In a row, M and E
+// of a column need only that column, and F is a max-plus prefix scan: F(j) = max over beg <= k < j of
+// max(M_k - oe_ins, 0) - (j - 1 - k) e_ins.  Every column row i touches lies in [i - w, i + w + 1] and beg never
+// decreases, so `ring` (2 w + 3 entries or more) holds bwa's eh array; a column above `top` was never written and still
+// has its row-0 value.
+template <class Q, class T>
+__device__ ExtOut warp_extend(const ExtParams& o, int qlen, Q qsym, int tlen, T tsym, int w, int end_bonus, int h0, int2* ring, u32 lane) {
+    const int oe_del = o.o_del + o.e_del, oe_ins = o.o_ins + o.e_ins, RS = (int)o.ring;
+    const int max_ins = max((int)((double)(qlen * o.a + end_bonus - o.o_ins) / o.e_ins + 1.), 1);
+    const int max_del = max((int)((double)(qlen * o.a + end_bonus - o.o_del) / o.e_del + 1.), 1);
+    w = min(w, min(max_ins, max_del));
+    auto row0 = [&](int j) -> int {
+        if (j == 0) return h0;
+        if (h0 <= oe_ins) return 0;
+        const long long v = (long long)h0 - oe_ins - (long long)(j - 1) * o.e_ins;
+        return v > 0 ? (int)v : 0;
+    };
+    int beg = 0, end = qlen, mx = h0, max_i = -1, max_j = -1, max_ie = -1, gscore = -1, max_off = 0, top = -1;
+    for (int i = 0; i < tlen; ++i) {
+        beg = max(beg, i - w);
+        end = min(min(end, i + w + 1), qlen);
+        int h1 = 0;
+        if (beg == 0) {
+            const long long v = (long long)h0 - (o.o_del + (long long)o.e_del * (i + 1));
+            h1 = v > 0 ? (int)v : 0;
+        }
+        const u32 tb = tsym(i);
+        long long P = NEG;                                                        // max of M'_k + k e_ins over earlier chunks
+        int hc = h1;                                                              // H(i, c - 1)
+        unsigned long long best = 0;                                              // (m, mj) with the last j reaching m
+        bool any = false;
+        int first_nz = -1, last_nz = -1;
+        for (int c = beg; c < end; c += 32) {
+            const int j = c + (int)lane;
+            const bool act = j < end;
+            int ho = 0, eo = 0;
+            u32 qs = 4;
+            if (act) {
+                if (j > top) ho = row0(j);
+                else { const int2 v = ring[j % RS]; ho = v.x; eo = v.y; }
+                qs = qsym(j);
+            }
+            const int M = ho ? ho + (qs > 3 ? -1 : qs == tb ? o.a : -o.b) : 0;
+            const long long v = warp_incl_max(act ? (long long)max(M - oe_ins, 0) + (long long)j * o.e_ins : NEG, lane);
+            long long ex = __shfl_up_sync(FULL, v, 1);
+            ex = max(lane ? ex : NEG, P);
+            const int f = j == beg ? 0 : (int)(ex - (long long)(j - 1) * o.e_ins);
+            const int h = max(max(M, eo), f);
+            int hp = __shfl_up_sync(FULL, h, 1);
+            if (lane == 0) hp = hc;
+            const int en = max(eo - o.e_del, max(M - oe_del, 0));
+            const u32 nz = __ballot_sync(FULL, act && (hp || en));
+            if (nz) {
+                if (first_nz < 0) first_nz = c + __ffs(nz) - 1;
+                last_nz = c + 31 - __clz(nz);
+            }
+            unsigned long long key = act ? ((unsigned long long)(u32)h << 32 | (u32)j) : 0ull;
+#pragma unroll
+            for (int d = 16; d; d >>= 1) key = max(key, __shfl_xor_sync(FULL, key, d));
+            best = max(best, key);
+            any = true;
+            if (act) ring[j % RS] = make_int2(hp, en);
+            const int last = min(end - c, 32) - 1;
+            hc = __shfl_sync(FULL, h, last);
+            P = max(P, __shfl_sync(FULL, v, last));
+            __syncwarp();
+        }
+        if (lane == 0) ring[end % RS] = make_int2(hc, 0);
+        __syncwarp();
+        top = max(top, end);
+        if (max(beg, end) == qlen) {
+            max_ie = gscore > hc ? max_ie : i;
+            gscore = max(gscore, hc);
+        }
+        const int m = any ? (int)(best >> 32) : 0, mj = any ? (int)(u32)best : -1;
+        if (m == 0) break;
+        if (m > mx) {
+            mx = m; max_i = i; max_j = mj;
+            max_off = max(max_off, abs(mj - i));
+        } else if (o.zdrop > 0) {
+            const long long di = i - max_i, dj = mj - max_j;
+            if (di > dj) {
+                if (mx - m - (di - dj) * o.e_del > o.zdrop) break;
+            } else if (mx - m - (dj - di) * o.e_ins > o.zdrop) break;
+        }
+        const int nb = first_nz >= 0 ? first_nz : end;
+        const int lj = hc ? end : last_nz >= 0 ? last_nz : nb - 1;
+        beg = nb;
+        end = min(lj + 2, qlen);
+    }
+    return ExtOut{mx, max_j + 1, max_i + 1, max_ie + 1, gscore, max_off};
+}
+
+// ksw_align2's score for one warp: Gotoh local alignment, rows over the target, lanes over the query.  buf[j] holds
+// (H(i - 1, j), E(i, j)).  Opening a gap from an H that came from F is never better than extending F, so F is again a
+// prefix scan, over G = max(M, E, 0): F(j) = max(0, max over k < j of G_k - oe_ins - (j - 1 - k) e_ins).
+template <class Q, class T>
+__device__ int warp_seed_sw(const ExtParams& o, int qlen, Q qsym, int tlen, T tsym, int2* buf, u32 lane) {
+    const int oe_del = o.o_del + o.e_del, oe_ins = o.o_ins + o.e_ins;
+    for (int j = (int)lane; j < qlen; j += 32) buf[j] = make_int2(0, 0);
+    __syncwarp();
+    int best = 0;
+    for (int i = 0; i < tlen; ++i) {
+        const u32 tb = tsym(i);
+        int hd = 0;
+        long long P = NEG;
+        for (int c = 0; c < qlen; c += 32) {
+            const int j = c + (int)lane;
+            const bool act = j < qlen;
+            const int2 v = act ? buf[j] : make_int2(0, 0);
+            const u32 qs = act ? qsym(j) : 4;
+            int hdiag = __shfl_up_sync(FULL, v.x, 1);
+            if (lane == 0) hdiag = hd;
+            const int G = max(max(hdiag + (qs > 3 ? -1 : qs == tb ? o.a : -o.b), v.y), 0);
+            const long long u = warp_incl_max(act ? (long long)G - oe_ins + (long long)j * o.e_ins : NEG, lane);
+            long long ex = __shfl_up_sync(FULL, u, 1);
+            ex = max(lane ? ex : NEG, P);
+            const int H = max(G, (int)max(0ll, ex - (long long)(j - 1) * o.e_ins));
+            if (act) {
+                best = max(best, H);
+                buf[j] = make_int2(H, max(max(v.y - o.e_del, H - oe_del), 0));
+            }
+            const int last = min(qlen - c, 32) - 1;
+            hd = __shfl_sync(FULL, v.x, last);
+            P = max(P, __shfl_sync(FULL, u, last));
+            __syncwarp();
+        }
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) best = max(best, __shfl_xor_sync(FULL, best, d));
+    return best;
+}
+
+// bns_fetch_seq's clip of [beg, end) to the record `rec` on the strand of mid; F(r) = seps[r - 1] + 1 - r
+__device__ __forceinline__ void clip_to_record(const u64* __restrict__ seps, u64 l_pac, u32 rec, long long mid, long long& beg, long long& end) {
+    const long long start = rec ? (long long)seps[rec - 1] + 1 : 0;
+    long long fb = start - rec, fe = fb + ((long long)seps[rec] - start);
+    if (mid >= (long long)l_pac) {
+        const long long t = fb;
+        fb = 2 * (long long)l_pac - fe;
+        fe = 2 * (long long)l_pac - t;
+    }
+    beg = max(beg, fb);
+    end = min(end, fe);
+}
+
+__device__ __forceinline__ int warp_sum(int v) {
+#pragma unroll
+    for (int d = 16; d; d >>= 1) v += __shfl_xor_sync(FULL, v, d);
+    return v;
+}
+
+// One warp per read in flight, reads from the work counter `next`: mem_flt_chained_seeds over the read's kept chains,
+// then mem_chain2aln chain by chain.  Every lane runs the read's control flow (it depends only on values all lanes
+// read alike); lanes split the DP rows, the containment and overlap tests and seedcov; lane 0 writes.  The regions go
+// to the read's slots from its first chain seed on; reg_cnt[rd] receives their number.
+__global__ void __launch_bounds__(EXT_WARPS * 32) ext_kernel(const u8* __restrict__ reads, const u64* __restrict__ offs, u64 n_reads,
+                                                            const debwt_chain* __restrict__ chains, const u64* __restrict__ chain_off,
+                                                            const debwt_chain_seed* __restrict__ cseeds, const u64* __restrict__ cseed_off,
+                                                            const u32* __restrict__ pac, const u64* __restrict__ seps, ExtParams o,
+                                                            ExtScratch s, unsigned long long* __restrict__ next, u64* __restrict__ reg_cnt) {
+    extern __shared__ int2 ext_smem[];
+    const u32 lane = threadIdx.x & 31;
+    int2* ring = ext_smem + (threadIdx.x >> 5) * o.ring;
+    const long long l_pac = (long long)o.l_pac;
+    for (;;) {
+        unsigned long long rd = 0;
+        if (lane == 0) rd = atomicAdd(next, 1ull);
+        rd = __shfl_sync(FULL, rd, 0);
+        if (rd >= n_reads) break;
+        const u8* q = reads + offs[rd];
+        const int L = (int)(offs[rd + 1] - offs[rd]);
+        const u64 c0 = chain_off[rd], c1 = chain_off[rd + 1], sb = cseed_off[rd];
+        // mem_flt_chained_seeds
+        const double min_l = o.min_chain_weight ? (double)(1.1f * (float)o.min_chain_weight) : (double)5.5f * log((double)L);
+        const int min_hsp = (int)(o.a * min_l + .499);
+        const bool flt = !(min_l > (double)(0.05f * (float)L));
+        for (u64 ci = c0; ci < c1; ++ci) {
+            const debwt_chain ch = chains[ci];
+            const debwt_chain_seed* sd = cseeds + ch.seed_begin;
+            u32 k = 0;
+            for (u32 j = 0; j < ch.n_seeds; ++j) {
+                const debwt_chain_seed t = sd[j];
+                int sc = (int)t.len;
+                if (flt) {
+                    sc = -1;
+                    if (t.len < 200) {
+                        const long long rbeg = (long long)t.rbeg;
+                        const long long qb = max((long long)t.qbeg - 50, 0ll), qe = min((long long)t.qbeg + t.len + 50, (long long)L);
+                        long long rb = max(rbeg - 50, 0ll), re = min(rbeg + t.len + 50, 2 * l_pac);
+                        const long long mid = (rbeg + rbeg + t.len) >> 1;
+                        if (rb < l_pac && l_pac < re) {
+                            if (mid < l_pac) re = l_pac;
+                            else rb = l_pac;
+                        }
+                        if (qe - qb < 200 && re - rb < 200) {
+                            clip_to_record(seps, o.l_pac, ch.record, mid, rb, re);
+                            sc = warp_seed_sw(o, (int)(qe - qb), [&](int x) { return nt4(q[qb + x]); }, (int)(re - rb),
+                                              [&](int y) { return ref_base(pac, o.l_pac, (u64)(rb + y)); }, ring, lane);
+                        }
+                    }
+                    if (sc >= 0 && sc < min_hsp) continue;
+                    if (sc < 0) sc = (int)t.len * o.a;
+                }
+                if (lane == 0) {
+                    s.fs[ch.seed_begin + k] = t;
+                    s.sc[ch.seed_begin + k] = sc;
+                }
+                ++k;
+            }
+            if (lane == 0) s.fn[ci] = k;
+        }
+        __syncwarp();
+        // mem_chain2aln
+        u32 n_reg = 0;
+        debwt_region* reg = s.reg + sb;
+        for (u64 ci = c0; ci < c1; ++ci) {
+            const debwt_chain ch = chains[ci];
+            const u32 n = s.fn[ci];
+            if (n == 0) continue;
+            const debwt_chain_seed* S = s.fs + ch.seed_begin;
+            u64* srt = s.srt + ch.seed_begin;
+            long long rmax0 = 2 * l_pac, rmax1 = 0;
+            for (u32 i = 0; i < n; ++i) {
+                const debwt_chain_seed t = S[i];
+                const int r = L - (int)(t.qbeg + t.len);
+                rmax0 = min(rmax0, (long long)t.rbeg - (t.qbeg + cal_max_gap(o, (int)t.qbeg)));
+                rmax1 = max(rmax1, (long long)t.rbeg + t.len + (r + cal_max_gap(o, r)));
+            }
+            rmax0 = max(rmax0, 0ll);
+            rmax1 = min(rmax1, 2 * l_pac);
+            if (rmax0 < l_pac && l_pac < rmax1) {
+                if ((long long)S[0].rbeg < l_pac) rmax1 = l_pac;
+                else rmax0 = l_pac;
+            }
+            clip_to_record(seps, o.l_pac, ch.record, (long long)S[0].rbeg, rmax0, rmax1);
+            if (lane == 0) {
+                for (u32 i = 0; i < n; ++i) srt[i] = (u64)(u32)s.sc[ch.seed_begin + i] << 32 | i;
+                sort_keys(srt, n);
+            }
+            __syncwarp();
+            for (int k = (int)n - 1; k >= 0; --k) {
+                const debwt_chain_seed sd = S[(u32)srt[k]];
+                const long long srb = (long long)sd.rbeg;
+                const int sq = (int)sd.qbeg, sl = (int)sd.len;
+                bool covered = false;
+                for (u32 i0 = 0; i0 < n_reg && !covered; i0 += 32) {
+                    bool hit = false;
+                    if (i0 + lane < n_reg) {
+                        const debwt_region p = reg[i0 + lane];
+                        const long long prb = (long long)p.rb, pre = (long long)p.re;
+                        const int pqb = (int)p.qb, pqe = (int)p.qe, pw = (int)p.w;
+                        if (!(srb < prb || srb + sl > pre || sq < pqb || sq + sl > pqe) && !(sl - (int)p.seedlen0 > .1 * L)) {
+                            int qd = sq - pqb;
+                            long long rd2 = srb - prb;
+                            int wd = min(cal_max_gap(o, (int)min((long long)qd, rd2)), pw);
+                            hit = qd - rd2 < wd && rd2 - qd < wd;
+                            if (!hit) {
+                                qd = pqe - (sq + sl);
+                                rd2 = pre - (srb + sl);
+                                wd = min(cal_max_gap(o, (int)min((long long)qd, rd2)), pw);
+                                hit = qd - rd2 < wd && rd2 - qd < wd;
+                            }
+                        }
+                    }
+                    covered = __any_sync(FULL, hit);
+                }
+                if (covered) {
+                    bool ov = false;
+                    for (u32 i0 = (u32)k + 1; i0 < n && !ov; i0 += 32) {
+                        bool hit = false;
+                        const u32 i = i0 + lane;
+                        if (i < n && srt[i] != 0) {
+                            const debwt_chain_seed t = S[(u32)srt[i]];
+                            const int tq = (int)t.qbeg, tl = (int)t.len;
+                            const long long trb = (long long)t.rbeg;
+                            if (!(tl < sl * .95))
+                                hit = (sq <= tq && sq + sl - tq >= (sl >> 2) && (long long)(tq - sq) != trb - srb) ||
+                                      (tq <= sq && tq + tl - sq >= (sl >> 2) && (long long)(sq - tq) != srb - trb);
+                        }
+                        ov = __any_sync(FULL, hit);
+                    }
+                    if (!ov) {
+                        if (lane == 0) srt[k] = 0;
+                        __syncwarp();
+                        continue;
+                    }
+                }
+                int aw0 = o.w, aw1 = o.w, score, truesc;
+                long long qb, rb, qe, re;
+                if (sq) {
+                    ExtOut x{};
+                    score = -1;
+                    for (int t = 0; t < 2; ++t) {
+                        const int prev = score;
+                        aw0 = o.w << t;
+                        x = warp_extend(o, sq, [&](int j) { return nt4(q[sq - 1 - j]); }, (int)(srb - rmax0),
+                                        [&](int i) { return ref_base(pac, o.l_pac, (u64)(srb - 1 - i)); }, aw0, o.pen_clip5, sl * o.a, ring, lane);
+                        score = x.score;
+                        if (score == prev || x.max_off < (aw0 >> 1) + (aw0 >> 2)) break;
+                    }
+                    if (x.gscore <= 0 || x.gscore <= score - o.pen_clip5) {
+                        qb = sq - x.qle; rb = srb - x.tle; truesc = score;
+                    } else {
+                        qb = 0; rb = srb - x.gtle; truesc = x.gscore;
+                    }
+                } else {
+                    score = truesc = sl * o.a;
+                    qb = 0; rb = srb;
+                }
+                if (sq + sl != L) {
+                    const int sc0 = score, qe0 = sq + sl;
+                    const long long re0 = srb + sl - rmax0;
+                    ExtOut x{};
+                    for (int t = 0; t < 2; ++t) {
+                        const int prev = score;
+                        aw1 = o.w << t;
+                        x = warp_extend(o, L - qe0, [&](int j) { return nt4(q[qe0 + j]); }, (int)(rmax1 - rmax0 - re0),
+                                        [&](int i) { return ref_base(pac, o.l_pac, (u64)(rmax0 + re0 + i)); }, aw1, o.pen_clip3, sc0, ring, lane);
+                        score = x.score;
+                        if (score == prev || x.max_off < (aw1 >> 1) + (aw1 >> 2)) break;
+                    }
+                    if (x.gscore <= 0 || x.gscore <= score - o.pen_clip3) {
+                        qe = qe0 + x.qle; re = rmax0 + re0 + x.tle; truesc += score - sc0;
+                    } else {
+                        qe = L; re = rmax0 + re0 + x.gtle; truesc += x.gscore - sc0;
+                    }
+                } else {
+                    qe = L; re = srb + sl;
+                }
+                int cov = 0;
+                for (u32 i = lane; i < n; i += 32) {
+                    const debwt_chain_seed t = S[i];
+                    if ((long long)t.qbeg >= qb && (long long)t.qbeg + t.len <= qe && (long long)t.rbeg >= rb && (long long)t.rbeg + t.len <= re)
+                        cov += (int)t.len;
+                }
+                cov = warp_sum(cov);
+                if (lane == 0)
+                    reg[n_reg] = debwt_region{(u64)rb, (u64)re, (u32)qb, (u32)qe, score, truesc, (u32)max(aw0, aw1), (u32)cov, (u32)sl,
+                                              (u32)(ci - c0), ch.record, ch.strand, ch.frac_rep, 0};
+                __syncwarp();
+                ++n_reg;
+            }
+        }
+        if (lane == 0) reg_cnt[rd] = n_reg;
+    }
+}
+
+// One thread per read: its regions from its slots to reg_off
+__global__ void __launch_bounds__(TPB) region_write_kernel(u64 n_reads, const u64* __restrict__ cseed_off, const debwt_region* __restrict__ slots,
+                                                          const u64* __restrict__ reg_off, debwt_region* __restrict__ out) {
+    const u64 rd = (u64)blockIdx.x * TPB + threadIdx.x;
+    if (rd >= n_reads) return;
+    const debwt_region* a = slots + cseed_off[rd];
+    debwt_region* b = out + reg_off[rd];
+    for (u64 i = 0, n = reg_off[rd + 1] - reg_off[rd]; i < n; ++i) b[i] = a[i];
+}
+
 FmView view_of(const debwt_ctx* c) {
     FmView f;
     f.bwt = c->d_bwt; f.spec = c->d_spec_bits; f.occ = c->d_occ; f.sharp = c->d_sharp_sorted;
@@ -1030,7 +1473,8 @@ void drop_samples(debwt_ctx* c) {
     if (c->d_sa_vals) cudaFree(c->d_sa_vals);
     if (c->d_isa_vals) cudaFree(c->d_isa_vals);
     if (c->d_seps_sorted) cudaFree(c->d_seps_sorted);
-    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr; c->d_isa_vals = nullptr; c->d_seps_sorted = nullptr;
+    if (c->d_pac) cudaFree(c->d_pac);
+    c->d_sa_bits = nullptr; c->d_sa_vals = nullptr; c->d_isa_vals = nullptr; c->d_seps_sorted = nullptr; c->d_pac = nullptr;
     c->sa_rate = 0;
 }
 
@@ -1418,6 +1862,19 @@ int debwt_index_locate(debwt_ctx* c, const char* patterns, const uint64_t* offse
     return 0;
 }
 
+// The inverse samples, built from the SA samples the first time after sampling and kept with them
+static int inverse_samples(debwt_ctx* c, const char* name) {
+    if (c->d_isa_vals) return 0;
+    if (cudaMalloc(reinterpret_cast<void**>(&c->d_isa_vals), c->n_sa_samples * 4) != cudaSuccess) {
+        cudaGetLastError();
+        c->d_isa_vals = nullptr;
+        FAIL(std::string(name) + ": out of device memory for the inverse samples");
+    }
+    isa_from_sa_kernel<<<grid_for(c->n), TPB, 0, c->st>>>(sa_view_of(c), c->n, c->d_isa_vals);
+    DEBWT_COUNT(1);
+    return 0;
+}
+
 int debwt_index_extract(debwt_ctx* c, const uint64_t* starts, const uint64_t* ends, uint64_t n_intervals, char* out, uint64_t out_cap) {
     if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
     if (n_intervals == 0) return 0;
@@ -1443,15 +1900,7 @@ int debwt_index_extract(debwt_ctx* c, const uint64_t* starts, const uint64_t* en
     if (!out) FAIL("null argument");
     CUDA_TRY(cudaSetDevice(c->device));
     cudaStream_t st = c->st;
-    if (!c->d_isa_vals) {
-        if (cudaMalloc(reinterpret_cast<void**>(&c->d_isa_vals), c->n_sa_samples * 4) != cudaSuccess) {
-            cudaGetLastError();
-            c->d_isa_vals = nullptr;
-            FAIL("index_extract: out of device memory for the inverse samples");
-        }
-        isa_from_sa_kernel<<<grid_for(n), TPB, 0, st>>>(sa_view_of(c), n, c->d_isa_vals);
-        DEBWT_COUNT(1);
-    }
+    if (inverse_samples(c, "index_extract")) return -1;
     u64* d = nullptr;
     if (cudaMalloc(reinterpret_cast<void**>(&d), h.size() * 8 + total) != cudaSuccess) {
         cudaGetLastError();
@@ -1757,36 +2206,51 @@ int debwt_index_seeds(debwt_ctx* c, const char* reads, const uint64_t* offsets, 
 static_assert(sizeof(debwt_chain) == 40, "debwt_chain is 2 u64 + 5 u32 + float");
 static_assert(sizeof(debwt_chain_seed) == 16, "debwt_chain_seed is u64 + 2 u32");
 
-int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* seed_opts,
-                       const debwt_chain_opts* chain_opts, uint64_t* chain_offsets, uint64_t* n_chain_seeds_out, debwt_chain* chains,
-                       uint64_t chains_cap, debwt_chain_seed* chain_seeds, uint64_t chain_seeds_cap) {
-    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
-    if (!offsets || !chain_offsets || !n_chain_seeds_out || !seed_opts || !chain_opts || (n_reads && !reads) || (chains && !chain_seeds))
-        FAIL("null argument");
-    const debwt_seed_opts op = *seed_opts;
-    const debwt_chain_opts co = *chain_opts;
+}  // extern "C"
+
+// The checks of debwt_chain_opts; `name` starts the messages
+static int check_chain_opts(const char* name, const debwt_chain_opts& co) {
     const std::pair<int32_t, const char*> ints[] = {{co.w, "w"}, {co.max_chain_gap, "max_chain_gap"}, {co.min_chain_weight, "min_chain_weight"},
                                                      {co.max_chain_extend, "max_chain_extend"}};
     for (const auto& [v, nm] : ints)
-        if (v < 0) FAIL(std::string("index_chains: ") + nm + " must not be negative, not " + std::to_string(v));
+        if (v < 0) FAIL(std::string(name) + ": " + nm + " must not be negative, not " + std::to_string(v));
     const std::pair<float, const char*> reals[] = {{co.mask_level, "mask_level"}, {co.drop_ratio, "drop_ratio"}};
     for (const auto& [v, nm] : reals)
-        if (!std::isfinite(v) || v < 0) FAIL(std::string("index_chains: ") + nm + " must be finite and not negative, not " + std::to_string(v));
-    const u64 m = n_reads;
-    u64 max_len = 0;
-    if (check_seed_input(c, "index_chains", offsets, m, op, max_len)) return -1;
-    if (m == 0) {
-        chain_offsets[0] = 0;
-        *n_chain_seeds_out = 0;
-        return 0;
+        if (!std::isfinite(v) || v < 0) FAIL(std::string(name) + ": " + nm + " must be finite and not negative, not " + std::to_string(v));
+    return 0;
+}
+
+// The device buffers of one chaining run (its seeding run included), freed with it
+struct ChainRun {
+    SeedRun seeds;
+    char* scratch = nullptr;          // ChainScratch | chain counts | seed counts | chain offsets | seed offsets | n_sorted | frac_rep
+    char* out = nullptr;              // the kept chains | their seeds
+    u64 *d_coff = nullptr, *d_soff = nullptr;
+    debwt_chain* chains = nullptr;
+    debwt_chain_seed* cseeds = nullptr;
+    u64 total = 0, total_seeds = 0;
+    ChainRun() = default;
+    ChainRun(const ChainRun&) = delete;
+    ~ChainRun() {
+        if (scratch) cudaFree(scratch);
+        if (out) cudaFree(out);
     }
-    SeedRun r;
-    const int rc = run_seeds(c, "index_chains", reads, offsets, m, op, max_len, nullptr, r, [](u64, u64 total_hits) { return total_hits ? 1 : 0; });
+};
+
+// The seeding and chaining of debwt_index_chains for m >= 1 checked reads, leaving everything in r: chain_kernel and the
+// two scans (chain_offsets, when given, receives the chain offsets; all zero when the reads have no hits), then
+// proceed(total chains, total chain seeds): 1 goes on to write the kept chains and their seeds on the device, 0 stops
+// there, -1 fails the call.  Returns 0 also when there are no hits.
+template <class Proceed>
+static int run_chains(debwt_ctx* c, const char* name, const char* reads, const uint64_t* offsets, u64 m, const debwt_seed_opts& op,
+                      const debwt_chain_opts& co, u64 max_len, uint64_t* chain_offsets, ChainRun& cr, Proceed&& proceed) {
+    const std::string nm(name);
+    SeedRun& r = cr.seeds;
+    const int rc = run_seeds(c, name, reads, offsets, m, op, max_len, nullptr, r, [](u64, u64 total_hits) { return total_hits ? 1 : 0; });
     if (rc < 0) return -1;
     if (rc == 0) {                                                                // no hits: no chains
-        std::fill(chain_offsets, chain_offsets + m + 1, 0ull);
-        *n_chain_seeds_out = 0;
-        return 0;
+        if (chain_offsets) std::fill(chain_offsets, chain_offsets + m + 1, 0ull);
+        return proceed(0, 0) < 0 ? -1 : 0;
     }
     cudaStream_t st = c->st;
     const u64 H = r.total_hits, nb = (m + TPB - 1) / TPB;
@@ -1804,7 +2268,7 @@ int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets,
     // seeds, the offsets of both, chains after the weight pass, frac_rep; the slot bitmap and its summary
     const u64 n_bits = H / 64 + m + 1, n_summary = H / 4096 + m + 1;
     ChainScratch s;
-    u64 *d_ccnt, *d_scnt, *d_coff, *d_soff;
+    u64 *d_ccnt, *d_scnt;
     u32* d_nsorted;
     float* d_frac;
     char* p = nullptr;
@@ -1815,17 +2279,16 @@ int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets,
     auto lay_out = [&]() {
         take(s.cs, H); take(s.key, H); take(s.rec, H); take(s.idx, H); take(s.nxt, H); take(s.tail, H); take(s.list, H);
         take(s.bits, n_bits); take(s.summary, n_summary);
-        take(d_ccnt, m); take(d_scnt, m); take(d_coff, m + 1); take(d_soff, m + 1); take(d_nsorted, m); take(d_frac, m);
+        take(d_ccnt, m); take(d_scnt, m); take(cr.d_coff, m + 1); take(cr.d_soff, m + 1); take(d_nsorted, m); take(d_frac, m);
     };
     lay_out();
     const u64 scratch_bytes = (u64)reinterpret_cast<uintptr_t>(p);
-    char* d_c = nullptr;
-    if (cudaMalloc(reinterpret_cast<void**>(&d_c), scratch_bytes) != cudaSuccess) {
+    if (cudaMalloc(reinterpret_cast<void**>(&cr.scratch), scratch_bytes) != cudaSuccess) {
         cudaGetLastError();
-        FAIL("index_chains: out of device memory for " + std::to_string(scratch_bytes) + " bytes of chaining scratch (" + std::to_string(H) + " hits)");
+        cr.scratch = nullptr;
+        FAIL(nm + ": out of device memory for " + std::to_string(scratch_bytes) + " bytes of chaining scratch (" + std::to_string(H) + " hits)");
     }
-    struct Free { char* p; ~Free() { cudaFree(p); } } free_c{d_c};
-    p = d_c;
+    p = cr.scratch;
     lay_out();
     int sms = 0, per_sm = 0;
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
@@ -1836,34 +2299,200 @@ int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets,
                                                       d_ccnt, d_scnt, d_nsorted, d_frac);
     hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_ccnt, m, r.d_tot);
     scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
-    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_ccnt, m, r.d_base, d_coff);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_ccnt, m, r.d_base, cr.d_coff);
     hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_scnt, m, r.d_tot);
     scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
-    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_scnt, m, r.d_base, d_soff);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_scnt, m, r.d_base, cr.d_soff);
     DEBWT_COUNT(7);
-    u64 total_seeds = 0;
-    CUDA_TRY(cudaMemcpyAsync(chain_offsets, d_coff, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(&total_seeds, d_soff + m, 8, cudaMemcpyDeviceToHost, st));
+    if (chain_offsets) CUDA_TRY(cudaMemcpyAsync(chain_offsets, cr.d_coff, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&cr.total, cr.d_coff + m, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&cr.total_seeds, cr.d_soff + m, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
-    *n_chain_seeds_out = total_seeds;
-    const u64 total = chain_offsets[m];
-    if (!chains || total == 0) return 0;                                          // size query
-    if (total > chains_cap || total_seeds > chain_seeds_cap)
-        FAIL("index_chains: the reads have " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds; chains holds " +
-             std::to_string(chains_cap) + " and chain_seeds " + std::to_string(chain_seeds_cap));
-    char* d_out = nullptr;
-    if (cudaMalloc(reinterpret_cast<void**>(&d_out), total * sizeof(debwt_chain) + total_seeds * sizeof(debwt_chain_seed)) != cudaSuccess) {
+    const int go = proceed(cr.total, cr.total_seeds);
+    if (go <= 0) return go;
+    const u64 total = cr.total, total_seeds = cr.total_seeds;
+    if (cudaMalloc(reinterpret_cast<void**>(&cr.out), total * sizeof(debwt_chain) + total_seeds * sizeof(debwt_chain_seed)) != cudaSuccess) {
         cudaGetLastError();
-        FAIL("index_chains: out of device memory for " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds");
+        cr.out = nullptr;
+        FAIL(nm + ": out of device memory for " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds");
     }
-    Free free_out{d_out};
-    debwt_chain* d_chains = reinterpret_cast<debwt_chain*>(d_out);
-    debwt_chain_seed* d_cseeds = reinterpret_cast<debwt_chain_seed*>(d_chains + total);
-    chain_write_kernel<<<grid_for(m), TPB, 0, st>>>(m, r.hits, r.d_hoff, s, d_nsorted, d_frac, d_coff, d_soff, d_chains, d_cseeds);
+    cr.chains = reinterpret_cast<debwt_chain*>(cr.out);
+    cr.cseeds = reinterpret_cast<debwt_chain_seed*>(cr.chains + total);
+    chain_write_kernel<<<grid_for(m), TPB, 0, st>>>(m, r.hits, r.d_hoff, s, d_nsorted, d_frac, cr.d_coff, cr.d_soff, cr.chains, cr.cseeds);
     DEBWT_COUNT(1);
-    CUDA_TRY(cudaMemcpyAsync(chains, d_chains, total * sizeof(debwt_chain), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(chain_seeds, d_cseeds, total_seeds * sizeof(debwt_chain_seed), cudaMemcpyDeviceToHost, st));
+    return 1;
+}
+
+extern "C" {
+
+int debwt_index_chains(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* seed_opts,
+                       const debwt_chain_opts* chain_opts, uint64_t* chain_offsets, uint64_t* n_chain_seeds_out, debwt_chain* chains,
+                       uint64_t chains_cap, debwt_chain_seed* chain_seeds, uint64_t chain_seeds_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !chain_offsets || !n_chain_seeds_out || !seed_opts || !chain_opts || (n_reads && !reads) || (chains && !chain_seeds))
+        FAIL("null argument");
+    const debwt_seed_opts op = *seed_opts;
+    const debwt_chain_opts co = *chain_opts;
+    if (check_chain_opts("index_chains", co)) return -1;
+    const u64 m = n_reads;
+    u64 max_len = 0;
+    if (check_seed_input(c, "index_chains", offsets, m, op, max_len)) return -1;
+    if (m == 0) {
+        chain_offsets[0] = 0;
+        *n_chain_seeds_out = 0;
+        return 0;
+    }
+    ChainRun cr;
+    const int rc = run_chains(c, "index_chains", reads, offsets, m, op, co, max_len, chain_offsets, cr, [&](u64 total, u64 total_seeds) -> int {
+        *n_chain_seeds_out = total_seeds;
+        if (!chains || total == 0) return 0;                                      // size query
+        if (total > chains_cap || total_seeds > chain_seeds_cap)
+            FAIL("index_chains: the reads have " + std::to_string(total) + " chains and " + std::to_string(total_seeds) + " chain seeds; chains holds " +
+                 std::to_string(chains_cap) + " and chain_seeds " + std::to_string(chain_seeds_cap));
+        return 1;
+    });
+    if (rc <= 0) return rc;
+    cudaStream_t st = c->st;
+    CUDA_TRY(cudaMemcpyAsync(chains, cr.chains, cr.total * sizeof(debwt_chain), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(chain_seeds, cr.cseeds, cr.total_seeds * sizeof(debwt_chain_seed), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+}  // extern "C"
+
+static_assert(sizeof(debwt_region) == 64, "debwt_region is 2 u64 + 11 u32 + float");
+
+// bwa's pac, derived from the index the first time after sampling: the forward records' bases by the LF walks of
+// extract_kernel (inverse samples built here if extract has not built them), 2 bits each.
+static int build_pac(debwt_ctx* c, const char* name) {
+    if (c->d_pac) return 0;
+    const std::string nm(name);
+    if (sorted_separators(c, name) || inverse_samples(c, name)) return -1;
+    cudaStream_t st = c->st;
+    const u64 R = c->n_rec, l_pac = (c->n - R) / 2, words = l_pac / 16 + 1;
+    u64 fwd_end = 0;
+    CUDA_TRY(cudaMemcpyAsync(&fwd_end, c->d_seps_sorted + R / 2 - 1, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (fwd_end - (R / 2 - 1) != l_pac) FAIL("internal: the forward records do not hold (N - R) / 2 bases");
+    if (cudaMalloc(reinterpret_cast<void**>(&c->d_pac), words * 4) != cudaSuccess) {
+        cudaGetLastError();
+        c->d_pac = nullptr;
+        FAIL(nm + ": out of device memory for the " + std::to_string(words * 4) + "-byte reference (pac)");
+    }
+    CUDA_TRY(cudaMemsetAsync(c->d_pac, 0, words * 4, st));
+    const u64 n_blocks = (fwd_end + c->sa_rate - 1) / c->sa_rate;
+    if (n_blocks) {
+        pac_kernel<<<grid_for(n_blocks), TPB, 0, st>>>(view_of(c), sa_view_of(c), c->d_isa_vals, c->d_seps_sorted, R, fwd_end, n_blocks, c->d_pac);
+        DEBWT_COUNT(1);
+    }
+    return 0;
+}
+
+extern "C" {
+
+int debwt_index_regions(debwt_ctx* c, const char* reads, const uint64_t* offsets, uint64_t n_reads, const debwt_seed_opts* seed_opts,
+                        const debwt_chain_opts* chain_opts, const debwt_ext_opts* ext_opts, uint64_t* region_offsets, debwt_region* regions,
+                        uint64_t regions_cap) {
+    if (!c || !c->indexed || !c->sa_rate) FAIL("no sampled suffix array: call debwt_index_sample_sa first");
+    if (!offsets || !region_offsets || !seed_opts || !chain_opts || !ext_opts || (n_reads && !reads)) FAIL("null argument");
+    const debwt_seed_opts op = *seed_opts;
+    const debwt_chain_opts co = *chain_opts;
+    const debwt_ext_opts eo = *ext_opts;
+    if (check_chain_opts("index_regions", co)) return -1;
+    const std::pair<int32_t, const char*> pos[] = {{eo.a, "a"}, {eo.e_del, "e_del"}, {eo.e_ins, "e_ins"}};
+    for (const auto& [v, nm] : pos)
+        if (v < 1) FAIL(std::string("index_regions: ") + nm + " must be at least 1, not " + std::to_string(v));
+    const std::pair<int32_t, const char*> nonneg[] = {{eo.b, "b"}, {eo.o_del, "o_del"}, {eo.o_ins, "o_ins"}, {eo.pen_clip5, "pen_clip5"},
+                                                       {eo.pen_clip3, "pen_clip3"}, {eo.zdrop, "zdrop"}};
+    for (const auto& [v, nm] : nonneg)
+        if (v < 0) FAIL(std::string("index_regions: ") + nm + " must not be negative, not " + std::to_string(v));
+    for (const auto& [v, nm] : {std::pair<int32_t, const char*>{eo.a, "a"}, {eo.b, "b"}})
+        if (v > 127) FAIL(std::string("index_regions: ") + nm + " = " + std::to_string(v) + " does not fit bwa's int8_t scoring matrix (at most 127)");
+    if (co.w > kMaxExtW)
+        FAIL("index_regions: w = " + std::to_string(co.w) + " is too wide: the band w << 1 of a retry must fit the DP window of " +
+             std::to_string(2 * (kMaxExtW << 1) + 3) + " columns (w at most " + std::to_string(kMaxExtW) + ")");
+    const u64 m = n_reads;
+    u64 max_len = 0;
+    if (check_seed_input(c, "index_regions", offsets, m, op, max_len)) return -1;
+    {
+        const long long mul = std::max({eo.a, eo.b, eo.e_del, eo.e_ins}), add = std::max({eo.o_del, eo.o_ins, eo.pen_clip5, eo.pen_clip3, eo.zdrop});
+        const long double bound = (long double)(2 * max_len + 4 * (u64)co.w + 2) * mul + add;
+        if (bound >= 2147483648.0L)
+            FAIL("index_regions: the options can overflow a 32-bit score: (2 x " + std::to_string(max_len) + " (the longest read) + 4 w + 2) x " +
+                 "max(a, b, e_del, e_ins) + max(o_del, o_ins, pen_clip5, pen_clip3, zdrop) = " + std::to_string((double)bound) + " is not below 2^31");
+    }
+    region_offsets[0] = 0;
+    if (m == 0) return 0;
+    ChainRun cr;
+    const int rc = run_chains(c, "index_regions", reads, offsets, m, op, co, max_len, nullptr, cr, [](u64 total, u64) { return total ? 1 : 0; });
+    if (rc < 0) return -1;
+    if (rc == 0) {                                                                // no chains: no regions
+        std::fill(region_offsets, region_offsets + m + 1, 0ull);
+        return 0;
+    }
+    if (build_pac(c, "index_regions")) return -1;
+    cudaStream_t st = c->st;
+    SeedRun& r = cr.seeds;
+    const u64 S = cr.total_seeds, nc = cr.total, nb = (m + TPB - 1) / TPB;
+    // per chain seed: kept seed, its score, srt, a region slot (92 bytes); per chain: kept seeds; per read: regions, offsets
+    ExtScratch xs;
+    u64 *d_rcnt, *d_roff;
+    char* p = nullptr;
+    auto take = [&](auto*& dst, u64 n) {
+        dst = reinterpret_cast<std::remove_reference_t<decltype(dst)>>(p);
+        p += (n * sizeof(*dst) + 15) / 16 * 16;
+    };
+    auto lay_out = [&]() {
+        take(xs.reg, S); take(xs.fs, S); take(xs.srt, S); take(xs.sc, S); take(xs.fn, nc); take(d_rcnt, m); take(d_roff, m + 1);
+    };
+    lay_out();
+    const u64 scratch_bytes = (u64)reinterpret_cast<uintptr_t>(p);
+    char* d_x = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_x), scratch_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL("index_regions: out of device memory for " + std::to_string(scratch_bytes) + " bytes of extension scratch (" + std::to_string(S) +
+             " chain seeds)");
+    }
+    struct Free { char* p; ~Free() { cudaFree(p); } } free_x{d_x};
+    p = d_x;
+    lay_out();
+    ExtParams prm;
+    prm.a = eo.a; prm.b = eo.b; prm.o_del = eo.o_del; prm.e_del = eo.e_del; prm.o_ins = eo.o_ins; prm.e_ins = eo.e_ins;
+    prm.pen_clip5 = eo.pen_clip5; prm.pen_clip3 = eo.pen_clip3; prm.zdrop = eo.zdrop; prm.w = co.w; prm.min_chain_weight = co.min_chain_weight;
+    prm.ring = std::max<u32>(2 * ((u32)co.w << 1) + 3, 200);
+    prm.l_pac = (c->n - c->n_rec) / 2;
+    const size_t smem = (size_t)EXT_WARPS * prm.ring * sizeof(int2);
+    CUDA_TRY(cudaFuncSetAttribute(ext_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int sms = 0, per_sm = 0;
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    CUDA_TRY(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxThreadsPerMultiProcessor, c->device));
+    const u64 n_warps = std::min<u64>((u64)sms * (u64)per_sm / 32, m);
+    CUDA_TRY(cudaMemsetAsync(r.d_next, 0, 8, st));
+    ext_kernel<<<(unsigned)((n_warps + EXT_WARPS - 1) / EXT_WARPS), EXT_WARPS * 32, smem, st>>>(
+        reinterpret_cast<const u8*>(r.d), r.d_o, m, cr.chains, cr.d_coff, cr.cseeds, cr.d_soff, c->d_pac, c->d_seps_sorted, prm, xs, r.d_next, d_rcnt);
+    hit_count_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_rcnt, m, r.d_tot);
+    scan_u64_kernel<<<1, TPB, 0, st>>>(r.d_tot, nb, r.d_base);
+    hit_offsets_kernel<<<(unsigned)nb, TPB, 0, st>>>(d_rcnt, m, r.d_base, d_roff);
+    DEBWT_COUNT(4);
+    CUDA_TRY(cudaMemcpyAsync(region_offsets, d_roff, (m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    const u64 total = region_offsets[m];
+    if (!regions || total == 0) return 0;                                         // size query
+    if (total > regions_cap)
+        FAIL("index_regions: the reads have " + std::to_string(total) + " regions; regions holds " + std::to_string(regions_cap));
+    debwt_region* d_out = nullptr;
+    if (cudaMalloc(reinterpret_cast<void**>(&d_out), total * sizeof(debwt_region)) != cudaSuccess) {
+        cudaGetLastError();
+        FAIL("index_regions: out of device memory for " + std::to_string(total) + " regions");
+    }
+    Free free_out{reinterpret_cast<char*>(d_out)};
+    region_write_kernel<<<grid_for(m), TPB, 0, st>>>(m, cr.d_soff, xs.reg, d_roff, d_out);
+    DEBWT_COUNT(1);
+    CUDA_TRY(cudaMemcpyAsync(regions, d_out, total * sizeof(debwt_region), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
     return 0;

@@ -304,7 +304,7 @@ int debwt_index_seeds(debwt_ctx* ctx, const char* reads, const uint64_t* offsets
    max_chain_extend, on a negative or non-finite mask_level or drop_ratio (the message names the option), and on NULL
    arguments (chain_seeds may be NULL only with chains).  Besides the seeding scratch the call holds 68 bytes of device
    memory per hit.  n_reads = 0 only writes chain_offsets[0] = 0 and *n_chain_seeds_out = 0.  Not done here: bwa's
-   mem_flt_chained_seeds (it needs the extension's scores) and ALT contigs (is_alt is 0). */
+   mem_flt_chained_seeds (it needs the extension's scores; debwt_index_regions runs it) and ALT contigs (is_alt is 0). */
 typedef struct debwt_chain_opts {
     int32_t w, max_chain_gap, min_chain_weight, max_chain_extend;  /* bwa: 100, 10000, 0 (-W), 1 << 30 */
     float mask_level, drop_ratio;                                   /* bwa: 0.50, 0.50 (-D) */
@@ -325,6 +325,82 @@ int debwt_index_chains(debwt_ctx* ctx, const char* reads, const uint64_t* offset
                        const debwt_seed_opts* seed_opts, const debwt_chain_opts* chain_opts,
                        uint64_t* chain_offsets /* n_reads + 1 */, uint64_t* n_chain_seeds_out,
                        debwt_chain* chains, uint64_t chains_cap, debwt_chain_seed* chain_seeds, uint64_t chain_seeds_cap);
+/* BWA-MEM's seed extension (bwa 0.7.17's mem_flt_chained_seeds and mem_chain2aln) from reads to alignment regions, with
+   the seeding and chaining of debwt_index_chains inside (seed_opts and chain_opts as there; chain_opts->w is also the
+   extension's band, as bwa's one -w).  ext_opts are bwa's -A, -B, -O, -E (deletion, insertion), -L (5', 3') and -d.
+   Scoring: mat[i][j] = i == j ? a : -b for bases i, j < 4; any pair with code 4 scores -1.  Read symbols A, C, G, T in
+   either case are 0-3, anything else 4; reference bases are 0-3.  A deletion skips reference bases (o_del, e_del), an
+   insertion skips query bases (o_ins, e_ins); a gap of k costs o + k e.  The reference is bwa's pac: the forward records
+   concatenated, l_pac = (N - R) / 2 bases; coordinate x >= l_pac is the complement of forward base 2 l_pac - 1 - x.
+     cal_max_gap(L): l_del = (int)((double)(L a - o_del) / e_del + 1.), l_ins likewise; min(max(l_del, l_ins, 1), w << 1).
+     fetch(beg, mid, end): [beg, end) clipped to the record holding mid, on mid's strand (the reverse copy of a record at
+       forward [fb, fe) spans [2 l_pac - fe, 2 l_pac - fb)).
+     seed_sw(s): -1 if len >= 200.  qb = max(qbeg - 50, 0), qe = min(qend + 50, l_query), rb = max(rbeg - 50, 0),
+       re = min(rbeg + len + 50, 2 l_pac), mid = (2 rbeg + len) >> 1; if rb < l_pac < re: re = l_pac when mid < l_pac,
+       else rb = l_pac.  -1 if qe - qb >= 200 or re - rb >= 200.  Else the best local (Gotoh, H >= 0, gaps open from H)
+       score of query[qb, qe) against fetch(rb, mid, re).
+     mem_flt_chained_seeds: min_l = min_chain_weight ? 1.1f min_chain_weight : 5.5f log(l_query) (double); min_HSP =
+       (int)(a min_l + .499).  If min_l > 0.05f l_query nothing is filtered and every seed's score is len.  Otherwise a
+       chain keeps, in order, the seeds with sc = seed_sw < 0 (score len a) or sc >= min_HSP (score sc).
+     extend(qlen, q, tlen, t, w, end_bonus, h0) is ksw_extend2: row 0 h[0] = h0, h[1] = max(h0 - oe_ins, 0) when
+       h0 > oe_ins, then h[j] = h[j-1] - e_ins while h[j-1] > e_ins; w = min(w, max_ins, max_del), max_ins =
+       max(1, (int)((double)(qlen a + end_bonus - o_ins) / e_ins + 1.)), max_del likewise; max = h0, max_i = max_j =
+       max_ie = gscore = -1, max_off = 0, beg = 0, end = qlen.  Row i over t: beg = max(beg, i - w), end = min(end, i + w
+       + 1, qlen); h1 = beg ? 0 : max(0, h0 - o_del - e_del (i + 1)); f = m = 0, mj = -1; for j in [beg, end): M =
+       h[j] ? h[j] + mat : 0, h = max(M, e[j], f), h[j] = h1, h1 = h, if m <= h: m = h, mj = j; e[j] = max(e[j] - e_del,
+       M - oe_del, 0); f = max(f - e_ins, M - oe_ins, 0).  Then h[end] = h1, e[end] = 0; if max(beg, end) == qlen:
+       max_ie = gscore > h1 ? max_ie : i, gscore = max(gscore, h1).  Stop if m == 0.  If m > max: max = m, max_i = i,
+       max_j = mj, max_off = max(max_off, |mj - i|); else with zdrop > 0 stop when max - m - (di - dj) e_del > zdrop
+       (di = i - max_i > dj = mj - max_j) or max - m - (dj - di) e_ins > zdrop (otherwise).  beg = the first j in
+       [beg, end) with (h, e) != 0 (else end); end = min(j + 2, qlen) for the last j in [beg, end] with (h, e) != 0 (else
+       beg - 1).  Returns max, qle = max_j + 1, tle = max_i + 1, gtle = max_ie + 1, gscore, max_off.
+     mem_chain2aln(c), over each kept chain in filter order after the seed filter: nothing if it has no seeds.  rmax =
+       [min(rbeg - qbeg - cal_max_gap(qbeg)), max(rbeg + len + r + cal_max_gap(r))] (r = l_query - qend) clamped to
+       [0, 2 l_pac]; if it crosses l_pac, the side of the first seed's rbeg; then fetch(rmax0, first rbeg, rmax1).  The
+       seeds are visited by descending (score, index).  Seed s is covered by an earlier region p of the read when s lies
+       inside p on both query and reference, s.len - p.seedlen0 <= .1 l_query, and with qd = s.qbeg - p.qb, rd = s.rbeg -
+       p.rb, w' = min(cal_max_gap(min(qd, rd)), p.w): |qd - rd| < w', or the same behind the seed (p.qe - s.qend, p.re -
+       s.rend).  A covered seed is skipped (and marked) unless an unmarked seed t visited before it has t.len >= .95 s.len
+       and overlaps it by >= s.len >> 2 on the query, on another diagonal (either order).  Else a region: left, if qbeg >
+       0, extend(reversed query[0, qbeg), reversed ref[rmax0, rbeg), w << k, pen_clip5, h0 = len a) for k = 0, 1, stopping
+       when the score equals the one before (-1 at first) or max_off < (bw >> 1) + (bw >> 2); local (qb = qbeg - qle, rb =
+       rbeg - tle, truesc = score) if gscore <= 0 or gscore <= score - pen_clip5, else to-end (qb = 0, rb = rbeg - gtle,
+       truesc = gscore); with qbeg = 0, score = truesc = len a, qb = 0, rb = rbeg.  Right, if qend < l_query, the same over
+       query[qend, l_query) and ref[rbeg + len, rmax1) with h0 = sc0 = score (so the first try stops when it returns sc0)
+       and pen_clip3: qe = qend + qle, re = rbeg + len + tle (local) or qe = l_query, re = rbeg + len + gtle (to-end), and
+       truesc += chosen - sc0; else qe = l_query, re = rbeg + len.  seedcov = the len of the chain's seeds inside [qb, qe) x
+       [rb, re); w = the widest band used; seedlen0 = len; frac_rep, record and strand the chain's.
+   A read's regions are regions[region_offsets[i] .. region_offsets[i + 1]) in bwa's order: chain by chain, inside a
+   chain in the order of extension.  region_offsets[n_reads + 1] is always written; regions == NULL is a size query.
+   More regions than regions_cap fails, names the total and writes nothing into regions.  The regions are computed once
+   per call: a call whose cap is large enough seeds, chains and extends once.  Needs debwt_index_sample_sa; the first
+   call after it derives the pac from the index (N / 8 bytes, kept and dropped with the samples).  Fails, writing nothing
+   into regions, on every input that debwt_index_chains refuses (the messages name index_regions), on a or e_del or e_ins
+   below 1, on a negative b, o_del, o_ins, pen_clip5, pen_clip3 or zdrop, on a or b above 127 (bwa's scoring matrix is
+   int8_t), on w above 1024 (the band w << 1 of a retry must fit the kernel's DP window of 4099 columns), and on options
+   under which a score could leave int32: (2 x longest read + 4 w + 2) max(a, b, e_del, e_ins) + max(o_del, o_ins,
+   pen_clip5, pen_clip3, zdrop) must stay below 2^31.  Not done here: mem_sort_dedup_patch, mem_mark_primary_se, mapq,
+   CIGAR, SAM, pairing and ALT contigs. */
+typedef struct debwt_ext_opts {
+    int32_t a, b;                  /* match score, mismatch penalty        bwa: 1, 4   (-A, -B) */
+    int32_t o_del, e_del;          /* deletion open / extend               bwa: 6, 1   (-O, -E) */
+    int32_t o_ins, e_ins;          /* insertion open / extend              bwa: 6, 1            */
+    int32_t pen_clip5, pen_clip3;  /* clipping penalties                   bwa: 5, 5   (-L)     */
+    int32_t zdrop;                 /* Z-dropoff, 0 disables                bwa: 100    (-d)     */
+} debwt_ext_opts;
+typedef struct debwt_region {      /* bwa's mem_alnreg_t, the fields mem_chain2aln sets */
+    uint64_t rb, re;               /* reference span [rb, re) in bwa's forward-reverse coordinate */
+    uint32_t qb, qe;               /* query span [qb, qe) */
+    int32_t  score, truesc;
+    uint32_t w, seedcov, seedlen0;
+    uint32_t chain;                /* index of its chain among the read's chains (debwt_index_chains order) */
+    uint32_t record, strand;       /* the chain's */
+    float    frac_rep;
+    uint32_t pad_;
+} debwt_region;                    /* 64 bytes */
+int debwt_index_regions(debwt_ctx* ctx, const char* reads, const uint64_t* offsets, uint64_t n_reads,
+                        const debwt_seed_opts* seed_opts, const debwt_chain_opts* chain_opts, const debwt_ext_opts* ext_opts,
+                        uint64_t* region_offsets /* n_reads + 1 */, debwt_region* regions, uint64_t regions_cap);
 /* At-scale verifier: inverts the BWT by its LF mapping (the walk of src/LFsearch.c:49-166, as parallel list ranking) and
    compares every symbol with the text T given by the caller (ASCII, '#' between records, '$' last; host or device
    pointer).  *n_bad_out = rows that are not on the one N-cycle or whose symbol differs; 0 <=> the result is the BWT of
